@@ -1,13 +1,16 @@
 #!/usr/bin/env python
 """bench.py -- batched env-steps/sec of the tabletop_manipulation hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-envs E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--num-envs E] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): tabletop_manipulation, sparse reward, reset-free train horizon
 200,000, 1,048,576 envs per GPU (weak scaling), random actions pre-generated on the device
 (torch.rand, seed 1234+rank) in a ring of 64 batches (768 MB > L2), observations / rewards / dones
 written to a ring of 16 output slots (848 MB > L2).  One "step" = one launch of the fused step kernel
-over the whole batch (env.step + PersistentStateWrapper bookkeeping).
+over the whole batch (env.step + PersistentStateWrapper bookkeeping).  `--steps K` is the number of timed
+steps: after one untimed K-step priming block, K steps run inside one CUDA-event pair.  e2e times K host-buffer
+steps (or --e2e-steps) after three untimed ones; at K = 20 that region is only tens of ms, so a steady e2e figure
+wants a larger K.
 
 One JSON line on stdout (rank 0):
   value        whole-job env-steps/s, inputs resident in HBM, CUDA-event timed, max over ranks
@@ -497,8 +500,9 @@ def config_dict(args, n_total):
 
 # ----------------------------------------------------------------------------------------------- GPU arm
 
-MIN_REGION_S = 0.30      # the CUDA-event pair always brackets at least this much device time (VERDICT r1: a 0.33 ms region
-                         # made the driver's --steps 20 run measure the NCCL barrier's aftermath, not the kernel)
+MIN_REGION_S = 0.30      # a sweep point repeats its K-step block until the CUDA-event pair brackets this much device time
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this many bytes in all, .npy headers included
+NPY_HEADER_BYTES = 4096  # bound on the header numpy writes in front of one .npy array
 
 
 def pin_to_gpu_numa(local):
@@ -518,27 +522,28 @@ def pin_to_gpu_numa(local):
         return f"unavailable ({type(e).__name__})"
 
 
-def timed_blocks(rollout, steps, barrier, dev):
+def timed_blocks(rollout, steps, barrier, dev, reps=None):
     """Time R repetitions of the K-step block with ONE CUDA-event pair on the launching stream.
 
     barrier -> one untimed K-step priming block (the NCCL barrier kernel evicts the L2-resident state and the first
-    launches after it pay for that; at N=1 it is a no-op) -> estimate the block time -> choose R so the timed region is
-    >= MIN_REGION_S (same R on every rank) -> barrier -> priming block -> e0, R x K steps, e1 -> sync -> max over ranks.
-    Returns (ms_total, reps)."""
+    launches after it pay for that; at N=1 it is a no-op) -> [reps None: estimate the block time -> choose R so the timed
+    region is >= MIN_REGION_S (same R on every rank) -> barrier -> priming block] -> e0, R x K steps, e1 -> sync -> max
+    over ranks.  Returns (ms_total, reps)."""
     import torch
 
     from earl_benchmark_b200.distributed import max_over_ranks
     barrier()
     rollout(steps)
-    a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a0.record()
-    rollout(steps)
-    a1.record()
-    torch.cuda.synchronize()
-    est_ms = max(max_over_ranks(a0.elapsed_time(a1), dev), 1e-3)
-    reps = int(min(4096, max(1, -(-MIN_REGION_S * 1e3 // est_ms))))
-    barrier()
-    rollout(steps)
+    if reps is None:
+        a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a0.record()
+        rollout(steps)
+        a1.record()
+        torch.cuda.synchronize()
+        est_ms = max(max_over_ranks(a0.elapsed_time(a1), dev), 1e-3)
+        reps = int(min(4096, max(1, -(-MIN_REGION_S * 1e3 // est_ms))))
+        barrier()
+        rollout(steps)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(reps):
@@ -659,6 +664,27 @@ def ncu_traffic(num_envs):
         return None, None
 
 
+def dump_outputs(out_dir, outputs):
+    """Write the device tensors `outputs` (name -> [N, ...], one row per env) as out_dir/<name>.npy in float32.  When they
+    would exceed DUMP_BYTES, the same seeded sample of rows is written for every tensor, its env indices as
+    env_index.npy (float64)."""
+    import numpy as np
+    import torch
+    n = next(iter(outputs.values())).shape[0]
+    row_bytes = sum(4 * t[0].numel() for t in outputs.values())
+    payload = DUMP_BYTES - NPY_HEADER_BYTES * (len(outputs) + 1)
+    idx = None
+    if n * row_bytes > payload:
+        idx = np.sort(np.random.RandomState(0).choice(n, payload // (row_bytes + 8), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if idx is not None:
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    if idx is not None:
+        np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -693,15 +719,19 @@ def run_ours(args):
     env = train.env
     sampler = ClockSampler(local) if rank == 0 else None
 
-    # warm-up: W steps as asked, then keep the GPU busy for >= 1 s so clocks are sampled under load
+    # warm-up: W steps as asked, then keep the GPU busy for >= 1 s so clocks are sampled under load; that second part runs a
+    # time-dependent number of steps, so the state is put back to where the W steps left it: with the same arguments the
+    # timed steps see the same inputs in every run
     env.rollout_into(actions, max(args.warmup, 3), obs, rew, done)
-    torch.cuda.synchronize()
+    warm_state = env.get_state()
     t_w = time.perf_counter()
     while not args.profile and time.perf_counter() - t_w < 1.0:
         env.rollout_into(actions, 256, obs, rew, done)
         torch.cuda.synchronize()
+    env.set_state(warm_state)
+    del warm_state
 
-    # ---- device-resident timing: `reps` repetitions of the K-step block inside one CUDA-event pair
+    # ---- device-resident timing: the K timed steps inside one CUDA-event pair
     launches0 = env.launch_count
     t_region0 = time.perf_counter()
     if args.profile:
@@ -711,14 +741,17 @@ def run_ours(args):
         env.rollout_into(actions, args.steps, obs, rew, done)
         e1.record()
         barrier()
-        ms, reps = max_over_ranks(e0.elapsed_time(e1), dev), 1
+        ms = max_over_ranks(e0.elapsed_time(e1), dev)
         launches = env.launch_count - launches0
     else:
-        ms, reps = timed_blocks(lambda k: env.rollout_into(actions, k, obs, rew, done), args.steps, barrier, dev)
-        launches = args.steps * reps            # one kernel per step (the estimate / priming blocks are outside the region)
+        ms, _ = timed_blocks(lambda k: env.rollout_into(actions, k, obs, rew, done), args.steps, barrier, dev, reps=1)
+        launches = env.launch_count - launches0 - args.steps   # the K-step priming block is outside the region
     t_region1 = time.perf_counter()
-    per_launch_s = ms * 1e-3 / (args.steps * reps)
+    per_launch_s = ms * 1e-3 / args.steps
     value = n_total / per_launch_s
+    if args.dump_outputs and rank == 0:
+        last = (args.steps - 1) % OUT_RING
+        dump_outputs(args.dump_outputs, {"obs": obs[last], "reward": rew[last], "done": done[last]})
 
     # ---- end to end through the public API with host buffers
     e2e_steps = args.steps if args.e2e_steps is None else args.e2e_steps
@@ -727,25 +760,13 @@ def run_ours(args):
     host_actions = [(torch.rand((n, 3), dtype=torch.float32) * 2 - 1).pin_memory() for _ in range(4)]
     for k in range(3):
         train.step(host_actions[k % 4])
-    # like `value`: the K-step block is repeated inside ONE timed region until it is >= MIN_REGION_S long (a 20-step block is
-    # 25 ms of wall clock: page-fault and scheduler noise of that size showed up as 0.78-0.91 of the PCIe ceiling run to run);
-    # the repetition count comes from an untimed pilot block and is the same on every rank
-    e2e_reps = 1
-    if not args.profile:
-        barrier()
-        t0 = time.perf_counter()
-        for k in range(e2e_steps):
-            train.step(host_actions[k % 4])
-        barrier()
-        pilot_s = max_over_ranks(time.perf_counter() - t0, dev)
-        e2e_reps = int(min(64, max(1, -(-MIN_REGION_S // max(pilot_s, 1e-6)))))
     barrier()
     t0 = time.perf_counter()
-    for k in range(e2e_steps * e2e_reps):
+    for k in range(e2e_steps):
         ho, hr, hd, hinfo = train.step(host_actions[k % 4])   # numpy views of pinned result buffers
     barrier()
     e2e_s = max_over_ranks(time.perf_counter() - t0, dev)
-    e2e_value = n_total * e2e_steps * e2e_reps / e2e_s
+    e2e_value = n_total * e2e_steps / e2e_s
     h2d = n * 3 * 4
     d2h = n * (12 * 4 + 4 + 1 + 1)
     ceiling = None
@@ -795,7 +816,7 @@ def run_ours(args):
             pt["frac"] = pt["achieved"] / peak
         achieved = ALG_BYTES_PER_ENV_STEP * n / per_launch_s / 1e9
         traffic, traffic_src = (args.traffic_bytes, "--traffic-bytes") if args.traffic_bytes is not None else ncu_traffic(n)
-        line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "reps": reps,
+        line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
                 "warmup": args.warmup, "ms_per_step": per_launch_s * 1e3, "timed_region_s": ms * 1e-3,
                 "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "f64", "state_dtype": "float32",
@@ -804,7 +825,7 @@ def run_ours(args):
                               "and is bit-exact over whole rollouts",
                 "data": "synthetic", "config": config_dict(args, n_total),
                 "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d * world,
-                        "d2h_bytes_per_step": d2h * world, "steps": e2e_steps, "reps": e2e_reps,
+                        "d2h_bytes_per_step": d2h * world, "steps": e2e_steps,
                         "api": "PersistentStateWrapper.step(pinned host actions) -> host obs/reward/done/success (earl_step_host: " + host_path_note() + ")",
                         "pcie_ceiling": ceiling,
                         "frac_of_pcie_ceiling": (e2e_value / ceiling["value"]) if ceiling else None},
@@ -856,7 +877,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of the device-resident run (and of e2e by default)")
     ap.add_argument("--warmup", type=int, default=100)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--num-envs", type=int, default=1 << 20, help="envs per GPU")
@@ -868,7 +889,14 @@ def main():
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch of the step kernel; default: looked up by batch size in "
                          "profiles/ncu_traffic.json (committed `ncu --set full` captures), else null")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the observations, rewards and dones of the last timed step (rank 0's "
+                         "envs) as DIR/{obs,reward,done}.npy, float32; a seeded sample of envs beyond 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:

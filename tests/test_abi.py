@@ -1,8 +1,10 @@
 """The C-ABI library loads on a CPU-only box and exports every symbol include/earl_b200.h declares."""
 import ctypes
+import functools
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -46,10 +48,24 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_lib.MjTask) == 8 * 4 + 8 * 4 + 6 * 4 + 7 * 4
 
 
+def without_gpu(test):
+    """Run `test` where no GPU is visible: in this process on a machine without one, else in a child pytest that is shown
+    none (CUDA_VISIBLE_DEVICES empty), so the no-fallback checks run on GPU machines too."""
+    @functools.wraps(test)
+    def run():
+        import torch
+        if not torch.cuda.is_available():
+            return test()
+        r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", f"{os.path.abspath(__file__)}::{test.__name__}"],
+                           cwd=REPO, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stdout[-4000:] + r.stderr[-4000:]
+    return run
+
+
+@without_gpu
 def test_no_cpu_fallback_without_gpu():
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is visible")
+    assert not torch.cuda.is_available()
     import earl_benchmark_b200 as e
     tr, _ = e.EARLEnvs("tabletop_manipulation", num_envs=4).get_envs()
     with pytest.raises(_lib.EarlError) as ei:
@@ -57,10 +73,10 @@ def test_no_cpu_fallback_without_gpu():
     assert ei.value.code == -2  # EARL_ERR_CUDA: fails loudly, no silent CPU path
 
 
+@without_gpu
 def test_kitchen_has_no_cpu_fallback_either():
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is visible")
+    assert not torch.cuda.is_available()
     import numpy as np
     from earl_benchmark_b200.envs import kitchen
     env = kitchen.Kitchen(num_envs=2)           # construction is lazy: host constants only
@@ -107,6 +123,7 @@ def test_sqrt_free_thresholds_are_exact():
     assert np.array_equal(np.sqrt(ys).astype(np.float64) <= 0.2, ys <= y)
 
 
+@without_gpu
 def test_three_object_tabletop_has_no_cpu_fallback_and_validates_its_config():
     import torch
     L = _lib.lib()
@@ -119,8 +136,7 @@ def test_three_object_tabletop_has_no_cpu_fallback_and_validates_its_config():
     cfg.num_goals, cfg.flags = 1, _lib.FLAG_LIFELONG
     assert L.earl_tt3_create(ctypes.byref(cfg), ctypes.sizeof(cfg), ctypes.byref(h)) == -4          # unsupported flag
     assert b"three-object" in L.earl_last_error()
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is visible")
+    assert not torch.cuda.is_available()
     from earl_benchmark_b200.envs.tabletop_manipulation_3obj import TabletopManipulation
     from earl_benchmark_b200.wrappers.persistent_state_wrapper import PersistentStateWrapper
     env = PersistentStateWrapper(TabletopManipulation(reward_type="sparse", num_envs=4), 100)

@@ -39,6 +39,29 @@ def test_engine_sections_cite_their_own_committed_ncu_capture():
     assert k is not None and "kitchen" in k["source"] and k["registers_per_thread"] == 246 and 12 < k["achieved_occupancy_pct"] <= 12.6
 
 
+def test_dump_outputs_writes_float32_and_a_fixed_sample_beyond_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    obs = torch.arange(40 * 12, dtype=torch.float32).reshape(40, 12)
+    done = (torch.arange(40) % 3 == 0).to(torch.uint8)
+    bench.dump_outputs(str(tmp_path / "all"), {"obs": obs, "done": done})
+    assert sorted(os.listdir(tmp_path / "all")) == ["done.npy", "obs.npy"]
+    o, d = np.load(tmp_path / "all" / "obs.npy"), np.load(tmp_path / "all" / "done.npy")
+    assert o.dtype == d.dtype == np.float32 and np.array_equal(o, obs.numpy()) and np.array_equal(d, done.float().numpy())
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 10 * (13 * 4 + 8) + 3 * bench.NPY_HEADER_BYTES)
+    for run in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / run), {"obs": obs, "done": done})
+    idx = np.load(tmp_path / "s1" / "env_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 10 and np.all(np.diff(idx) > 0)
+    rows = idx.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "s1" / "obs.npy"), obs.numpy()[rows])
+    assert np.array_equal(np.load(tmp_path / "s1" / "done.npy"), done.float().numpy()[rows])
+    assert sum(os.path.getsize(tmp_path / "s1" / f) for f in os.listdir(tmp_path / "s1")) <= bench.DUMP_BYTES
+    for f in os.listdir(tmp_path / "s1"):
+        assert np.array_equal(np.load(tmp_path / "s1" / f), np.load(tmp_path / "s2" / f))
+
+
 def test_bench_names_the_host_data_path_it_measured(monkeypatch):
     import bench
     for k in ("LOCAL_WORLD_SIZE", "WORLD_SIZE", "EARL_TT_HOST_ZEROCOPY"):
