@@ -65,17 +65,8 @@ struct earl_handle {
   int device = 0;
   int sm_count = 0;
   int step_grid = 0;
-  int variant = -1;       // EARL_TT_VARIANT: -1 = auto (LSU kernel up to 3M envs, one-tile-per-CTA kernel above); 5 = tile kernel;
-                          // 0 = LSU kernel; 6/8 = LSU kernel with min 6/8 CTAs per SM; 2/3/4 = TMA pipeline stages
-  bool pdl = true;        // EARL_TT_PDL=0 disables programmatic dependent launch between consecutive steps
-  int host_chunks = 0;    // EARL_TT_HOST_CHUNKS: chunks of the host-buffer pipeline (0 = one per 256k envs, at most 16)
-  bool host_tail = true;  // EARL_TT_HOST_TAIL=0: copy reward / done / success per chunk instead of once per step
-  bool tile_vec = false;  // set around the zero-copy launch: tile kernel with 16-byte vector stores for reward / done / success
-  int host_zerocopy = 1;  // EARL_TT_HOST_ZEROCOPY=0: staged copy pipeline instead of the step kernel reading / writing the pinned host buffers itself
-  int tma_grid = 0;
-  int tma_tile = 256;
-  size_t tma_smem = 0;
-  void (*tma_kernel)(const earl::TabletopParams, int) = nullptr;
+  bool tile_step = false;  // the one-tile-per-CTA kernel runs the step instead of the persistent LSU kernel (see earl_create)
+  int host_zerocopy = 1;   // EARL_TT_HOST_ZEROCOPY=0: staged copy pipeline instead of the step kernel reading / writing the pinned host buffers itself
   int64_t total_steps = 0;
   int64_t launches = 0;
   // owned device memory
@@ -137,34 +128,19 @@ int upload_goal_tables(earl_handle* h) {
   return 0;
 }
 
-// Launch with the programmatic-stream-serialization attribute (PDL) when enabled.
-template <typename K>
-cudaError_t launch_pdl(K kernel, int grid, int block, size_t smem, cudaStream_t s, bool pdl, const earl::TabletopParams& p) {
+// Launch a step kernel with the programmatic-stream-serialization attribute (PDL): it may start while the previous
+// grid in the stream drains, and waits for it in griddepcontrol.wait.
+cudaError_t launch_pdl(void (*kernel)(const earl::TabletopParams), int grid, cudaStream_t s, const earl::TabletopParams& p) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3((unsigned)block);
-  cfg.dynamicSmemBytes = smem;
+  cfg.blockDim = dim3((unsigned)earl::kTTBlock);
   cfg.stream = s;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, p);
-}
-template <typename K>
-cudaError_t launch_pdl(K kernel, int grid, int block, size_t smem, cudaStream_t s, bool pdl, const earl::TabletopParams& p, int tiles) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3((unsigned)block);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, p, tiles);
 }
 
 template <typename K>
@@ -177,8 +153,10 @@ int occupancy_grid(K kernel, int sm_count, int* grid) {
 }
 
 // One step of envs [first, first+count) (whole batch: first=0, count=N).  IO pointers are those of env 0.
+// zero_copy: the outputs are pinned host memory (step_host_zerocopy); the tile kernel writes reward / done / success as
+// 16-byte vectors.  Only for handles on the FAST fp32 path.
 int launch_step_range(earl_handle* h, int first, int count, const float* actions, float* obs, float* reward,
-                      uint8_t* done, uint8_t* success, cudaStream_t s) {
+                      uint8_t* done, uint8_t* success, cudaStream_t s, bool zero_copy = false) {
   earl::TabletopParams p = h->p;
   p.n_total = h->p.n;
   p.n = first + count;
@@ -189,31 +167,9 @@ int launch_step_range(earl_handle* h, int first, int count, const float* actions
   p.success = success;
   const bool fast = fast_path(h);
   p.first = first;
-  const uintptr_t all_ptrs = (uintptr_t)actions | (uintptr_t)obs | (uintptr_t)reward | (uintptr_t)done | (uintptr_t)success;
-  const bool tma = (h->variant == 2 || h->variant == 3 || h->variant == 4) && fast && !f64(h) && !(all_ptrs & 15u);
-  if (tma) {  // whole tiles through the bulk-copy pipeline, ragged tail below
-    const int full_tiles = count / h->tma_tile;
-    if (full_tiles > 0) {
-      const int g = full_tiles < h->tma_grid ? full_tiles : h->tma_grid;
-      CU(launch_pdl(h->tma_kernel, g, h->tma_tile, h->tma_smem, s, h->pdl, p, full_tiles));
-      h->launches += 1;
-    }
-    p.first = first + full_tiles * h->tma_tile;
-    if (p.first >= p.n) return 0;
-  }
   const int tiles = (p.n - p.first + earl::kTTBlock - 1) / earl::kTTBlock;
-  if (h->variant == 5 && fast && !f64(h)) {  // one 256-env tile per CTA (obs rows are 48 B: every tile starts 16-byte aligned)
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)tiles);
-    cfg.blockDim = dim3((unsigned)earl::kTTBlock);
-    cfg.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = h->pdl ? 1 : 0;
-    if (h->tile_vec) CU(cudaLaunchKernelEx(&cfg, earl::tabletop_step_tile_kernel<true>, p));
-    else CU(cudaLaunchKernelEx(&cfg, earl::tabletop_step_tile_kernel<false>, p));
+  if (zero_copy || h->tile_step) {  // one 256-env tile per CTA (obs rows are 48 B: every tile starts 16-byte aligned)
+    CU(launch_pdl(zero_copy ? earl::tabletop_step_tile_kernel<true> : earl::tabletop_step_tile_kernel<false>, tiles, s, p));
     h->launches += 1;
     return 0;
   }
@@ -222,9 +178,7 @@ int launch_step_range(earl_handle* h, int first, int count, const float* actions
     if (fast) earl::tabletop_step_kernel<true, true><<<grid, earl::kTTBlock, 0, s>>>(p);
     else earl::tabletop_step_kernel<true, false><<<grid, earl::kTTBlock, 0, s>>>(p);
   } else {
-    if (fast && h->variant == 8) CU(launch_pdl(earl::tabletop_step_kernel<false, true, 8>, grid, earl::kTTBlock, 0, s, h->pdl, p));
-    else if (fast && h->variant == 6) CU(launch_pdl(earl::tabletop_step_kernel<false, true, 6>, grid, earl::kTTBlock, 0, s, h->pdl, p));
-    else if (fast) CU(launch_pdl(earl::tabletop_step_kernel<false, true>, grid, earl::kTTBlock, 0, s, h->pdl, p));
+    if (fast) CU(launch_pdl(earl::tabletop_step_kernel<false, true>, grid, s, p));
     else earl::tabletop_step_kernel<false, false><<<grid, earl::kTTBlock, 0, s>>>(p);
   }
   CU(cudaGetLastError());
@@ -348,43 +302,11 @@ int earl_create(const earl_config* cfg, const void* model_blob, size_t model_nby
   else rc = fast ? occupancy_grid(earl::tabletop_step_kernel<false, true>, h->sm_count, &h->step_grid)
                  : occupancy_grid(earl::tabletop_step_kernel<false, false>, h->sm_count, &h->step_grid);
   if (rc) { earl_destroy(h); return rc; }
-  if (const char* v = getenv("EARL_TT_VARIANT")) h->variant = atoi(v);
-  // measured on B200 (profiles/round1_variants.md): while the 24 B/env state fits in L2 next to the streams
-  // the LSU kernel wins (more resident warps hide L2 latency); once everything streams from HBM the
-  // bulk-copy pipeline keeps more bytes in flight and wins.
-  if (h->variant < 0) h->variant = cfg->num_envs > 3 * 1024 * 1024 ? 5 : 0;
-  if (const char* v = getenv("EARL_TT_PDL")) h->pdl = atoi(v) != 0;
-  if (const char* v = getenv("EARL_TT_HOST_CHUNKS")) h->host_chunks = atoi(v);
-  if (const char* v = getenv("EARL_TT_HOST_TAIL")) h->host_tail = atoi(v) != 0;
+  // measured on B200 (DESIGN.md section 4): while the 24 B/env state fits in L2 next to the streams the persistent LSU
+  // kernel wins (more resident warps hide L2 latency); once everything streams from HBM (above ~3M envs) the
+  // one-tile-per-CTA kernel does.  It only implements the FAST fp32 step.
+  h->tile_step = fast && !f64(h) && cfg->num_envs > 3 * 1024 * 1024;
   if (const char* v = getenv("EARL_TT_HOST_ZEROCOPY")) h->host_zerocopy = atoi(v);
-  if (fast && !f64(h) && (h->variant == 8 || h->variant == 6)) {
-    rc = h->variant == 8 ? occupancy_grid(earl::tabletop_step_kernel<false, true, 8>, h->sm_count, &h->step_grid)
-                         : occupancy_grid(earl::tabletop_step_kernel<false, true, 6>, h->sm_count, &h->step_grid);
-    if (rc) { earl_destroy(h); return rc; }
-  }
-  if ((h->variant == 2 || h->variant == 3 || h->variant == 4) && fast && !f64(h)) {
-    int per_sm = 0;
-    cudaError_t e2 = cudaSuccess;
-    if (const char* v = getenv("EARL_TT_TILE")) h->tma_tile = atoi(v) == 128 ? 128 : 256;
-    auto setup = [&](auto kernel, size_t smem) {
-      h->tma_smem = smem;
-      h->tma_kernel = kernel;
-      e2 = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e2 == cudaSuccess) e2 = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, h->tma_tile, smem);
-    };
-    if (h->tma_tile == 128) {
-      if (h->variant == 4) setup(earl::tabletop_step_tma_kernel<4, 128>, sizeof(earl::TTStage<128>) * 4);
-      else if (h->variant == 2) setup(earl::tabletop_step_tma_kernel<2, 128>, sizeof(earl::TTStage<128>) * 2);
-      else setup(earl::tabletop_step_tma_kernel<3, 128>, sizeof(earl::TTStage<128>) * 3);
-    } else {
-      if (h->variant == 4) setup(earl::tabletop_step_tma_kernel<4, 256>, sizeof(earl::TTStage<256>) * 4);
-      else if (h->variant == 2) setup(earl::tabletop_step_tma_kernel<2, 256>, sizeof(earl::TTStage<256>) * 2);
-      else setup(earl::tabletop_step_tma_kernel<3, 256>, sizeof(earl::TTStage<256>) * 3);
-    }
-    if (e2 != cudaSuccess) { earl_destroy(h); return fail(EARL_ERR_CUDA, "TMA kernel setup: %s", cudaGetErrorString(e2)); }
-    if (const char* v = getenv("EARL_TT_CTAS_PER_SM")) { int c = atoi(v); if (c >= 1 && c < per_sm) per_sm = c; }
-    h->tma_grid = h->sm_count * (per_sm < 1 ? 1 : per_sm);
-  }
   e = cudaStreamCreateWithFlags(&h->host_stream, cudaStreamNonBlocking);
   if (e != cudaSuccess) { earl_destroy(h); return fail(EARL_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e)); }
   *out = h;
@@ -504,13 +426,7 @@ bool step_host_zerocopy(earl_handle* h, const float* actions_host, float* obs_ho
       if (h->in_stream) CU(cudaStreamWaitEvent(h->in_stream, h->order_ev, 0));
       h->order_pending = false;
     }
-    const int variant = h->variant;
-    h->variant = 5;
-    h->tile_vec = true;
-    const int rc = launch_step_range(h, 0, h->p.n, a, o, r, d, su, so);
-    h->variant = variant;
-    h->tile_vec = false;
-    if (rc) return rc;
+    if (int rc = launch_step_range(h, 0, h->p.n, a, o, r, d, su, so, /*zero_copy=*/true)) return rc;
     h->total_steps += 1;
     CU(cudaStreamSynchronize(so));
     return 0;
@@ -543,13 +459,13 @@ int earl_step_host(earl_handle* h, const float* actions_host, float* obs_host, f
   // Chunked software pipeline over the PCIe link: the host->device copy of chunk c+1 (in_stream) overlaps the
   // kernel and the device->host copies of chunk c (host_stream); the link is full duplex.
   constexpr int kMaxChunks = earl_handle::kMaxChunks;
-  int chunks = h->host_chunks > 0 ? h->host_chunks : (int)(n / (256 * 1024));
+  int chunks = (int)(n / (256 * 1024));
   chunks = chunks < 1 ? 1 : (chunks > kMaxChunks ? kMaxChunks : chunks);
   // the three small outputs (6 B per env) go back in one copy each after the last chunk instead of one per chunk:
   // fewer, larger device->host copies per step: their fixed costs are what separates this path from the link rate
   // (1M envs, env-steps/s: 8 chunks, all outputs per chunk 7.8e8; 8 chunks + tail 8.4e8; 4 chunks + tail 8.8e8; 2 chunks
   // + tail 8.7e8; 16 chunks + tail 7.9e8; one chunk 8.2e8 -- profiles/r01/e2e_sweep_r01.txt)
-  const bool tail = h->host_tail && chunks > 1;
+  const bool tail = chunks > 1;
   // ceil(n / chunks) rounded up to whole 256-env tiles: at most `chunks` iterations (floor could give chunks + 1 and
   // index chunk_ev out of bounds, ADVICE r1); chunk boundaries stay tile- and 16-byte aligned
   const size_t per = (((n + chunks - 1) / chunks + 255) / 256) * 256;

@@ -251,7 +251,6 @@ struct earl_tt3_handle {
   T3Params p{};
   int64_t total_steps = 0;
   int64_t launches = 0;
-  bool pdl = true;
   std::vector<void*> owned;
   float* d_act = nullptr;
   float* d_obs = nullptr;
@@ -304,7 +303,7 @@ int launch_step(earl_tt3_handle* h, int first, int count, const float* actions, 
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = h->pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   CU(cudaLaunchKernelEx(&cfg, tt3_step_kernel, p));
   h->launches += 1;
   return 0;
@@ -367,8 +366,6 @@ int earl_tt3_create(const earl_tt3_config* cfg, size_t cfg_nbytes, earl_tt3_hand
   p.clip = cfg->clip;
   p.success_radius = cfg->success_radius;
   for (int k = 0; k < 8; ++k) p.init_qpos[k] = cfg->initial_state[k];
-  const char* e = getenv("EARL_TT_PDL");
-  h->pdl = !(e && e[0] == '0');
   *out = h;
   return 0;
 }

@@ -64,7 +64,7 @@ struct TabletopParams {
   int n;        // one past the last env this launch touches (chunked host path: first + count)
   int n_total;  // envs of the handle = row stride of goal_stream[R,N]; never changes with the chunk (ADVICE r1: a chunked
                 // launch used `n` as the stride and read other envs' draws)
-  int first;  // first env this launch touches (chunked host path; ragged tail after the TMA kernel); multiple of 32
+  int first;  // first env this launch touches (chunked host path); multiple of 32
               // the launch covers envs [first, n)
   int goal_stream_rows;
   uint32_t features;
@@ -390,148 +390,6 @@ __global__ void __launch_bounds__(kTTBlock, 8) tabletop_step_tile_kernel(const _
     p.done[i] = s_done[t];
     if (p.success) p.success[i] = s_succ[t];
   }
-}
-
-// ------------------------------------------------------------------------------------------ TMA pipeline
-// Same step, restructured around the Blackwell/Hopper bulk-copy engine (cp.async.bulk, SASS UBLKCP):
-// a persistent CTA walks its tiles of kTile envs through an S-stage shared-memory ring.  One elected
-// thread issues three bulk loads per tile (qpos, meta, actions: contiguous 4 KB / 2 KB / 3 KB runs) that
-// complete on an mbarrier, every thread computes its env out of shared memory, the results are laid
-// out in shared memory exactly as they sit in HBM, and the elected thread issues bulk stores
-// (qpos, meta, obs 12 KB, reward, done[, success]).  Bytes in flight are set by the ring depth instead of
-// by occupancy x registers, loads/stores are full-line by construction, and the LSU sees no global
-// traffic at all.  Only whole tiles go through this kernel; a ragged tail (< kTile envs) is finished by
-// tabletop_step_kernel launched on the remainder.
-
-template <int kTile>
-struct alignas(128) TTStage {
-  float4 in_qpos[kTile];
-  uint2 in_meta[kTile];
-  float in_act[kTile * kTTAct];
-  float4 out_qpos[kTile];
-  uint2 out_meta[kTile];
-  float out_obs[kTile * kTTObs];
-  float out_reward[kTile];
-  uint8_t out_done[kTile];
-  uint8_t out_success[kTile];
-};
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* dst_gmem, const void* src_smem, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem), "r"(smem_u32(src_smem)),
-               "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// FAST configuration only: fp32 state, sparse reward, no lifelong / auto-reset / eval-stats.
-template <int STAGES, int kTile>
-__global__ void __launch_bounds__(kTile) tabletop_step_tma_kernel(const TabletopParams p, int num_tiles) {
-  extern __shared__ __align__(128) uint8_t smem_raw[];
-  TTStage<kTile>* st = reinterpret_cast<TTStage<kTile>*>(smem_raw);
-  __shared__ __align__(8) uint64_t full[STAGES];
-  const int tid = threadIdx.x;
-  const bool wide = p.features & kWide;
-  constexpr uint32_t kInBytes = kTile * (16 + 8 + 4 * kTTAct);
-
-  auto issue_loads = [&](int tile, int s) {
-    const size_t e = (size_t)p.first + (size_t)tile * kTile;
-    mbar_expect_tx(&full[s], kInBytes);
-    bulk_g2s(st[s].in_qpos, reinterpret_cast<const float4*>(p.qpos) + e, kTile * 16, &full[s]);
-    bulk_g2s(st[s].in_meta, p.meta + e, kTile * 8, &full[s]);
-    bulk_g2s(st[s].in_act, p.actions + e * kTTAct, kTile * 4 * kTTAct, &full[s]);
-  };
-
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) mbar_init(&full[s], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  pdl_wait_prior_grid();  // barrier setup above overlaps the previous step's tail
-  __syncthreads();
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
-      const int tile = blockIdx.x + s * gridDim.x;
-      if (tile < num_tiles) issue_loads(tile, s);
-    }
-  }
-
-  int it = 0;
-  for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x, ++it) {
-    const int s = it % STAGES;
-    const uint32_t parity = (uint32_t)(it / STAGES) & 1u;
-    mbar_wait(&full[s], parity);
-    TTStage<kTile>& b = st[s];
-
-    TTState sdev;
-    const float4 q = b.in_qpos[tid];
-    const uint2 m = b.in_meta[tid];
-    const float a0 = b.in_act[tid * kTTAct + 0], a1 = b.in_act[tid * kTTAct + 1], a2 = b.in_act[tid * kTTAct + 2];
-    sdev.fx = q.x; sdev.fy = q.y; sdev.mx = q.z; sdev.my = q.w;
-    sdev.flags = m.x;
-    uint32_t steps = m.y;
-    const uint32_t gi = (sdev.flags & kGoalMask) >> kGoalShift;
-    const float4 g0 = __ldg(p.goal32 + 2 * gi);
-    const float4 g1 = __ldg(p.goal32 + 2 * gi + 1);
-    tt_move(sdev, a0, a1, a2, p);
-    const float4 pos32 = make_float4(__double2float_rn(sdev.fx), __double2float_rn(sdev.fy),
-                                     __double2float_rn(sdev.mx), __double2float_rn(sdev.my));
-    const bool succ = tt_success(pos32, g0, wide, p.success_sq);
-    steps = steps == 0xffffffffu ? steps : steps + 1u;
-    const bool done = (unsigned long long)steps >= p.horizon;
-    const float att = (sdev.flags & kAttached) ? 0.f : -1.f;
-
-    b.out_qpos[tid] = pos32;
-    b.out_meta[tid] = make_uint2(sdev.flags, steps);
-    float4* row = reinterpret_cast<float4*>(b.out_obs + tid * kTTObs);
-    row[0] = pos32;
-    row[1] = make_float4(att, att, g0.x, g0.y);
-    row[2] = make_float4(g0.z, g0.w, g1.x, g1.y);
-    b.out_reward[tid] = succ ? 1.f : 0.f;
-    b.out_done[tid] = done ? 1 : 0;
-    b.out_success[tid] = succ ? 1 : 0;
-    fence_proxy_async();  // generic-proxy smem writes -> visible to the bulk-copy (async) proxy
-    // out[] of the stage the NEXT iteration writes must have been drained by its previous bulk stores
-    if (tid == 0) bulk_wait_read<(STAGES >= 2 ? STAGES - 2 : 0)>();
-    __syncthreads();
-    if (tid == 0) {
-      const size_t e = (size_t)p.first + (size_t)tile * kTile;
-      bulk_s2g(reinterpret_cast<float4*>(p.qpos) + e, b.out_qpos, kTile * 16);
-      bulk_s2g(p.meta + e, b.out_meta, kTile * 8);
-      bulk_s2g(p.obs + e * kTTObs, b.out_obs, kTile * 4 * kTTObs);
-      bulk_s2g(p.reward + e, b.out_reward, kTile * 4);
-      bulk_s2g(p.done + e, b.out_done, kTile);
-      if (p.success) bulk_s2g(p.success + e, b.out_success, kTile);
-      bulk_commit();
-      const int next = tile + STAGES * gridDim.x;  // in[] of this stage is free: everyone passed the barrier
-      if (next < num_tiles) issue_loads(next, s);
-    }
-  }
-  if (tid == 0) bulk_wait_all();
 }
 
 // ------------------------------------------------------------------------------------------ cold kernels

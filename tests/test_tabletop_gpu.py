@@ -513,12 +513,11 @@ def test_f32_state_against_the_fp64_reference_over_the_benchmarked_horizon():
 
 # ---------------------------------------------------------------------------------------- round 2: kernel variants, host path
 
-@pytest.mark.parametrize("variant", ["0", "3", "5", "6"])
-@pytest.mark.parametrize("n", [255, 4099, 70001])
-def test_every_step_kernel_variant_vs_oracle(monkeypatch, variant, n):
-    """The persistent LSU kernel (0, 6), the cp.async.bulk pipeline (3) and the one-tile-per-CTA kernel (5, the default above
-    3M envs) are the same arithmetic: ragged batches, attach / drag / clip, horizon `done`, host path included -- bit-exact."""
-    monkeypatch.setenv("EARL_TT_VARIANT", variant)
+@pytest.mark.parametrize("n", [255, 4099, 70001, 3 * 2**20 + 4099])
+def test_selected_step_kernels_vs_oracle(n):
+    """The step kernel the library selects for the batch size -- the persistent LSU kernel up to 3M envs, the one-tile-per-CTA
+    kernel above (3 * 2**20 + 4099 envs: a ragged last tile of 3 envs) -- against the oracle: ragged batches, attach / drag /
+    clip, horizon `done`, host path included -- bit-exact."""
     steps, horizon = 24, 17
     env = make(n, horizon, seed=n)
     orc = TabletopOracle(n, horizon, state_f32=True)
@@ -543,12 +542,11 @@ def test_every_step_kernel_variant_vs_oracle(monkeypatch, variant, n):
 
 
 @pytest.mark.parametrize("mode", ["lifelong", "auto_reset"])
-def test_chunked_host_path_reads_its_own_goal_stream(monkeypatch, mode):
+def test_chunked_host_path_reads_its_own_goal_stream(mode):
     """ADVICE r1 (medium): a chunked host step used the chunk's end as the row stride of goal_stream[R, N], so every chunk but
     the last read other envs' draws once a goal was drawn inside the step (lifelong swap, auto-reset).  Host path with 4
     chunks == device path, with goals actually changing."""
-    monkeypatch.setenv("EARL_TT_HOST_CHUNKS", "4")
-    n, steps = 2051, 40
+    n, steps = 4 * 2**18 + 2051, 40                                     # one chunk per 256k envs: 4 chunks
     if mode == "lifelong":
         kw = dict(setup_as_lifelong_learning=True, goal_change_frequency=7, train_horizon=10**6)
     else:
@@ -560,11 +558,13 @@ def test_chunked_host_path_reads_its_own_goal_stream(monkeypatch, mode):
     assert np.array_equal(oa, ob_)
     acts = actions(n, steps, seed=21, grip_bias=0.2)
     goals = set()
+    launches = b.launch_count
     for t in range(steps):
         o, r, d, _ = a.step(torch.from_numpy(acts[t]).to(DEV))
         ho, hr, hd, _ = b.step(acts[t])
         assert np.array_equal(ho, np_(o)) and np.array_equal(hr, np_(r)) and np.array_equal(hd, np_(d)), t
         goals |= set(map(tuple, np.unique(ho[:, 8:10], axis=0)))
+    assert b.launch_count - launches == 4 * steps                       # one step kernel per chunk: the batch ran in 4 chunks
     assert len(goals) == 4                                              # all four goals were drawn along the way
 
 
@@ -627,7 +627,7 @@ def test_lifelong_goal_stream_covers_the_horizon():
     assert base._goal_stream.shape[0] >= 127
 
 
-@pytest.mark.parametrize("n", [2051, 300000])
+@pytest.mark.parametrize("n", [2051, 3 * 2**20 + 2051])               # the latter: 12 chunks of the copy pipeline
 def test_zero_copy_host_step_equals_the_copy_pipeline_and_the_device_path(monkeypatch, n):
     """EARL_TT_HOST_ZEROCOPY=1: the one-tile-per-CTA step kernel reads the pinned host actions and writes the pinned host
     outputs itself (no staging copies).  Same observations, rewards, done / success flags and state as the chunked copy
