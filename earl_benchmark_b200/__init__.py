@@ -3,7 +3,8 @@
 `EARLEnvs` keeps the surface of the reference loader (`earl_benchmark/__init__.py:83-247`):
     EARLEnvs(env_name, reward_type, reset_train_env_at_goal, setup_as_lifelong_learning, **kwargs)
         .get_envs() / .get_initial_states() / .get_goal_states() / .get_demonstrations() / .has_demos()
-and adds the batched arguments `num_envs`, `device`, `seed`, `state_dtype`, `auto_reset`, `eval_stats`,
+and adds the batched arguments `num_envs`, `device`, `seed`, `state_dtype`, `auto_reset` (with `reset_stream_rows` for
+sawyer_door, sawyer_peg and kitchen), `eval_stats`,
 `rank` / `world_size` (shard a global batch of `num_envs` across processes, one GPU each).
 """
 from . import demos
@@ -79,6 +80,11 @@ class EARLEnvs(object):
         b.update(num_envs=self._hi - self._lo, env_offset=self._lo, total_envs=self._num_envs)
         return b
 
+    def _auto_reset_kwargs(self):
+        """train envs of the articulated-body tasks: reset in the step when the horizon fires (eval envs never do)"""
+        return dict(auto_reset=bool(self._kwargs.get('auto_reset', False)),
+                    reset_stream_rows=int(self._kwargs.get('reset_stream_rows', 64)))
+
     def _not_built(self):
         raise NotImplementedError(
             f"{self._env_name}: the batched CUDA step for this task is not built yet "
@@ -99,16 +105,17 @@ class EARLEnvs(object):
             from .envs import sawyer_door
             train_env = sawyer_door.SawyerDoorV2(reward_type=self._reward_type,
                                                  reset_at_goal=self._reset_train_env_at_goal,
-                                                 eval_stats=False, **self._shard_kwargs(0))
+                                                 eval_stats=False, **self._auto_reset_kwargs(), **self._shard_kwargs(0))
         elif self._env_name == 'sawyer_peg':
             from .envs import sawyer_peg
             train_env = sawyer_peg.SawyerPegV2(reward_type=self._reward_type,
                                                reset_at_goal=self._reset_train_env_at_goal,
-                                               eval_stats=False, **self._shard_kwargs(0))
+                                               eval_stats=False, **self._auto_reset_kwargs(), **self._shard_kwargs(0))
         elif self._env_name == 'kitchen':
             from .envs import kitchen
             kitchen_task = self._kwargs.get('kitchen_task', deployment_eval_config[self._env_name]['task'])
-            train_env = kitchen.Kitchen(task=kitchen_task, reward_type=self._reward_type, **self._shard_kwargs(0))
+            train_env = kitchen.Kitchen(task=kitchen_task, reward_type=self._reward_type, **self._auto_reset_kwargs(),
+                                        **self._shard_kwargs(0))
         else:
             deployment_eval_config[self._env_name]  # KeyError for unknown names
             self._not_built()

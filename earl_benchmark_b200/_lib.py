@@ -92,6 +92,7 @@ SIGNATURES = [
     ("earl_rng_tabletop_goal_rows", None, [_VP, _VP, _U32, _I64, _VP]),
     ("earl_rng_np_randint", None, [_VP, _U32, _I64, _VP]),
     ("earl_rng_np_uniform", None, [_VP, C.c_double, C.c_double, _I64, _VP]),
+    ("earl_rng_peg_reset_draws", None, [_VP, _I32, _I32, _I64, _VP, _VP]),
     # include/earl_tt3_b200.h: three-object tabletop
     ("earl_tt3_create", C.c_int, [C.POINTER(Tt3Config), _SZ, C.POINTER(_VP)]),
     ("earl_tt3_destroy", C.c_int, [_VP]),
@@ -115,6 +116,7 @@ SIGNATURES = [
     ("earl_mj_nv", C.c_int, [_VP]),
     ("earl_mj_set_goal_table", C.c_int, [_VP, _VP, _I32]),
     ("earl_mj_build_reset_template", C.c_int, [_VP, _VP, _VP, _I32]),
+    ("earl_mj_set_reset_stream", C.c_int, [_VP, _VP, _VP, _I32, _VP]),
     ("earl_mj_reset", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mj_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mj_step_host", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
@@ -134,6 +136,7 @@ SIGNATURES = [
     ("earl_mjk_create", C.c_int, [_VP, _VP, _SZ, C.POINTER(_VP)]),
     ("earl_mjk_destroy", C.c_int, [_VP]),
     ("earl_mjk_seed", C.c_int, [_VP, _VP]),
+    ("earl_mjk_set_reset_stream", C.c_int, [_VP, _VP, _I32, _VP, _I32]),
     ("earl_mjk_reset", C.c_int, [_VP, _VP, C.c_int32, _VP, _VP, _VP]),
     ("earl_mjk_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mjk_get_state", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),

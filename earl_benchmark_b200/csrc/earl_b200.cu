@@ -686,4 +686,53 @@ void earl_rng_np_uniform(earl_rng* r, double low, double high, int64_t count, do
   for (int64_t k = 0; k < count; ++k) out[k] = low + (high - low) * r->mt.np_double();
 }
 
+// Replays envs/sawyer_peg.py SawyerPegV2._draw_one (reference sawyer_peg.py:144-152,192-229) with the same double operations
+// in the same order, so the results are bit-identical with the numpy arithmetic there.
+void earl_rng_peg_reset_draws(earl_rng* r, int32_t wide_init, int32_t reset_at_goal, int64_t count, int32_t* rows_out, double* pos_out) {
+  // _random_reset_space = (obj_low, goal_low) .. (obj_high, goal_high), sawyer_peg.py:64-69,102-105
+  static const double lo[6] = {0.0, 0.5, 0.02, -0.35, 0.4, -0.001}, hi[6] = {0.2, 0.7, 0.02, -0.25, 0.7, 0.001};
+  // wide_initial_states (sawyer_peg.py:50-58)
+  static const double wide[22][3] = {{-0.3, 0.8, 0.02}, {-0.4, 0.8, 0.02}, {-0.3, 0.9, 0.02}, {-0.4, 0.9, 0.02}, {-0.2, 0.8, 0.02},
+                                     {-0.2, 0.75, 0.02}, {-0.2, 0.9, 0.02}, {-0.1, 0.77, 0.02}, {0.0, 0.9, 0.02}, {0.1, 0.8, 0.02},
+                                     {0.15, 0.75, 0.02}, {-0.3, 0.4, 0.02}, {-0.4, 0.4, 0.02}, {-0.3, 0.45, 0.02}, {-0.4, 0.45, 0.02},
+                                     {-0.2, 0.4, 0.02}, {-0.2, 0.45, 0.02}, {-0.2, 0.38, 0.02}, {-0.1, 0.42, 0.02}, {0.0, 0.45, 0.02},
+                                     {0.1, 0.36, 0.02}, {0.15, 0.44, 0.02}};
+  const double goal[3] = {-0.3 + 0.03, 0.6, 0.0 + 0.13};                   // goal_states[0][4:] (sawyer_peg.py:46)
+  const double box[2] = {goal[0] - 0.03, goal[1] - 0.0};                    // pos_box[:2] = goal[4:] - (0.03, 0, 0.13)
+  earl::MT19937& mt = r->mt;
+  auto uniform = [&](double l, double h) { return l + (h - l) * mt.np_double(); };
+  auto sample_peg = [&](double* p) {  // _get_state_rand_vec()[:3], redrawn while ||p[:2] - box|| < 0.1
+    for (;;) {
+      double u[6];
+      for (int k = 0; k < 6; ++k) u[k] = uniform(0.0, 1.0);
+      for (int k = 0; k < 3; ++k) p[k] = lo[k] + (hi[k] - lo[k]) * u[k];
+      const double dx = p[0] - box[0], dy = p[1] - box[1];
+      if (!(std::sqrt(dx * dx + dy * dy) < 0.1)) return;
+    }
+  };
+  for (int64_t i = 0; i < count; ++i) {
+    double* p = pos_out + 3 * i;
+    int row = 0;
+    if (!reset_at_goal) {
+      mt.np_randint(1);  // get_next_goal() over one goal: consumes nothing
+      if (wide_init) {
+        if (uniform(0.0, 1.0) < 0.5) {
+          sample_peg(p);
+        } else {
+          const uint32_t k = mt.np_randint(22);
+          const double base[3] = {wide[k][0] - -0.1, wide[k][1] - 0.0, wide[k][2] - 0.0};
+          for (int c = 0; c < 3; ++c) p[c] = base[c] + uniform(-0.02, 0.02);
+        }
+      } else {
+        sample_peg(p);  // random_init
+      }
+    } else {
+      row = 1 + (int)mt.np_randint(15);
+      const double base[3] = {goal[0] - -0.1, goal[1] - 0.0, goal[2] - 0.0};
+      for (int c = 0; c < 3; ++c) p[c] = base[c] + uniform(-0.02, 0.02);
+    }
+    rows_out[i] = row;
+  }
+}
+
 }  // extern "C"

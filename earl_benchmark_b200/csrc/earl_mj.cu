@@ -36,6 +36,8 @@ int earl_mjs_set_goal_table(void* h, const double* rows_host, int32_t count);
 int earl_mjl_set_goal_table(void* h, const double* rows_host, int32_t count);
 int earl_mjs_build_reset_template(void* h, const double* hand_init_pos_host, const float* ctrl_host, int32_t steps);
 int earl_mjl_build_reset_template(void* h, const double* hand_init_pos_host, const float* ctrl_host, int32_t steps);
+int earl_mjs_set_reset_stream(void* h, const double* obj_qpos_host, const int32_t* goal_rows_host, int32_t rows, int32_t* goal_rows_dev);
+int earl_mjl_set_reset_stream(void* h, const double* obj_qpos_host, const int32_t* goal_rows_host, int32_t rows, int32_t* goal_rows_dev);
 int earl_mjs_reset(void* h, const uint8_t* mask_dev, const double* obj_qpos_dev, const int32_t* goal_idx_dev, float* obs_out_dev, void* stream);
 int earl_mjl_reset(void* h, const uint8_t* mask_dev, const double* obj_qpos_dev, const int32_t* goal_idx_dev, float* obs_out_dev, void* stream);
 int earl_mjs_step(void* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev, uint8_t* success_dev, void* stream);
@@ -115,6 +117,11 @@ int earl_mj_set_goal_table(earl_mj_handle* h, const double* rows_host, int32_t c
 int earl_mj_build_reset_template(earl_mj_handle* h, const double* hand_init_pos_host, const float* ctrl_host, int32_t steps) {
   if (!h) return earl::set_error(EARL_ERR_INVALID, "null handle");
   return h->set ? earl_mjl_build_reset_template(h->impl, hand_init_pos_host, ctrl_host, steps) : earl_mjs_build_reset_template(h->impl, hand_init_pos_host, ctrl_host, steps);
+}
+
+int earl_mj_set_reset_stream(earl_mj_handle* h, const double* obj_qpos_host, const int32_t* goal_rows_host, int32_t rows, int32_t* goal_rows_dev) {
+  if (!h) return earl::set_error(EARL_ERR_INVALID, "null handle");
+  return h->set ? earl_mjl_set_reset_stream(h->impl, obj_qpos_host, goal_rows_host, rows, goal_rows_dev) : earl_mjs_set_reset_stream(h->impl, obj_qpos_host, goal_rows_host, rows, goal_rows_dev);
 }
 
 int earl_mj_reset(earl_mj_handle* h, const uint8_t* mask_dev, const double* obj_qpos_dev, const int32_t* goal_idx_dev, float* obs_out_dev, void* stream) {

@@ -154,6 +154,12 @@ struct TaskArgs {
   // kernel at the START of its next step (heavy envs lead the visiting order), so that its latency overlaps the step kernel
   unsigned char* heavy;             // [N]
   int prim_efc, prim_con, prim_hit;
+  // pre-drawn reset stream (EARL_FLAG_AUTO_RESET): draw e of env i is configuration ring_config[e * n + i], a row of
+  // ring_table [K,14] (object qpos), e = ring_cursor[i] mod ring_rows
+  const unsigned char* ring_config;
+  const double* ring_table;
+  unsigned* ring_cursor;
+  int ring_rows;
 };
 enum { kRedoCount = 0, kRedoNext = 1, kMainDone = 2, kNextChunk = 3, kSchedWords = 4 };
 
@@ -259,16 +265,20 @@ struct TaskIo {
 };
 
 // One environment of the task kernels, all lanes of its warp.  mode 0: env step, mode 1: reset (slot = row of object_qpos /
-// obs_out), mode 2: env step of the redo pass.  `own` false: the warp only keeps its block's phase barriers company.
+// obs_out; object_qpos null: the env's next draw of the reset stream), mode 2: env step of the redo pass, mode 3: reset
+// from the reset stream after a step (obs row = env).  `own` false: the warp only keeps its block's phase barriers company.
 // Returns false when the step overflowed the capacities and was handed to the redo pass (nothing stored).
 __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const TaskArgs& a, const TaskIo& io, Work& w, int mode, int env,
                                          int slot, bool own, int lane, TaskCounters& c) {
   Pcg g;
   double last_qp[kRobot];
-  const bool stepping = mode != 1;
+  const bool stepping = mode == 0 || mode == 2;
+  const bool ring = mode == 3 || (mode == 1 && !io.object_qpos);
   if (!stepping) {  // Kitchen.reset_model: robot.reset (sim.reset, qpos write, forward, 5 cached observations at ratio 1)
+    const double* obj = ring ? a.ring_table + (size_t)kObj * a.ring_config[(size_t)(a.ring_cursor[env] % (unsigned)a.ring_rows) * a.n + env]
+                             : io.object_qpos + (size_t)slot * kObj;
     for (int k = lane; k < kNQ; k += 32) {
-      const double q = k < kRobot ? a.init_qpos[k] : io.object_qpos[(size_t)slot * kObj + (k - kRobot)];
+      const double q = k < kRobot ? a.init_qpos[k] : obj[k - kRobot];
       w.qpos[k] = (real)q; w.qvel[k] = 0; w.warm[k] = 0;
     }
     if (lane == 0) {
@@ -334,7 +344,7 @@ __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const
     for (int k = 0; k < kRobot; ++k) a.last_qp[(size_t)env * kRobot + k] = last_qp[k];
     unsigned long long* r = a.rng + (size_t)env * 4;
     r[0] = (unsigned long long)(g.state >> 64); r[1] = (unsigned long long)g.state;
-    double* orow = io.obs_out ? io.obs_out + (size_t)(stepping ? env : slot) * kObs : nullptr;
+    double* orow = io.obs_out ? io.obs_out + (size_t)(mode == 1 ? slot : env) * kObs : nullptr;
     // estimated warp instructions above the contact-free baseline: loose broad-phase passes (~9k each), extra Newton
     // iterations (~6k), contacts (~1.5k per contact and substep), portal-refinement support calls (~0.3k)
     a.cost[env] = 9000 * w.acc_rebuild + 6000 * (w.acc_iter - a.frame_skip) + 1500 * w.acc_con + 300 * w.acc_sup;
@@ -373,6 +383,7 @@ __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const
       a.steps_since_goal_change[env] = 0;               // LifelongWrapper.reset (:25-28)
       a.num_interventions[env] += 1;
       a.heavy[env] = 0;
+      if (ring) a.ring_cursor[env] += 1;
     }
     c.it += w.acc_iter; c.rows += w.acc_rows; c.con += w.acc_con; c.bad += (w.bad & 1) ? 1 : 0; c.over += (w.bad & 14) ? 1 : 0; c.env += 1;
     c.ov_hit += (w.bad & 2) ? 1 : 0; c.ov_con += (w.bad & 4) ? 1 : 0; c.ov_row += (w.bad & 8) ? 1 : 0;
@@ -383,8 +394,9 @@ __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const
 
 __device__ __forceinline__ void task_flush(const TaskArgs& a, const TaskCounters& c, int mode, int lane) {
   if (lane == 0 && c.env) {
-    atomicAdd(&a.work[0], mode != 1 ? c.env : 0ULL);
-    atomicAdd(&a.work[1], c.env * (unsigned long long)(mode == 1 ? 10 * a.frame_skip : a.frame_skip));
+    const bool resetting = mode == 1 || mode == 3;
+    atomicAdd(&a.work[0], resetting ? 0ULL : c.env);
+    atomicAdd(&a.work[1], c.env * (unsigned long long)(resetting ? 10 * a.frame_skip : a.frame_skip));
     atomicAdd(&a.work[2], c.it); atomicAdd(&a.work[3], c.rows); atomicAdd(&a.work[4], c.con);
     atomicAdd(&a.work[5], c.bad); atomicAdd(&a.work[6], c.over); atomicAdd(&a.work[7], c.redone);
     atomicAdd(&a.work[8], c.ov_hit); atomicAdd(&a.work[9], c.ov_con); atomicAdd(&a.work[10], c.ov_row);
@@ -392,7 +404,8 @@ __device__ __forceinline__ void task_flush(const TaskArgs& a, const TaskCounters
 }
 
 #ifndef MJK_XL
-// mode 0: one env step of every environment.  mode 1: reset of the environments in env_ids.
+// mode 0: one env step of every environment.  mode 1: reset of the environments in env_ids.  mode 3: reset of every
+// environment whose io.done_out (read here: the done array of the step just taken) is set, from the reset stream.
 __global__ void __launch_bounds__(kWPB * 32, kBPS)
 mjk_task_kernel(const Model* __restrict__ gm, const real* __restrict__ hull, const TaskArgs a, int mode, const int* env_ids, int count,
                 const TaskIo io) {
@@ -401,6 +414,20 @@ mjk_task_kernel(const Model* __restrict__ gm, const real* __restrict__ hull, con
   Work& w = *reinterpret_cast<Work*>(smem + warp * kWorkStride);
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // lets the concurrent redo kernel start (no-op otherwise)
   TaskCounters c;
+  if (mode == 3) {
+    // static stride over chunks of kWPB consecutive envs; a chunk without a done env is left at once, in one with some the
+    // other warps shadow a reset they do not store (the phase barriers are block-wide)
+    for (int base = blockIdx.x * kWPB; base < count; base += gridDim.x * kWPB) {
+      const bool in = base + warp < count;
+      const int env = in ? base + warp : count - 1;
+      const bool own = in && io.done_out[env];
+      if (!__syncthreads_or(own)) continue;
+      task_env(*gm, hull, a, io, w, 3, env, env, own, lane, c);
+      __syncthreads();
+    }
+    task_flush(a, c, 3, lane);
+    return;
+  }
   // Step: chunks of kWPB consecutive entries of the cost-sorted order are handed out dynamically (a block that draws expensive
   // chunks takes fewer of them).  Reset: static stride.
   __shared__ int s_chunk;
@@ -666,6 +693,7 @@ struct earl_mjk_handle {
   int bucket_width = 60000;  // flat between 40k and 160k (measured); EARL_MJK_BUCKET_WIDTH overrides
   bool redo_sms_fixed = false;      // EARL_MJ_REDO_SMS given: no adaptation
   unsigned* h_redo_seen = nullptr;  // pinned: redo-list length of a recent step (async copy, read without waiting)
+  int ring_configs = 0;             // rows of the reset stream's configuration table
   int redo_sms = 4;          // SMs the step kernel leaves to the concurrent redo kernel (EARL_MJ_REDO_SMS; measured 2: 1.49e5, 4: 1.54e5, 6: 1.53e5)
   std::vector<void*> owned;
   template <typename T>
@@ -725,6 +753,7 @@ int earl_mjk_create(const earl_mjk_config* cfg, const void* model_blob, size_t m
   if (!cfg || !model_blob || !out) return failf(EARL_ERR_INVALID, "null argument");
   *out = nullptr;
   if (cfg->num_envs <= 0 || cfg->frame_skip <= 0 || cfg->episode_horizon <= 0) return failf(EARL_ERR_INVALID, "bad kitchen config");
+  if (cfg->flags & ~(uint32_t)(EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET)) return failf(EARL_ERR_UNSUPPORTED, "unsupported flags %#x", cfg->flags);
   earl_mjk_engine* eng = nullptr;
   if (int rc = earl_mjk_engine_create(model_blob, model_nbytes, cfg->device, &eng)) return rc;
   earl_mjk_handle* h = new (std::nothrow) earl_mjk_handle();
@@ -787,9 +816,37 @@ int earl_mjk_seed(earl_mjk_handle* h, const uint64_t* pcg_state_host) {
   return 0;
 }
 
+int earl_mjk_set_reset_stream(earl_mjk_handle* h, const uint8_t* config_host, int32_t rows, const double* table_host, int32_t num_configs) {
+  if (!h || !config_host || !table_host) return failf(EARL_ERR_INVALID, "null argument");
+  if (!(h->a.flags & EARL_FLAG_AUTO_RESET)) return failf(EARL_ERR_INVALID, "the reset stream belongs to EARL_FLAG_AUTO_RESET handles");
+  if (rows < 1 || num_configs < 1 || num_configs > 256) return failf(EARL_ERR_INVALID, "bad reset stream shape (%d rows, %d configurations)", rows, num_configs);
+  if (h->a.ring_rows && (h->a.ring_rows != rows || h->ring_configs != num_configs))
+    return failf(EARL_ERR_INVALID, "reset stream already has %d rows of %d configurations", h->a.ring_rows, h->ring_configs);
+  const size_t n = (size_t)h->a.n, cells = (size_t)rows * n;
+  for (size_t k = 0; k < cells; ++k)
+    if (config_host[k] >= num_configs) return failf(EARL_ERR_INVALID, "configuration %d out of range", (int)config_host[k]);
+  CU(cudaSetDevice(h->eng->device));
+  TaskArgs& a = h->a;
+  if (!a.ring_rows) {
+    int rc = h->alloc(const_cast<unsigned char**>(&a.ring_config), cells);
+    if (!rc) rc = h->alloc(const_cast<double**>(&a.ring_table), (size_t)num_configs * kObj);
+    if (!rc) rc = h->alloc(&a.ring_cursor, n);
+    if (rc) return rc;
+    a.ring_rows = rows;
+    h->ring_configs = num_configs;
+  }
+  CU(cudaDeviceSynchronize());
+  CU(cudaMemcpy(const_cast<unsigned char*>(a.ring_config), config_host, cells, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(const_cast<double*>(a.ring_table), table_host, (size_t)num_configs * kObj * sizeof(double), cudaMemcpyHostToDevice));
+  CU(cudaMemset(a.ring_cursor, 0, n * sizeof(unsigned)));
+  return 0;
+}
+
 int earl_mjk_reset(earl_mjk_handle* h, const int32_t* env_ids_dev, int32_t count, const double* object_qpos_dev, double* obs_out_dev,
                    void* stream) {
-  if (!h || !object_qpos_dev) return failf(EARL_ERR_INVALID, "null argument");
+  if (!h) return failf(EARL_ERR_INVALID, "null argument");
+  if (!object_qpos_dev && !h->a.ring_rows)
+    return failf(EARL_ERR_INVALID, "object_qpos is required (NULL draws from the reset stream of an auto-reset handle, which has none yet)");
   if (!h->seeded) return failf(EARL_ERR_INVALID, "earl_mjk_seed must be called before the first reset (the observation noise stream)");
   if (!env_ids_dev) count = h->a.n;
   if (count <= 0 || count > h->a.n) return failf(EARL_ERR_INVALID, "bad env count %d", count);
@@ -801,6 +858,7 @@ int earl_mjk_reset(earl_mjk_handle* h, const int32_t* env_ids_dev, int32_t count
 int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev, double* reward_dev, uint8_t* done_dev, uint8_t* success_dev,
                   void* stream) {
   if (!h || !actions_dev || !obs_dev || !reward_dev || !done_dev) return failf(EARL_ERR_INVALID, "null argument");
+  if ((h->a.flags & EARL_FLAG_AUTO_RESET) && !h->a.ring_rows) return failf(EARL_ERR_INVALID, "auto-reset handles need earl_mjk_set_reset_stream before the first step");
   CU(cudaSetDevice(h->eng->device));
   h->a.mocap_quat = make_float4(h->eng->mocap_quat[0], h->eng->mocap_quat[1], h->eng->mocap_quat[2], h->eng->mocap_quat[3]);
   h->total_steps += 1;
@@ -811,6 +869,9 @@ int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev,
   mjk_order_kernel<<<64, 256, 0, s>>>(h->d_bucket, h->d_rank, h->a.n, h->d_counts, h->d_order);
   CU(cudaGetLastError());
   if (h->h_redo_seen && h->a.redo_list) CU(cudaMemcpyAsync(h->h_redo_seen, h->a.sched + kRedoCount, sizeof(unsigned), cudaMemcpyDeviceToHost, s));
+  // auto reset: the envs whose horizon fired in this step, after the step, redo, bucket and order kernels (plain launch)
+  if (h->a.flags & EARL_FLAG_AUTO_RESET)
+    if (int rc = launch_task(h, 3, nullptr, h->a.n, nullptr, nullptr, obs_dev, nullptr, done_dev, nullptr, stream)) return rc;
   return 0;
 }
 

@@ -10,6 +10,7 @@
 #define earl_mj_nv earl_mjl_nv
 #define earl_mj_set_goal_table earl_mjl_set_goal_table
 #define earl_mj_build_reset_template earl_mjl_build_reset_template
+#define earl_mj_set_reset_stream earl_mjl_set_reset_stream
 #define earl_mj_reset earl_mjl_reset
 #define earl_mj_step earl_mjl_step
 #define earl_mj_step_host earl_mjl_step_host

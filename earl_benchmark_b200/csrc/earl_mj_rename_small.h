@@ -10,6 +10,7 @@
 #define earl_mj_nv earl_mjs_nv
 #define earl_mj_set_goal_table earl_mjs_set_goal_table
 #define earl_mj_build_reset_template earl_mjs_build_reset_template
+#define earl_mj_set_reset_stream earl_mjs_set_reset_stream
 #define earl_mj_reset earl_mjs_reset
 #define earl_mj_step earl_mjs_step
 #define earl_mj_step_host earl_mjs_step_host

@@ -10,6 +10,7 @@
 #define earl_mj_nv earl_mjx_nv
 #define earl_mj_set_goal_table earl_mjx_set_goal_table
 #define earl_mj_build_reset_template earl_mjx_build_reset_template
+#define earl_mj_set_reset_stream earl_mjx_set_reset_stream
 #define earl_mj_reset earl_mjx_reset
 #define earl_mj_step earl_mjx_step
 #define earl_mj_step_host earl_mjx_step_host

@@ -34,7 +34,8 @@ class SawyerBatchedEnv:
     HAS_DENSE_REWARD = False
 
     def __init__(self, reward_type="sparse", reset_at_goal=False, num_envs=1, device=None, seed=0, eval_stats=False,
-                 env_offset=0, total_envs=None, model_path=None, max_newton=0, host_io=False, **_tabletop_only):
+                 env_offset=0, total_envs=None, model_path=None, max_newton=0, host_io=False, auto_reset=False,
+                 reset_stream_rows=64, **_tabletop_only):
         name = type(self).__name__
         if reward_type == "dense" and not self.HAS_DENSE_REWARD:
             raise NotImplementedError(f"{name}: the dense reward (metaworld reward_utils, gripper caging) is not built yet")
@@ -66,6 +67,12 @@ class SawyerBatchedEnv:
         self._obs = self._reward = self._done = self._success = None
         self._host_bufs = None
         self._host_mode = bool(host_io)   # host_io=True: reset() returns numpy like the numpy-driven step()
+        # auto_reset=True: an env whose horizon fires is reset inside step() on the device, and every reset without an
+        # override takes its draws from a pre-drawn stream of `reset_stream_rows` full resets per env (see reset_stream())
+        self._auto_reset = bool(auto_reset)
+        self._reset_stream_rows = int(reset_stream_rows)
+        if self._reset_stream_rows < 1:
+            raise ValueError("reset_stream_rows must be >= 1")
 
     # ------------------------------------------------------------------ task hooks
     def _task_spec(self):
@@ -73,6 +80,11 @@ class SawyerBatchedEnv:
 
     def _draw_reset(self, mask):
         """-> (obj_qpos float64 [N,k], goal rows int32 [N] or None): the random draws of reset_model(), env order."""
+        raise NotImplementedError
+
+    def _reset_stream(self, rows):
+        """-> (obj_qpos float64 [rows,N,k], goal rows int32 [rows,N] or None): this shard's columns of the pre-drawn
+        reset stream of an auto-reset handle."""
         raise NotImplementedError
 
     # ------------------------------------------------------------------ construction
@@ -93,6 +105,7 @@ class SawyerBatchedEnv:
             return
         L = _lib.lib()
         flags = (_lib.FLAG_EVAL_STATS if self._eval_stats else 0) | (_lib.FLAG_LIFELONG if self._lifelong else 0)
+        flags |= _lib.FLAG_AUTO_RESET if self._auto_reset else 0
         if self._reward_type == "dense":
             flags |= _lib.FLAG_DENSE_REWARD
         cfg = _lib.MjConfig(self.ENV_KIND, self.num_envs, self.device.index or 0, flags, self._episode_horizon,
@@ -112,7 +125,13 @@ class SawyerBatchedEnv:
         self._reward = torch.empty((n,), dtype=torch.float32, device=dev)
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
-        self._goal_rows = torch.zeros((n,), dtype=torch.int32, device=dev)
+        self._goal_rows = torch.zeros((n,), dtype=torch.int32, device=dev)   # the handle reads it (auto reset): never rebound
+        if self._auto_reset:
+            qpos, rows = self._reset_stream(self._reset_stream_rows)
+            qpos = np.ascontiguousarray(qpos, np.float64)
+            rows = None if rows is None else np.ascontiguousarray(rows, np.int32)
+            _lib.check(L.earl_mj_set_reset_stream(h, qpos.ctypes.data, None if rows is None else rows.ctypes.data,
+                                                  self._reset_stream_rows, self._goal_rows.data_ptr()))
 
     def _upload_goals(self):
         g = np.ascontiguousarray(np.stack(self._goal_table), np.float64)
@@ -158,9 +177,10 @@ class SawyerBatchedEnv:
         return torch.as_tensor(mask, device=self.device).to(torch.uint8).contiguous()
 
     def _reset_device(self, m, obj_qpos):
-        a = torch.as_tensor(np.array(obj_qpos, np.float64, order="C", copy=True)).to(self.device)
+        """obj_qpos None (auto-reset handles): each reset env's next draw of the pre-drawn reset stream."""
+        a = None if obj_qpos is None else torch.as_tensor(np.array(obj_qpos, np.float64, order="C", copy=True)).to(self.device)
         obs = torch.empty((self.num_envs, OBS_DIM), dtype=torch.float32, device=self.device)
-        _lib.check(_lib.lib().earl_mj_reset(self._handle, _ptr(m), a.data_ptr(), self._goal_rows.data_ptr(), obs.data_ptr(), _stream()))
+        _lib.check(_lib.lib().earl_mj_reset(self._handle, _ptr(m), _ptr(a), self._goal_rows.data_ptr(), obs.data_ptr(), _stream()))
         if m is not None:  # rows of envs that were not reset still need their current observation
             obs = torch.where(m.view(-1, 1).bool(), obs, self._get_obs())
         return obs.cpu().numpy() if self._host_mode else obs   # numpy-driven env: numpy out, like its step()

@@ -102,6 +102,23 @@ def pcg64_states(seeds):
     return out
 
 
+def reset_stream(seed, total_envs, env_offset, num_envs, rows, task='all_pairs'):
+    """Initial configurations of `rows` successive full resets, (config uint8 [rows, num_envs], object-qpos table float64
+    [K,14]): row e is what reset() of a handle without auto_reset draws at its e-th full reset (np.random.randint(6) per
+    env of the global batch on np.random.seed(seed), this shard's slice kept).  Single-component tasks draw nothing: one
+    table row, all-zero configs."""
+    if task == 'all_pairs':
+        table = initial_states['all_pairs'][:, 9:]
+        r = rng.NumpyLegacyRandom(int(seed) & 0xFFFFFFFF)
+        config = np.empty((rows, num_envs), np.uint8)
+        for e in range(rows):
+            config[e] = r.randint(table.shape[0], total_envs)[env_offset:env_offset + num_envs]
+    else:
+        table = initial_states[task][None, 9:]
+        config = np.zeros((rows, num_envs), np.uint8)
+    return config, np.ascontiguousarray(table, np.float64)
+
+
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
@@ -112,7 +129,7 @@ class Kitchen:
     max_path_length = int(1e8)
 
     def __init__(self, task="all_pairs", reward_type="dense", num_envs=1, device=None, seed=0, env_offset=0, total_envs=None,
-                 model_path=None, **_unused):
+                 model_path=None, auto_reset=False, reset_stream_rows=64, **_unused):
         if reward_type != 'dense':
             raise ValueError("Kitchen environment only supports dense rewards.")     # kitchen.py:91-92
         self._initial_states = copy.deepcopy(initial_states)
@@ -138,6 +155,11 @@ class Kitchen:
         self._handle = None
         self._np_random = rng.NumpyLegacyRandom(self._seed & 0xFFFFFFFF)     # the global np.random of reset_model
         self._env_seed = self._seed
+        # auto_reset=True: an env whose horizon fires is reset inside step() on the device, and every reset without
+        # config_index takes its configuration from a pre-drawn stream of `reset_stream_rows` full resets (reset_stream())
+        self._auto_reset, self._reset_stream_rows = bool(auto_reset), int(reset_stream_rows)
+        if self._reset_stream_rows < 1:
+            raise ValueError("reset_stream_rows must be >= 1")
 
     # ------------------------------------------------------------------ reference surface
     def get_task(self):
@@ -179,7 +201,7 @@ class Kitchen:
             return
         cfg = MjkConfig()
         cfg.num_envs, cfg.device, cfg.frame_skip = self.num_envs, self.device.index or 0, FRAME_SKIP
-        cfg.flags = _lib.FLAG_LIFELONG if self._lifelong else 0
+        cfg.flags = (_lib.FLAG_LIFELONG if self._lifelong else 0) | (_lib.FLAG_AUTO_RESET if self._auto_reset else 0)
         cfg.episode_horizon = self._episode_horizon
         cfg.goal_change_frequency = self._goal_change_frequency if self._lifelong else 0
         cfg.goal[:] = self.goal.tolist()
@@ -200,6 +222,11 @@ class Kitchen:
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
         self.seed(self._env_seed)
+        if self._auto_reset:
+            config, table = reset_stream(self._seed, self._total_envs, self._env_offset, n, self._reset_stream_rows, self._task)
+            config = np.ascontiguousarray(config)
+            _lib.check(_lib.lib().earl_mjk_set_reset_stream(h, config.ctypes.data, self._reset_stream_rows, table.ctypes.data,
+                                                            len(table)))
 
     def close(self):
         if self._handle is not None:
@@ -226,7 +253,9 @@ class Kitchen:
 
     def reset(self, mask=None, config_index=None):
         """reset() of every env (or those in `mask`); `config_index` [count] overrides the random draw.  Returns the
-        observation float64 [N,46] of all environments (rows of environments that were not reset hold their last one)."""
+        observation float64 [N,46] of all environments (rows of environments that were not reset hold their last one).
+        On an auto_reset env the draw is each reset env's next entry of the pre-drawn reset stream, made on the device, and
+        last_config_index is None."""
         self._ensure()
         if mask is None:
             ids, count = None, self.num_envs
@@ -235,15 +264,19 @@ class Kitchen:
             count = int(ids.numel())
             if count == 0:
                 return self._obs
-        if config_index is None:
-            objs, self.last_config_index = self._draw_configs(count)
+        o = None
+        if config_index is None and self._auto_reset:
+            self.last_config_index = None
         else:
-            self.last_config_index = np.asarray(config_index, np.int64).reshape(count)
-            objs = self._initial_states['all_pairs'][self.last_config_index, 9:]
-        o = torch.as_tensor(np.array(objs, np.float64, order="C", copy=True)).to(self.device)
+            if config_index is None:
+                objs, self.last_config_index = self._draw_configs(count)
+            else:
+                self.last_config_index = np.asarray(config_index, np.int64).reshape(count)
+                objs = self._initial_states['all_pairs'][self.last_config_index, 9:]
+            o = torch.as_tensor(np.array(objs, np.float64, order="C", copy=True)).to(self.device)
         out = torch.empty((count, OBS_DIM), dtype=torch.float64, device=self.device)
-        _lib.check(_lib.lib().earl_mjk_reset(self._handle, None if ids is None else ids.data_ptr(), count, o.data_ptr(),
-                                             out.data_ptr(), _stream()))
+        _lib.check(_lib.lib().earl_mjk_reset(self._handle, None if ids is None else ids.data_ptr(), count,
+                                             None if o is None else o.data_ptr(), out.data_ptr(), _stream()))
         if ids is None:
             self._obs.copy_(out)
         else:

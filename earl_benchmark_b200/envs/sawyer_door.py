@@ -23,7 +23,7 @@ import os
 
 import numpy as np
 
-from .. import _lib
+from .. import _lib, rng
 from ._sawyer_base import ACT_DIM, MODEL_DIR, OBS_DIM, SawyerBatchedEnv  # noqa: F401
 
 # reference module-level constants, earl_benchmark/envs/sawyer_door.py:13-16
@@ -33,6 +33,23 @@ goal_states = np.array([[0.29072163, 0.74286009, 0.10003595, 1.0,
                          0.29072163, 0.74286009, 0.10003595]])
 
 MODEL_PATH = os.path.join(MODEL_DIR, "sawyer_door.npz")
+
+
+def _angle_range(reset_at_goal):
+    """(obj_init_angle, uniform low, uniform high) of reset_model(), sawyer_door.py:33,114-118"""
+    return (0.0, -np.pi / 20, 0.0) if reset_at_goal else (-np.pi / 3, 0.0, np.pi / 20)
+
+
+def reset_stream(seed, total_envs, env_offset, num_envs, rows, reset_at_goal=False):
+    """Door angles of `rows` successive full resets, float64 [rows, num_envs, 1]: row e is what reset() of a handle
+    without auto_reset draws at its e-th full reset (np.random.seed(seed), one uniform per env of the global batch,
+    this shard's slice kept)."""
+    angle0, lo, hi = _angle_range(reset_at_goal)
+    r = rng.NumpyLegacyRandom(int(seed) & 0xFFFFFFFF)
+    out = np.empty((rows, num_envs, 1), np.float64)
+    for e in range(rows):
+        out[e, :, 0] = np.full(num_envs, float(angle0)) + r.uniform(lo, hi, total_envs)[env_offset:env_offset + num_envs]
+    return out
 
 
 def task_spec(model, max_newton=0, hand_init_pos=(0.0, 0.4, 0.2)):
@@ -102,10 +119,13 @@ class SawyerDoorV2(SawyerBatchedEnv):
     def get_next_goal(self):  # sawyer_door.py:96-98
         return np.broadcast_to(self.goal_states[0], (self.num_envs, 7)).copy()
 
+    def _reset_stream(self, rows):
+        return reset_stream(self._seed, self._total_envs, self._env_offset, self.num_envs, rows, self._reset_at_goal), None
+
     def _draw_angles(self, mask):
         """obj_init_angle + np.random.uniform(0, pi/20)  (or (-pi/20, 0) when reset_at_goal), sawyer_door.py:114-118;
         one draw per reset env, in env order."""
-        lo, hi = (0.0, np.pi / 20) if not self._reset_at_goal else (-np.pi / 20, 0.0)
+        _, lo, hi = _angle_range(self._reset_at_goal)
         ang = np.full(self.num_envs, float(self.obj_init_angle))
         if mask is None:
             u = self._np_random.uniform(lo, hi, self._total_envs)[self._env_offset:self._env_offset + self.num_envs]
@@ -115,8 +135,11 @@ class SawyerDoorV2(SawyerBatchedEnv):
         return ang
 
     def reset(self, mask=None, door_angle=None):
-        """reset() of every env (or those in `mask`); `door_angle` [N] overrides the random draw."""
+        """reset() of every env (or those in `mask`); `door_angle` [N] overrides the random draw.  On an auto_reset env the
+        draw is each reset env's next row of the pre-drawn reset stream."""
         self._ensure()
         m = self._mask(mask)
+        if door_angle is None and self._auto_reset:
+            return self._reset_device(m, None)
         ang = self._draw_angles(m) if door_angle is None else np.broadcast_to(np.asarray(door_angle, np.float64), (self.num_envs,))
         return self._reset_device(m, np.asarray(ang, np.float64).reshape(self.num_envs, 1))

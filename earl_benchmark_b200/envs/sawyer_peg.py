@@ -19,7 +19,7 @@ import os
 
 import numpy as np
 
-from .. import _lib
+from .. import _lib, rng
 from ._sawyer_base import ACT_DIM, MODEL_DIR, OBS_DIM, SawyerBatchedEnv  # noqa: F401
 
 # reference module-level constants, earl_benchmark/envs/sawyer_peg.py:18-58
@@ -43,6 +43,19 @@ MODEL_PATH = os.path.join(MODEL_DIR, "sawyer_peg.npz")
 # _random_reset_space = Box(hstack(obj_low, goal_low), hstack(obj_high, goal_high)), sawyer_peg.py:64-69,102-105
 _RESET_LOW = np.array([0.0, 0.5, 0.02, -0.35, 0.4, -0.001])
 _RESET_HIGH = np.array([0.2, 0.7, 0.02, -0.25, 0.7, 0.001])
+
+
+def reset_stream(seed, total_envs, env_offset, num_envs, rows, reset_at_goal=False, wide_init=False):
+    """Goal rows int32 [rows, num_envs] and peg positions float64 [rows, num_envs, 3] of `rows` successive full resets: row e
+    is what reset() of a handle without auto_reset draws at its e-th full reset (_draw_one over the global batch in env
+    order on np.random.seed(seed), this shard's slice kept), replayed natively (rng.NumpyLegacyRandom.peg_reset_draws)."""
+    r = rng.NumpyLegacyRandom(int(seed) & 0xFFFFFFFF)
+    goal_rows = np.empty((rows, num_envs), np.int32)
+    pos = np.empty((rows, num_envs, 3), np.float64)
+    for e in range(rows):
+        g, p = r.peg_reset_draws(total_envs, wide_init, reset_at_goal)
+        goal_rows[e], pos[e] = g[env_offset:env_offset + num_envs], p[env_offset:env_offset + num_envs]
+    return goal_rows, pos
 
 
 def task_spec(model, max_newton=0):
@@ -91,6 +104,10 @@ class SawyerPegV2(SawyerBatchedEnv):
     def _task_spec(self):
         return task_spec(self.model, self._max_newton)
 
+    def _reset_stream(self, rows):
+        g, p = reset_stream(self._seed, self._total_envs, self._env_offset, self.num_envs, rows, self._reset_at_goal, self.wide_init)
+        return p, g
+
     # ------------------------------------------------------------------ the reference's draws, one env at a time
     def _rand_vec(self):  # _get_state_rand_vec(): np.random.uniform(low, high, size=6)
         return _RESET_LOW + (_RESET_HIGH - _RESET_LOW) * self._np_random.uniform(0.0, 1.0, 6)
@@ -138,9 +155,12 @@ class SawyerPegV2(SawyerBatchedEnv):
         return super().compute_reward(obs, actions)
 
     def reset(self, mask=None, peg_pos=None):
-        """reset() of every env (or those in `mask`); `peg_pos` [N,3] overrides the random draw."""
+        """reset() of every env (or those in `mask`); `peg_pos` [N,3] overrides the random draw.  On an auto_reset env the
+        draw (goal row and peg position) is each reset env's next row of the pre-drawn reset stream."""
         self._ensure()
         m = self._mask(mask)
+        if peg_pos is None and self._auto_reset:
+            return self._reset_device(m, None)
         n = self.num_envs
         pos = np.tile(self.init_config["obj_init_pos"], (n, 1)).astype(np.float64)
         rows = self._goal_rows.cpu().numpy().copy()

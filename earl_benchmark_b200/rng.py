@@ -5,6 +5,7 @@ Reference call sites (SURVEY.md Appendix D):
   random.sample(task_list, 1)    earl_benchmark/envs/tabletop_manipulation.py:66   -> PyRandom.tabletop_goal_rows
   np.random.uniform(-2.5, 2.5)   earl_benchmark/envs/tabletop_manipulation.py:115-117 -> NumpyLegacyRandom.uniform
   np.random.randint(0, n)        earl_benchmark/envs/sawyer_peg.py:147,151; envs/kitchen.py:123 -> .randint
+  SawyerPegV2.reset_model draws  earl_benchmark/envs/sawyer_peg.py:192-229        -> NumpyLegacyRandom.peg_reset_draws
 """
 import ctypes as C
 
@@ -81,3 +82,12 @@ class NumpyLegacyRandom(_Stream):
         out = np.empty(count, np.float64)
         _lib.lib().earl_rng_np_uniform(self._h, float(low), float(high), count, out.ctypes.data)
         return out
+
+    def peg_reset_draws(self, count, wide_init=False, reset_at_goal=False):
+        """`count` successive SawyerPegV2._draw_one() draws (goal row, peg position), replayed natively:
+        (rows int32 [count], pos float64 [count,3])."""
+        rows = np.empty(count, np.int32)
+        pos = np.empty((count, 3), np.float64)
+        _lib.lib().earl_rng_peg_reset_draws(self._h, int(bool(wide_init)), int(bool(reset_at_goal)), count, rows.ctypes.data,
+                                            pos.ctypes.data)
+        return rows, pos

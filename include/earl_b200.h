@@ -215,6 +215,12 @@ EARL_API void earl_rng_tabletop_goal_rows(earl_rng* r, const uint8_t* task_to_ro
 EARL_API void earl_rng_np_randint(earl_rng* r, uint32_t n, int64_t count, int32_t* out);
 /* legacy numpy uniform(low, high): 53-bit double from two draws */
 EARL_API void earl_rng_np_uniform(earl_rng* r, double low, double high, int64_t count, double* out);
+/* SawyerPegV2.reset_model's draws (sawyer_peg.py:192-229) for `count` successive environments on a legacy numpy stream, as
+ * the batched env's _draw_one() makes them: the goal row (0, or 1 + randint(15) when reset_at_goal) and the peg position
+ * (the 6-uniform _get_state_rand_vec redrawn while within 0.1 of the block, the wide_init mix of that and a jittered
+ * wide_initial_states row, or the jittered goal position when reset_at_goal).  rows_out i32 [count], pos_out f64 [count,3]. */
+EARL_API void earl_rng_peg_reset_draws(earl_rng* r, int32_t wide_init, int32_t reset_at_goal, int64_t count, int32_t* rows_out,
+                                       double* pos_out);
 
 #ifdef __cplusplus
 }

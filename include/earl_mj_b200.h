@@ -23,7 +23,7 @@ typedef struct {
   int32_t env_kind;         /* EARL_ENV_SAWYER_DOOR or EARL_ENV_SAWYER_PEG */
   int32_t num_envs;
   int32_t device;
-  uint32_t flags;           /* EARL_FLAG_EVAL_STATS | EARL_FLAG_LIFELONG | EARL_FLAG_DENSE_REWARD */
+  uint32_t flags;           /* EARL_FLAG_EVAL_STATS | EARL_FLAG_LIFELONG | EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET */
   int64_t episode_horizon;  /* PersistentStateWrapper(episode_horizon), persistent_state_wrapper.py:10-12 */
   int64_t goal_change_frequency; /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
 } earl_mj_config;
@@ -71,11 +71,24 @@ EARL_API int earl_mj_set_goal_table(earl_mj_handle* h, const double* rows_host, 
 EARL_API int earl_mj_build_reset_template(earl_mj_handle* h, const double* hand_init_pos_host, const float* ctrl_host,
                                           int32_t steps);
 
+/* Pre-drawn reset stream of an EARL_FLAG_AUTO_RESET handle: the random draws of reset_model() (sawyer_door.py:114-118,
+ * sawyer_peg.py:192-229) for `rows` successive full resets, host arrays obj_qpos f64 [rows, N, obj_qpos_count] and, for
+ * tasks whose reset draws the goal (peg reset_at_goal), goal_rows i32 [rows, N] (else NULL).  Every reset of such a handle
+ * that is given no obj_qpos -- the reset pass after a step whose horizon fired, and earl_mj_reset(obj_qpos NULL) -- takes
+ * the next row of each reset env's column through a per-env cursor, which wraps modulo `rows`.  goal_rows_dev i32 [N] is
+ * the caller's array of current goal rows (reset_goal(), sawyer_door.py:100-102): those resets read their goal row from
+ * it (and write the drawn one when goal_rows is given); it must stay allocated for the handle's lifetime.  Uploading
+ * again (same `rows`) replaces the stream and rewinds the cursors. */
+EARL_API int earl_mj_set_reset_stream(earl_mj_handle* h, const double* obj_qpos_host, const int32_t* goal_rows_host, int32_t rows,
+                                      int32_t* goal_rows_dev);
+
 /* PersistentStateWrapper.reset + reset_model (persistent_state_wrapper.py:17-20, sawyer_door.py:111-125) for every env
  * with mask[i] != 0 (NULL = all): state <- reset template, object joint <- obj_qpos[i,:] with zero velocity
  * (_set_obj_xyz), goal <- goal_idx[i] (NULL = row 0), num_interventions += 1, steps_since_reset = 0, then a fresh
  * forward-kinematics pass and the observation (obs_out may be NULL).  obj_qpos is f64 [N, obj_qpos_count] (door angle /
- * peg xyz; sawyer_peg.py:192-229): the host draws it from the bit-exact replica of the reference's np.random stream. */
+ * peg xyz; sawyer_peg.py:192-229): the host draws it from the bit-exact replica of the reference's np.random stream.
+ * On an EARL_FLAG_AUTO_RESET handle obj_qpos NULL takes the draws and goal rows from the reset stream instead
+ * (earl_mj_set_reset_stream; goal_idx is ignored) and writes the obs rows of the reset envs only. */
 EARL_API int earl_mj_reset(earl_mj_handle* h, const uint8_t* mask_dev, const double* obj_qpos_dev, const int32_t* goal_idx_dev,
                            float* obs_out_dev, void* stream);
 
@@ -83,8 +96,10 @@ EARL_API int earl_mj_reset(earl_mj_handle* h, const uint8_t* mask_dev, const dou
  * mj_step), EARL observation + sparse reward (sawyer_door.py:86-94,168-177), counters and horizon `done`
  * (persistent_state_wrapper.py:22-31).  With EARL_FLAG_LIFELONG also LifelongWrapper.step (lifelong_wrapper.py:30-44):
  * lifelong_return += reward and, every goal_change_frequency steps, reset_goal() -- the observation of that step then
- * carries the new goal while the reward is the pre-swap one.  actions [N,4] f32; obs [N,14] f32; reward [N] f32;
- * done [N] u8; success [N] u8 or NULL. */
+ * carries the new goal while the reward is the pre-swap one.  With EARL_FLAG_AUTO_RESET every env whose horizon fired
+ * is then reset as earl_mj_reset(obj_qpos NULL) would reset it (one more launch in `stream`, after the step): reward,
+ * done and success describe the step that ended, its obs row is the post-reset observation.  actions [N,4] f32;
+ * obs [N,14] f32; reward [N] f32; done [N] u8; success [N] u8 or NULL. */
 EARL_API int earl_mj_step(earl_mj_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev,
                           uint8_t* success_dev, void* stream);
 /* Same with HOST buffers (copies inside the call, synchronous). */

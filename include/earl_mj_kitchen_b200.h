@@ -44,7 +44,7 @@ typedef struct earl_mjk_handle earl_mjk_handle;
 
 typedef struct {
   int32_t num_envs, device;
-  uint32_t flags;                 /* EARL_FLAG_LIFELONG */
+  uint32_t flags;                 /* EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET (any other flag is rejected) */
   int32_t frame_skip;             /* 40 (KitchenV0.__init__, kitchen_multitask_v0.py:38) */
   int64_t episode_horizon;        /* PersistentStateWrapper(episode_horizon) */
   int64_t goal_change_frequency;  /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
@@ -64,10 +64,19 @@ EARL_API int earl_mjk_destroy(earl_mjk_handle* h);
  * numpy's PCG64(SeedSequence(seed)) exactly as gym 0.23.1 seeding.np_random builds env.np_random
  * (adept_envs/mujoco_env.py:113-118). */
 EARL_API int earl_mjk_seed(earl_mjk_handle* h, const uint64_t* pcg_state_host);
+/* Pre-drawn reset stream of an EARL_FLAG_AUTO_RESET handle: reset_model's np.random.randint(K) (ENV/kitchen.py:122-124)
+ * for `rows` successive full resets, config u8 [rows, N] on the HOST, indexing table f64 [num_configs, 14] (HOST, the object
+ * qpos of each initial configuration; single-component tasks: one row and an all-zero config).  Every reset of such a handle
+ * that is given no object_qpos -- the reset pass after a step whose horizon fired, and earl_mjk_reset(object_qpos NULL) --
+ * takes the next entry of each reset env's column through a per-env cursor, which wraps modulo `rows`.  Uploading again
+ * (same shape) replaces the stream and rewinds the cursors. */
+EARL_API int earl_mjk_set_reset_stream(earl_mjk_handle* h, const uint8_t* config_host, int32_t rows, const double* table_host,
+                                       int32_t num_configs);
 /* Kitchen.reset_model (ENV/kitchen.py:118-139) for the `count` environments listed in env_ids_dev (NULL = all):
  * qpos <- init_qpos with objects 9.. of object_qpos_dev [count,14] (the drawn initial configuration), zero velocity,
  * robot.reset's five cached observations at noise ratio 1, mocap <- midpoint, 10 x (40 substeps with the control computed
- * from the fifth of them), then the observation (obs_out_dev f64 [count,46], may be NULL). */
+ * from the fifth of them), then the observation (obs_out_dev f64 [count,46], may be NULL).  object_qpos_dev NULL (auto-reset
+ * handles only): the configuration is each env's next draw of the reset stream (earl_mjk_set_reset_stream). */
 EARL_API int earl_mjk_reset(earl_mjk_handle* h, const int32_t* env_ids_dev, int32_t count, const double* object_qpos_dev,
                             double* obs_out_dev, void* stream);
 /* One PersistentStateWrapper.step of every environment: KitchenV0.step (kitchen_multitask_v0.py:91-125: action clip and
@@ -75,7 +84,11 @@ EARL_API int earl_mjk_reset(earl_mjk_handle* h, const int32_t* env_ids_dev, int3
  * (franka_robot.py:137-168), Kitchen._get_reward_n_score / is_successful (ENV/kitchen.py:141-183), counters and horizon
  * done.  With EARL_FLAG_LIFELONG also LifelongWrapper.step (lifelong_wrapper.py:30-44): lifelong_return += reward and,
  * every goal_change_frequency steps, reset_goal() (one goal: no change) followed by env._get_obs() -- a SECOND noisy
- * observation (46 more draws), which is the one returned and the one the next control is computed from.  actions f32 [N,9]; obs f64 [N,46]; reward f64 [N]; done u8 [N]; success u8 [N] or NULL. */
+ * observation (46 more draws), which is the one returned and the one the next control is computed from.  With
+ * EARL_FLAG_AUTO_RESET every environment whose horizon fired is then reset as earl_mjk_reset(object_qpos NULL) would reset it
+ * (one more launch in `stream`, after the step, redo and ordering kernels): reward, done and success describe the step that
+ * ended, its obs row is the post-reset observation.  actions f32 [N,9]; obs f64 [N,46]; reward f64 [N]; done u8 [N]; success
+ * u8 [N] or NULL. */
 EARL_API int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev, double* reward_dev, uint8_t* done_dev,
                            uint8_t* success_dev, void* stream);
 /* sim state as host arrays (synchronous): qpos, qvel, qacc_warmstart f64 [N,23], mocap_pos f64 [N,3], last noisy robot
