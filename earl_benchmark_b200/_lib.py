@@ -106,6 +106,8 @@ SIGNATURES = [
     ("earl_tt3_counters", C.c_int, [_VP, C.POINTER(_I64), _VP, _VP, _VP]),
     ("earl_tt3_get_state", C.c_int, [_VP, _VP, _VP, _VP]),
     ("earl_tt3_set_state", C.c_int, [_VP, _VP, _VP, _VP]),
+    ("earl_tt3_set_reset_stream", C.c_int, [_VP, _VP, _I32]),
+    ("earl_tt3_eval_stats", C.c_int, [_VP, _VP, _VP]),
     ("earl_tt3_launch_count", _I64, [_VP]),
     # include/earl_mj_b200.h
     ("earl_mj_create", C.c_int, [C.POINTER(MjConfig), C.c_char_p, _SZ, C.POINTER(MjTask), C.POINTER(_VP)]),

@@ -8,7 +8,10 @@
 //   * actions [N,3] f32 and observations [N,20] f32 are row-major at the boundary: a block moves its 256-env
 //     tile through shared memory so the global accesses are contiguous float4 (3 KB in, 20 KB out per block);
 //   * algorithmic bytes per env-step: read 12 + 64 + 8 = 84, write fist 16 + meta 8 + obs 80 + 4 + 1 + 1 = 110  (194 B;
-//     + 16 for the envs that drag an object: only that plane is written back).
+//     + 16 for the envs that drag an object: only that plane is written back);
+//   * handles with EARL_FLAG_EVAL_STATS or EARL_FLAG_AUTO_RESET run the GENERAL instantiation of the step: + 16 B per
+//     env-step for the episode return (read + write), and per auto-reset env the object planes it did not write
+//     (48 B), the counter (16 B) and, with a reset stream, its row (64 B) and cursor (8 B).
 // Compiled with --fmad=false: every fp64 / fp32 operation below rounds exactly where numpy rounds; the one
 // fused operation numpy's BLAS performs (the 2-element fp64 dot) is written as an explicit fma.
 // There is no CPU fallback in this file.
@@ -23,6 +26,7 @@
 
 #include <cuda_runtime.h>
 
+#include "eval_stats.cuh"
 #include "tt3_env.cuh"
 
 namespace earl {
@@ -52,7 +56,18 @@ struct T3Params {
   unsigned long long horizon;
   double act_lo, act_span, threshold, clip, success_radius;
   double init_qpos[8];
+  // GENERAL step only (EARL_FLAG_EVAL_STATS / EARL_FLAG_AUTO_RESET); kept after the fields above so the parameter offsets of
+  // the plain step do not move
+  uint32_t features;         // kEvalStats | kAutoReset
+  int reset_rows;            // R of the reset stream (0: none)
+  double* ep_return;         // [N] or null
+  const double* reset_qpos;  // [R,N,8] or null: row e of env i at (e * n + i) * 8
+  uint32_t* reset_cursor;    // [N] or null
 };
+
+// meta.x bits 2 and 3: success at the last step / at any step of the episode (EARL_FLAG_EVAL_STATS)
+constexpr uint32_t kSuccLast = 4u, kSuccAny = 8u;
+constexpr uint32_t kEvalStats = 1u, kAutoReset = 2u;
 
 __device__ __forceinline__ void pdl_wait_prior_grid() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -80,6 +95,24 @@ __device__ __forceinline__ void flush_obs(const float4* tile, float* obs, int ba
   for (int k = threadIdx.x; k < rows * 5; k += kBlock) dst[k] = tile[k];
 }
 
+// qpos[0:8] of env i's next reset: its next reset-stream row when the handle has one (the cursor wraps modulo R), else
+// initial_state[0:8]
+__device__ __forceinline__ void next_reset_qpos(const T3Params& p, int i, double2 (&q)[4]) {
+  if (p.reset_qpos) {
+    const uint32_t c = p.reset_cursor[i];
+    const double2* r = reinterpret_cast<const double2*>(p.reset_qpos + ((size_t)(c % (uint32_t)p.reset_rows) * p.n + i) * 8);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) q[k] = r[k];
+    p.reset_cursor[i] = c + 1u;
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) q[k] = make_double2(p.init_qpos[2 * k], p.init_qpos[2 * k + 1]);
+  }
+}
+
+// GENERAL = false: dense / sparse reward only (the kernel bench.py measures).  GENERAL = true adds the episode statistics
+// and the auto-reset, each behind a warp-uniform test of p.features.
+template <bool GENERAL>
 __global__ void __launch_bounds__(kBlock) tt3_step_kernel(const __grid_constant__ T3Params p) {
   __shared__ float4 s_obs[kBlock * 5];
   __shared__ float4 s_act4[kBlock * kAct / 4];
@@ -129,15 +162,46 @@ __global__ void __launch_bounds__(kBlock) tt3_step_kernel(const __grid_constant_
         g[2 * k + 1] = v.y;
       }
     }
-    stage_obs(s_obs, t, o, marker(att), g);
+    if (!GENERAL) stage_obs(s_obs, t, o, marker(att), g);
     const bool succ = earl::tt3::success(o, g, p.success_radius);
     const float rew = p.dense ? (float)earl::tt3::dense(o, g) : (succ ? 1.0f : 0.0f);  // 3OBJ:146-159
     // PSW:22-31
     const uint32_t steps = m.y == 0xffffffffu ? m.y : m.y + 1u;
-    p.meta[i] = make_uint2((m.x & ~3u) | att, steps);
+    if (!GENERAL) p.meta[i] = make_uint2((m.x & ~3u) | att, steps);
     __stcs(p.reward + i, rew);
-    p.done[i] = (unsigned long long)steps >= p.horizon ? 1 : 0;
+    const bool done = (unsigned long long)steps >= p.horizon;
+    p.done[i] = done ? 1 : 0;
     if (p.success) p.success[i] = succ ? 1 : 0;
+    if (GENERAL) {
+      uint32_t mx = (m.x & ~3u) | att, ms = steps;
+      const bool reset = done && (p.features & kAutoReset);
+      if (p.features & kEvalStats) {
+        p.ep_return[i] = reset ? 0.0 : p.ep_return[i] + (double)rew;
+        mx = (mx & ~kSuccLast) | (succ ? (kSuccLast | kSuccAny) : 0u);
+      }
+      if (reset) {  // what earl_tt3_reset(init_qpos NULL) does to this env, fused: PSW:17-20 + 3OBJ:67-84
+        double2 q[4];
+        next_reset_qpos(p, i, q);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          p.q[k][i] = q[k];
+          o[2 * k] = (float)q[k].x;
+          o[2 * k + 1] = (float)q[k].y;
+        }
+        p.interventions[i] += 1;
+        mx &= ~(0xff00u | 0xfu);  // goal row 0 (get_next_goal() over one goal), nothing attached, success bits cleared
+        ms = 0u;
+        const float2* gr = reinterpret_cast<const float2*>(p.goal_f32);
+#pragma unroll
+        for (int k = 0; k < 5; ++k) {
+          const float2 v = __ldg(gr + k);
+          g[2 * k] = v.x;
+          g[2 * k + 1] = v.y;
+        }
+      }
+      p.meta[i] = make_uint2(mx, ms);
+      stage_obs(s_obs, t, o, marker(mx & 3u), g);
+    }
   }
   __syncthreads();
   flush_obs(s_obs, p.obs, base, end);
@@ -157,13 +221,19 @@ __global__ void __launch_bounds__(kBlock) tt3_reset_kernel(const __grid_constant
     row = row < 0 ? 0 : (row >= num_goals ? num_goals - 1 : row);
     m.x = (m.x & ~0xff00u) | ((uint32_t)row << 8);
     if (mode == 0) {
-      m.x &= ~3u;
+      m.x &= ~0xfu;  // nothing attached, success bits cleared
       m.y = 0;
       p.interventions[i] += 1;
+      double2 q[4];
+      if (init_qpos) {
 #pragma unroll
-      for (int k = 0; k < 4; ++k)
-        p.q[k][i] = init_qpos ? make_double2(init_qpos[(size_t)i * 8 + 2 * k], init_qpos[(size_t)i * 8 + 2 * k + 1])
-                              : make_double2(p.init_qpos[2 * k], p.init_qpos[2 * k + 1]);
+        for (int k = 0; k < 4; ++k) q[k] = make_double2(init_qpos[(size_t)i * 8 + 2 * k], init_qpos[(size_t)i * 8 + 2 * k + 1]);
+      } else {
+        next_reset_qpos(p, i, q);
+      }
+#pragma unroll
+      for (int k = 0; k < 4; ++k) p.q[k][i] = q[k];
+      if (p.ep_return) p.ep_return[i] = 0.0;
     }
     p.meta[i] = m;
   }
@@ -196,6 +266,19 @@ __global__ void __launch_bounds__(kBlock) tt3_reward_kernel(const float* obs, lo
   const bool succ = earl::tt3::success(o, g, radius);
   if (reward) reward[i] = dense ? (float)earl::tt3::dense(o, g) : (succ ? 1.0f : 0.0f);
   if (success) success[i] = succ ? 1 : 0;
+}
+
+// (sum episode return, #success at last step, #success at any step, N) -> out4 (pre-zeroed)
+__global__ void __launch_bounds__(kBlock) tt3_eval_stats_kernel(const __grid_constant__ T3Params p, double* __restrict__ out4) {
+  double ret = 0.0, last = 0.0, any = 0.0, cnt = 0.0;
+  for (int i = blockIdx.x * kBlock + threadIdx.x; i < p.n; i += gridDim.x * kBlock) {
+    const uint32_t f = p.meta[i].x;
+    ret += p.ep_return[i];
+    last += (f & kSuccLast) ? 1.0 : 0.0;
+    any += (f & kSuccAny) ? 1.0 : 0.0;
+    cnt += 1.0;
+  }
+  earl::block_add_eval_stats(ret, last, any, cnt, out4);
 }
 
 __global__ void __launch_bounds__(kBlock) tt3_state_kernel(const __grid_constant__ T3Params p, double* qpos_out, int32_t* att_out,
@@ -251,6 +334,8 @@ struct earl_tt3_handle {
   T3Params p{};
   int64_t total_steps = 0;
   int64_t launches = 0;
+  int sm_count = 0;
+  void (*step_kernel)(T3Params) = nullptr;  // chosen once from the flags in earl_tt3_create
   std::vector<void*> owned;
   float* d_act = nullptr;
   float* d_obs = nullptr;
@@ -283,6 +368,14 @@ int check(const earl_tt3_handle* h) {
   return 0;
 }
 
+// auto-reset with reset_at_goal draws every reset from the stream: stepping or resetting without one is an error
+int check_stream(const earl_tt3_handle* h) {
+  const uint32_t both = EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL;
+  if ((h->cfg.flags & both) == both && !h->p.reset_qpos)
+    return fail(EARL_ERR_INVALID, "EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL needs earl_tt3_set_reset_stream first");
+  return 0;
+}
+
 int grid_for(long long n) { return (int)((n + kBlock - 1) / kBlock); }
 
 int launch_step(earl_tt3_handle* h, int first, int count, const float* actions, float* obs, float* reward, uint8_t* done,
@@ -304,7 +397,7 @@ int launch_step(earl_tt3_handle* h, int first, int count, const float* actions, 
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  CU(cudaLaunchKernelEx(&cfg, tt3_step_kernel, p));
+  CU(cudaLaunchKernelEx(&cfg, h->step_kernel, p));
   h->launches += 1;
   return 0;
 }
@@ -320,7 +413,8 @@ int earl_tt3_create(const earl_tt3_config* cfg, size_t cfg_nbytes, earl_tt3_hand
   if (cfg_nbytes != sizeof(earl_tt3_config)) return fail(EARL_ERR_INVALID, "earl_tt3_config size mismatch (%zu)", cfg_nbytes);
   if (cfg->num_envs < 1) return fail(EARL_ERR_INVALID, "num_envs must be >= 1");
   if (cfg->num_goals < 1 || cfg->num_goals > EARL_TT3_MAX_GOALS) return fail(EARL_ERR_INVALID, "num_goals out of range");
-  if (cfg->flags & ~(uint32_t)EARL_FLAG_DENSE_REWARD) return fail(EARL_ERR_UNSUPPORTED, "unsupported flag for the three-object tabletop");
+  const uint32_t supported = EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL | EARL_FLAG_EVAL_STATS;
+  if (cfg->flags & ~supported) return fail(EARL_ERR_UNSUPPORTED, "unsupported flag for the three-object tabletop");
   if (cfg->episode_horizon < 1) return fail(EARL_ERR_INVALID, "episode_horizon must be >= 1");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || cfg->device < 0 || cfg->device >= ndev) {
@@ -341,6 +435,9 @@ int earl_tt3_create(const earl_tt3_config* cfg, size_t cfg_nbytes, earl_tt3_hand
   double* gd = nullptr;
   if (!rc) rc = h->alloc(&gf, (size_t)EARL_TT3_MAX_GOALS * 10);
   if (!rc) rc = h->alloc(&gd, (size_t)EARL_TT3_MAX_GOALS * 10);
+  if (!rc && (cfg->flags & EARL_FLAG_EVAL_STATS)) rc = h->alloc(&p.ep_return, n);
+  if (!rc) rc = cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, cfg->device) == cudaSuccess
+                    ? 0 : fail(EARL_ERR_CUDA, "cudaDeviceGetAttribute failed");
   if (rc) {
     earl_tt3_destroy(h);
     return rc;
@@ -366,6 +463,8 @@ int earl_tt3_create(const earl_tt3_config* cfg, size_t cfg_nbytes, earl_tt3_hand
   p.clip = cfg->clip;
   p.success_radius = cfg->success_radius;
   for (int k = 0; k < 8; ++k) p.init_qpos[k] = cfg->initial_state[k];
+  p.features = ((cfg->flags & EARL_FLAG_EVAL_STATS) ? kEvalStats : 0u) | ((cfg->flags & EARL_FLAG_AUTO_RESET) ? kAutoReset : 0u);
+  h->step_kernel = p.features ? tt3_step_kernel<true> : tt3_step_kernel<false>;
   *out = h;
   return 0;
 }
@@ -386,6 +485,9 @@ int earl_tt3_destroy(earl_tt3_handle* h) {
 int earl_tt3_reset(earl_tt3_handle* h, const uint8_t* mask_dev, const int32_t* goal_idx_dev, const double* init_qpos_dev,
                    float* obs_out_dev, void* stream) {
   if (int rc = check(h)) return rc;
+  if (!init_qpos_dev) {
+    if (int rc = check_stream(h)) return rc;
+  }
   T3Params p = h->p;
   p.obs = obs_out_dev;
   tt3_reset_kernel<<<grid_for(p.n), kBlock, 0, (cudaStream_t)stream>>>(p, mask_dev, goal_idx_dev, init_qpos_dev, 0, h->cfg.num_goals);
@@ -409,6 +511,7 @@ int earl_tt3_step(earl_tt3_handle* h, const float* actions_dev, float* obs_dev, 
   if (int rc = check(h)) return rc;
   if (!actions_dev || !obs_dev || !reward_dev || !done_dev) return fail(EARL_ERR_INVALID, "null device buffer");
   if (!aligned16(obs_dev)) return fail(EARL_ERR_INVALID, "obs must be 16-byte aligned");
+  if (int rc = check_stream(h)) return rc;
   if (int rc = launch_step(h, 0, h->p.n, actions_dev, obs_dev, reward_dev, done_dev, success_dev, (cudaStream_t)stream)) return rc;
   h->total_steps += 1;
   return 0;
@@ -421,6 +524,7 @@ int earl_tt3_rollout(earl_tt3_handle* h, const float* actions_dev, int32_t actio
     return fail(EARL_ERR_INVALID, "bad rollout argument");
   const size_t n = (size_t)h->p.n;
   if (!aligned16(obs_dev)) return fail(EARL_ERR_INVALID, "obs must be 16-byte aligned");
+  if (int rc = check_stream(h)) return rc;
   for (int t = 0; t < num_steps; ++t) {
     const size_t a = (size_t)(t % action_ring), o = (size_t)(t % out_ring);
     if (int rc = launch_step(h, 0, (int)n, actions_dev + a * n * kAct, obs_dev + o * n * kObs, reward_dev + o * n, done_dev + o * n,
@@ -435,6 +539,7 @@ int earl_tt3_step_host(earl_tt3_handle* h, const float* actions_host, float* obs
                        uint8_t* success_host) {
   if (int rc = check(h)) return rc;
   if (!actions_host || !obs_host || !reward_host || !done_host) return fail(EARL_ERR_INVALID, "null host buffer");
+  if (int rc = check_stream(h)) return rc;
   const size_t n = (size_t)h->p.n;
   if (!h->d_act) {
     int rc = h->alloc(&h->d_act, n * kAct, false);
@@ -470,6 +575,44 @@ int earl_tt3_step_host(earl_tt3_handle* h, const float* actions_host, float* obs
   if (success_host) CU(cudaMemcpyAsync(success_host, h->d_succ, n, cudaMemcpyDeviceToHost, so));
   h->total_steps += 1;
   CU(cudaStreamSynchronize(so));
+  return 0;
+}
+
+int earl_tt3_set_reset_stream(earl_tt3_handle* h, const double* qpos_rows_host, int32_t rows) {
+  if (int rc = check(h)) return rc;
+  const uint32_t both = EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL;
+  if ((h->cfg.flags & both) != both)
+    return fail(EARL_ERR_INVALID, "a reset stream needs EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL");
+  if (!qpos_rows_host || rows < 1) return fail(EARL_ERR_INVALID, "bad reset stream");
+  if (h->p.reset_qpos && rows != h->p.reset_rows)
+    return fail(EARL_ERR_INVALID, "the reset stream has %d rows; a new one must have as many", h->p.reset_rows);
+  const size_t n = (size_t)h->p.n;
+  CU(cudaDeviceSynchronize());  // no step or reset in flight reads the stream or the cursors while they are replaced
+  if (!h->p.reset_qpos) {
+    double* q = nullptr;
+    uint32_t* c = nullptr;
+    if (int rc = h->alloc(&q, (size_t)rows * n * 8, false)) return rc;
+    if (int rc = h->alloc(&c, n)) return rc;
+    h->p.reset_qpos = q;
+    h->p.reset_cursor = c;
+    h->p.reset_rows = rows;
+  }
+  CU(cudaMemcpy(const_cast<double*>(h->p.reset_qpos), qpos_rows_host, (size_t)rows * n * 8 * sizeof(double), cudaMemcpyHostToDevice));
+  CU(cudaMemset(h->p.reset_cursor, 0, n * sizeof(uint32_t)));
+  return 0;
+}
+
+int earl_tt3_eval_stats(earl_tt3_handle* h, double* out4_dev, void* stream) {
+  if (int rc = check(h)) return rc;
+  if (!out4_dev) return fail(EARL_ERR_INVALID, "null out4");
+  if (!h->p.ep_return) return fail(EARL_ERR_INVALID, "eval stats need EARL_FLAG_EVAL_STATS");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  CU(cudaMemsetAsync(out4_dev, 0, 4 * sizeof(double), s));
+  int grid = grid_for(h->p.n);
+  if (grid > h->sm_count * 4) grid = h->sm_count * 4;
+  tt3_eval_stats_kernel<<<grid, kBlock, 0, s>>>(h->p, out4_dev);
+  CU(cudaGetLastError());
+  h->launches += 1;
   return 0;
 }
 

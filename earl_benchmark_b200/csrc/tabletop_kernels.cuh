@@ -24,6 +24,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "eval_stats.cuh"
+
 namespace earl {
 
 constexpr int kTTBlock = 256;            // threads per CTA (8 warps)
@@ -489,31 +491,7 @@ __global__ void tabletop_eval_stats_kernel(const TabletopParams p, double* __res
     any += (f & kSuccessAny) ? 1.0 : 0.0;
     cnt += 1.0;
   }
-#pragma unroll
-  for (int o = 16; o; o >>= 1) {
-    ret += __shfl_xor_sync(0xffffffffu, ret, o);
-    last += __shfl_xor_sync(0xffffffffu, last, o);
-    any += __shfl_xor_sync(0xffffffffu, any, o);
-    cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-  }
-  __shared__ double sm[4][32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (lane == 0) { sm[0][warp] = ret; sm[1][warp] = last; sm[2][warp] = any; sm[3][warp] = cnt; }
-  __syncthreads();
-  if (warp == 0) {
-    const int nw = blockDim.x >> 5;
-    double v[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      v[k] = lane < nw ? sm[k][lane] : 0.0;
-#pragma unroll
-      for (int o = 16; o; o >>= 1) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-    }
-    if (lane == 0) {
-#pragma unroll
-      for (int k = 0; k < 4; ++k) atomicAdd(out4 + k, v[k]);
-    }
-  }
+  block_add_eval_stats(ret, last, any, cnt, out4);
 }
 
 }  // namespace earl

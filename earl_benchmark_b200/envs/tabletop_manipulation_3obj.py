@@ -13,7 +13,12 @@ Differences a caller can observe:
   * goals are rows of a goal table (`goal_states`; custom goals are appended, up to 16 rows);
   * `reset_at_goal` noise comes from a per-env-object replica of the legacy `np.random.seed(seed)` stream,
     consumed in env order (env 0's eight uniforms, then env 1's, ...), as a Python loop over N reference envs
-    sharing the global stream would.
+    sharing the global stream would.  A full reset draws the eight uniforms of all `total_envs` envs of the job and
+    keeps this shard's; a masked reset draws eight per selected env, in env order;
+  * `auto_reset=True`: an env whose horizon fires is reset inside step(), on the device, with the same result as
+    reset(mask=done).  With `reset_at_goal` too, every reset without `init_qpos` (auto or host) takes its qpos from a
+    pre-drawn stream of `reset_stream_rows` rows per env (see reset_stream()), so the draws do not depend on when an
+    env resets or on how the job is sharded.
 """
 import ctypes as C
 
@@ -34,6 +39,20 @@ OBS_DIM, ACT_DIM, MAX_GOALS = 20, 3, 16
 _NEVER = 1 << 62
 
 
+def reset_stream(seed, total_envs, env_offset, num_envs, rows):
+    """qpos[0:8] of `rows` successive reset_at_goal resets, float64 [rows, num_envs, 8]: row e, env j of the global batch
+    is goal_states[0][:8] + the eight uniforms of env j in draw e of np.random.seed(seed).uniform(-0.3, 0.3,
+    8 * total_envs) (tabletop_manipulation_3obj.py:72-76); this shard keeps columns [env_offset, env_offset + num_envs).
+    Row e is what the e-th full reset() of a handle without auto_reset draws.  Costs 16 * rows * total_envs draws of the
+    legacy Mersenne Twister (made natively) and 64 * rows bytes per env, on the host and on the device."""
+    r = rng.NumpyLegacyRandom(int(seed) & 0xFFFFFFFF)
+    out = np.empty((rows, num_envs, 8), np.float64)
+    for e in range(rows):
+        u = r.uniform(-0.3, 0.3, 8 * total_envs).reshape(total_envs, 8)[env_offset:env_offset + num_envs]
+        out[e] = goal_states[0][:8] + u
+    return out
+
+
 def _ptr(t):
     return 0 if t is None else t.data_ptr()
 
@@ -46,16 +65,29 @@ class TabletopManipulation:
     """N independent three-object tabletop envs stepped by one kernel launch.
 
     Reference-compatible arguments: reward_type, reset_at_goal (tabletop_manipulation_3obj.py:25-27).
-    Batched extras: num_envs, device, seed.
+    Batched extras: num_envs, device, seed, auto_reset (reset on the device when the horizon fires), reset_stream_rows
+    (rows of the pre-drawn reset_at_goal stream of an auto_reset env), eval_stats (per-env episode return and success,
+    reduced by eval_stats()), env_offset / total_envs (this shard's slice of a larger job: reset_at_goal draws are made
+    for `total_envs` envs and columns [env_offset, env_offset + N) kept).
     """
 
-    def __init__(self, reward_type="dense", reset_at_goal=False, num_envs=1, device=None, seed=0, host_io=False):
+    def __init__(self, reward_type="dense", reset_at_goal=False, num_envs=1, device=None, seed=0, host_io=False,
+                 auto_reset=False, reset_stream_rows=64, eval_stats=False, env_offset=0, total_envs=None):
         if reward_type not in ("sparse", "dense"):
             raise ValueError(f"reward_type must be 'sparse' or 'dense', got {reward_type!r}")
         self._reward_type = reward_type
         self._reset_at_goal = bool(reset_at_goal)
         self.num_envs = int(num_envs)
         self._seed = int(seed)
+        self._auto_reset = bool(auto_reset)
+        self._reset_stream_rows = int(reset_stream_rows)
+        if self._reset_stream_rows < 1:
+            raise ValueError("reset_stream_rows must be >= 1")
+        self._eval_stats = bool(eval_stats)
+        self._env_offset = int(env_offset)
+        self._total_envs = int(total_envs) if total_envs is not None else self.num_envs + self._env_offset
+        if self._env_offset < 0 or self._env_offset + self.num_envs > self._total_envs:
+            raise ValueError("envs [env_offset, env_offset + num_envs) must lie inside [0, total_envs)")
         if device is None:
             device = torch.cuda.current_device() if torch.cuda.is_available() else 0
         self.device = torch.device(device if not isinstance(device, int) else f"cuda:{device}")
@@ -91,6 +123,9 @@ class TabletopManipulation:
         cfg = _lib.Tt3Config()
         cfg.num_envs, cfg.device = self.num_envs, self.device.index or 0
         cfg.flags = _lib.FLAG_DENSE_REWARD if self._reward_type == "dense" else 0
+        cfg.flags |= _lib.FLAG_AUTO_RESET if self._auto_reset else 0
+        cfg.flags |= _lib.FLAG_RESET_AT_GOAL if self._reset_at_goal else 0
+        cfg.flags |= _lib.FLAG_EVAL_STATS if self._eval_stats else 0
         cfg.num_goals = MAX_GOALS          # every row is addressable; unused rows repeat row 0 until set
         cfg.episode_horizon = self._episode_horizon
         cfg.threshold, cfg.move_distance, cfg.clip, cfg.success_radius = self.threshold, self.move_distance, 2.8, 0.4
@@ -105,12 +140,19 @@ class TabletopManipulation:
         h = C.c_void_p()
         _lib.check(_lib.lib().earl_tt3_create(C.byref(cfg), C.sizeof(cfg), C.byref(h)))
         self._handle = h
+        if self._stream_resets():
+            rows = reset_stream(self._seed, self._total_envs, self._env_offset, self.num_envs, self._reset_stream_rows)
+            _lib.check(_lib.lib().earl_tt3_set_reset_stream(h, rows.ctypes.data, self._reset_stream_rows))
         n, dev = self.num_envs, self.device
         self._obs = torch.empty((n, OBS_DIM), dtype=torch.float32, device=dev)
         self._reward = torch.empty((n,), dtype=torch.float32, device=dev)
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._goal_rows = np.zeros(n, np.int32)
+
+    def _stream_resets(self):
+        """resets without init_qpos take their qpos from the device's reset stream"""
+        return self._auto_reset and self._reset_at_goal
 
     def close(self):
         if self._handle is not None:
@@ -172,19 +214,28 @@ class TabletopManipulation:
 
     # ------------------------------------------------------------------ reset / step
     def reset(self, mask=None, goal_rows=None, init_qpos=None):
-        """reset() of every env (or those in `mask`); goal_rows / init_qpos [N,8] override the draws."""
+        """reset() of every env (or those in `mask`); goal_rows / init_qpos [N,8] override the draws.
+
+        reset_at_goal without init_qpos: a full reset draws np.random.uniform(-0.3, 0.3, 8 * total_envs) and keeps this
+        shard's rows; a masked reset draws eight uniforms per selected env, in env order.  On an auto_reset env each
+        reset env instead takes its next row of the pre-drawn reset stream (reset_stream())."""
         self._ensure()
         m = self._mask(mask)
         sel = np.ones(self.num_envs, bool) if m is None else m.cpu().numpy().astype(bool)
         # per selected env, in env order: reset_goal() draws np.random.randint(len(goal list)) (one row: consumes
         # nothing), then reset_at_goal adds np.random.uniform(-0.3, 0.3, size=(8,)) to goal[:8]   (:70-73, :82)
         rows = self._goal_rows.copy() if goal_rows is None else np.broadcast_to(np.asarray(goal_rows, np.int32), (self.num_envs,)).copy()
-        noisy = init_qpos is None and self._reset_at_goal
+        noisy = init_qpos is None and self._reset_at_goal and not self._stream_resets()
         q = np.zeros((self.num_envs, 8))
         draw = goal_rows is None and len(self._goal_list) > 1
         if goal_rows is None and not draw:
             rows[sel] = 0
-        for i in np.flatnonzero(sel) if (draw or noisy) else ():
+        whole = noisy and not draw and m is None    # one draw for the whole job, this shard's slice kept
+        if whole:
+            lo, n = self._env_offset, self.num_envs
+            u = self._np_random.uniform(-0.3, 0.3, 8 * self._total_envs).reshape(self._total_envs, 8)[lo:lo + n]
+            q = np.asarray(self._goal_table)[rows, :8] + u
+        for i in np.flatnonzero(sel) if (draw or (noisy and not whole)) else ():
             if draw:
                 rows[i] = int(self._np_random.randint(len(self._goal_list), 1)[0])
             if noisy:
@@ -273,6 +324,15 @@ class TabletopManipulation:
         since = torch.empty((self.num_envs,), dtype=torch.int32, device=self.device)
         _lib.check(_lib.lib().earl_tt3_counters(self._handle, C.byref(total), interv.data_ptr(), since.data_ptr(), _stream()))
         return total.value, interv, since, None
+
+    def eval_stats(self):
+        """Device tensor [4] float64: (sum of episode returns, #envs successful at their last step, #envs successful at
+        any step of the episode, N), reduced on the device; needs eval_stats=True.  A reset clears an env's statistics.
+        Sum it over shards with distributed.all_reduce_eval_stats."""
+        self._ensure()
+        out = torch.empty((4,), dtype=torch.float64, device=self.device)
+        _lib.check(_lib.lib().earl_tt3_eval_stats(self._handle, out.data_ptr(), _stream()))
+        return out
 
     @property
     def launch_count(self):

@@ -11,7 +11,9 @@
  * Per-env state: qpos[0:8] as fp64 (fist x,y, object A x,y, object B x,y, object C x,y) like the
  * reference keeps it in MuJoCo's qpos, so open-loop rollouts of any length are bit-exact; one u32 of flags
  * (bits 0-1 attached object: 0 none, 1..3 = object_dict entries (0,0) / (0.5,0.5) / (1,1),
- * tabletop_manipulation_3obj.py:31-35; bits 8-15 goal row), u32 steps_since_reset, i64 num_interventions.
+ * tabletop_manipulation_3obj.py:31-35; bits 2-3 success at the last / at any step of the episode, kept with
+ * EARL_FLAG_EVAL_STATS; bits 8-15 goal row), u32 steps_since_reset, i64 num_interventions, and with
+ * EARL_FLAG_EVAL_STATS an f64 episode return.
  * Observation [N,20] f32 = qpos[0:8], attached marker x2, goal[0:10]  (:49-54).
  */
 #ifndef EARL_TT3_B200_H_
@@ -30,7 +32,8 @@ typedef struct earl_tt3_handle earl_tt3_handle;
 typedef struct {
   int32_t num_envs;          /* N >= 1 */
   int32_t device;            /* CUDA device ordinal */
-  uint32_t flags;            /* EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET (earl_b200.h) */
+  uint32_t flags;            /* EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL |
+                                EARL_FLAG_EVAL_STATS (earl_b200.h); any other flag is EARL_ERR_UNSUPPORTED */
   int32_t num_goals;         /* rows used in goal_table, 1..EARL_TT3_MAX_GOALS (reference: 1, :12-18) */
   int64_t episode_horizon;   /* PersistentStateWrapper(episode_horizon) */
   double threshold;          /* 0.4  attach radius, strict <            (:38, :107) */
@@ -48,7 +51,9 @@ EARL_API int earl_tt3_destroy(earl_tt3_handle* h);
 /* PersistentStateWrapper.reset + env.reset (:17-20; tabletop_manipulation_3obj.py:67-84) for envs with
  * mask[i] != 0 (NULL = all): num_interventions += 1, steps_since_reset = 0, attached cleared,
  * goal row <- goal_idx[i] (NULL = row 0), qpos[0:8] <- init_qpos[i] when given (the host computes
- * goal[:8] + uniform(-0.3, 0.3) for reset_at_goal, :72-76) else initial_state[0:8].
+ * goal[:8] + uniform(-0.3, 0.3) for reset_at_goal, :72-76).  With init_qpos NULL: on a handle with
+ * EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL each masked env's next reset-stream row (earl_tt3_set_reset_stream;
+ * EARL_ERR_INVALID before one is set), else initial_state[0:8].  Clears the episode statistics (EARL_FLAG_EVAL_STATS).
  * Writes the post-reset observation rows of the masked envs to obs_out when non-NULL. */
 EARL_API int earl_tt3_reset(earl_tt3_handle* h, const uint8_t* mask_dev, const int32_t* goal_idx_dev,
                             const double* init_qpos_dev /*[N,8]*/, float* obs_out_dev /*[N,20]*/, void* stream);
@@ -58,7 +63,11 @@ EARL_API int earl_tt3_set_goal(earl_tt3_handle* h, const uint8_t* mask_dev, cons
 
 /* The hot path: PersistentStateWrapper.step (:22-31) over env.step + move + _get_obs + compute_reward
  * (tabletop_manipulation_3obj.py:86-165).  actions [N,3] f32 in; obs [N,20] f32, reward [N] f32,
- * done [N] u8, success [N] u8 (nullable) out. */
+ * done [N] u8, success [N] u8 (nullable) out.
+ * EARL_FLAG_EVAL_STATS: episode_return += (double)reward, and the success bits are updated, every step.
+ * EARL_FLAG_AUTO_RESET: an env whose horizon fired is then reset, in the same kernel, as earl_tt3_reset(mask, goal_idx
+ * NULL, init_qpos NULL) resets it: reward, done and success describe the step that ended, its obs row is the post-reset
+ * observation. */
 EARL_API int earl_tt3_step(earl_tt3_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev,
                            uint8_t* done_dev, uint8_t* success_dev, void* stream);
 
@@ -70,6 +79,18 @@ EARL_API int earl_tt3_rollout(earl_tt3_handle* h, const float* actions_dev, int3
 /* same step with HOST buffers (copies inside the call, synchronous): the call a CPU-side RL loop makes */
 EARL_API int earl_tt3_step_host(earl_tt3_handle* h, const float* actions_host, float* obs_host, float* reward_host,
                                 uint8_t* done_host, uint8_t* success_host);
+
+/* Pre-drawn reset stream of an EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL handle (EARL_ERR_INVALID on any other):
+ * host array f64 [rows, N, 8], row e of env i = the qpos[0:8] of env i's e-th reset (goal[:8] + uniform(-0.3, 0.3),
+ * :72-76).  Every reset that is given no init_qpos -- an auto-reset in the step and earl_tt3_reset(init_qpos NULL) --
+ * takes the next row of the env's column through a per-env cursor, which wraps modulo `rows`.  Must be set before the
+ * first step or reset of such a handle.  Setting it again (same `rows`) replaces the rows and rewinds the cursors.
+ * Device memory: 64 * rows + 4 bytes per env.  Synchronous. */
+EARL_API int earl_tt3_set_reset_stream(earl_tt3_handle* h, const double* qpos_rows_host, int32_t rows);
+
+/* EARL_FLAG_EVAL_STATS: (sum of episode returns, #envs successful at their last step, #envs successful at any step of
+ * the episode, N) -> out4_dev f64 [4], reduced on the device.  A reset clears an env's statistics. */
+EARL_API int earl_tt3_eval_stats(earl_tt3_handle* h, double* out4_dev, void* stream);
 
 /* env._get_obs() (:49-54) */
 EARL_API int earl_tt3_get_obs(earl_tt3_handle* h, float* obs_dev, void* stream);
