@@ -3,9 +3,9 @@
     python -m earl_benchmark_b200.build [--force] [--verbose]
 
 Translation units: the tabletop step and its three-object variant (bit-exact fp64 arithmetic, so no FMA contraction), the articulated-body engine
-of the Sawyer tasks (fp32, FMA on) once per compile-time capacity set (earl_mj_small.cu, earl_mj_large.cu), and the
-dispatcher that exports the earl_mj_* entry points (earl_mj.cu).  The .so is git-ignored but travels to the GPU box with
-the repo snapshot.
+of the Sawyer tasks (fp32, FMA on) once per compile-time capacity set: the primary set that exports the earl_mj_* entry
+points (earl_mj.cu) and the extra-large set of its redo pass (earl_mj_xl.cu); the kitchen engine likewise
+(earl_mj_kitchen.cu, earl_mj_kitchen_xl.cu).  The .so is git-ignored but travels to the GPU box with the repo snapshot.
 """
 import os
 import subprocess
@@ -18,7 +18,7 @@ LIB = os.path.join(PKG, "libearl_b200.so")
 OBJDIR = os.path.join(PKG, "build")
 # (source, extra flags)
 MJ_EXTRA = os.environ.get("EARL_MJ_EXTRA_FLAGS", "").split()  # profiling / trace builds (-DMJ_PHASE_TIMING, -DMJ_TRACE_DEVICE)
-UNITS = [("earl_b200.cu", ["--fmad=false"]), ("earl_tt3.cu", ["--fmad=false"]), ("earl_mj.cu", []), ("earl_mj_small.cu", MJ_EXTRA), ("earl_mj_large.cu", MJ_EXTRA), ("earl_mj_xl.cu", MJ_EXTRA),
+UNITS = [("earl_b200.cu", ["--fmad=false"]), ("earl_tt3.cu", ["--fmad=false"]), ("earl_mj.cu", MJ_EXTRA), ("earl_mj_xl.cu", MJ_EXTRA),
          ("earl_mj_kitchen.cu", MJ_EXTRA), ("earl_mj_kitchen_xl.cu", MJ_EXTRA)]
 SOURCES = [os.path.join(CSRC, u[0]) for u in UNITS]
 DEPS = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(INCLUDE, f) for f in os.listdir(INCLUDE)]

@@ -73,8 +73,9 @@ constexpr int MAXCAND = 1;
 #define MJ_BROAD_SLACK 0.015f
 #endif
 constexpr float BROAD_SLACK = MJ_BROAD_SLACK;  // inflation of the cached broad phase (m)
-// Two capacity sets are compiled from these sources (earl_mj_small.cu / earl_mj_large.cu): the workspace of one
-// environment lives in shared memory, so rows x dofs and contacts decide how many environments one SM keeps in flight.
+// The door / peg engine is compiled twice from these sources: the primary set (earl_mj.cu) and the extra-large set of the
+// redo pass (earl_mj_xl.cu).  The workspace of one environment lives in shared memory, so rows x dofs and contacts decide
+// how many environments one SM keeps in flight.
 #if defined(MJ_CAPSET_KITCHEN)
 #if defined(MJ_CAPSET_KITCHEN_XL)
 // kitchen redo pass (earl_mj_kitchen_xl.cu): the few env steps with a substep beyond the primary set's rows (half a dozen
@@ -101,24 +102,14 @@ constexpr int MAXMG = 64;    // geoms on moving bodies (their world poses are re
 #else
 #if defined(MJ_CAPSET_XL)
 // "extra large": only used by the redo pass that re-steps the few environments whose substep overflowed the primary set
-// (peg wedged in the block, gripper jammed between handle and door: > 24 contacts or > 96 rows)
+// (peg wedged in the block, gripper jammed between handle and door: > 16 contacts or > 64 rows)
 constexpr int MAXEFC = 224; // constraint rows
 constexpr int MAXCON = 56;  // contacts
 constexpr int MAXHIT = 72;  // candidate pairs that survive the broad phase in one substep
-#elif defined(MJ_CAPSET_LARGE)
-constexpr int MAXEFC = 96;  // constraint rows
-constexpr int MAXCON = 24;  // contacts
-constexpr int MAXHIT = 32;  // candidate pairs that survive the broad phase in one substep
 #else
-#ifndef MJ_SMALL_MAXEFC
-#define MJ_SMALL_MAXEFC 64
-#endif
-#ifndef MJ_SMALL_MAXCON
-#define MJ_SMALL_MAXCON 16
-#endif
-constexpr int MAXEFC = MJ_SMALL_MAXEFC;
-constexpr int MAXCON = MJ_SMALL_MAXCON;
-constexpr int MAXHIT = 24;
+constexpr int MAXEFC = 64;  // constraint rows
+constexpr int MAXCON = 16;  // contacts
+constexpr int MAXHIT = 24;  // candidate pairs that survive the broad phase in one substep
 #endif
 constexpr int MAXPAIR = 192; // candidate geom pairs
 constexpr int MAXMG = 16;    // geoms on moving bodies (their world poses are recomputed every substep)

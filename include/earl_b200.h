@@ -30,10 +30,7 @@ extern "C" {
 
 #define EARL_ABI_VERSION 1
 
-#if defined(EARL_MJ_INTERNAL) && defined(__GNUC__)
-/* the library's own per-capacity-set translation units re-declare the entry points under internal names */
-#define EARL_API __attribute__((visibility("hidden")))
-#elif defined(__GNUC__)
+#if defined(__GNUC__)
 #define EARL_API __attribute__((visibility("default")))
 #else
 #define EARL_API

@@ -132,34 +132,60 @@ def test_dense_reward_matches_checker(oracle):
     assert worst < 2e-3 and rmax > rmin + 0.01
 
 
-def test_capacity_overflow_is_redone_by_the_extra_large_set_not_dropped(monkeypatch):
+def test_capacity_overflow_is_redone_by_the_extra_large_set_not_dropped(monkeypatch, oracle):
     """VERDICT r1 weak #3: a substep with more contacts / rows than the handle's fixed capacities used to DROP the excess
     (counted, but that env had left the parity claim).  Now such an env is not stored by the step kernel; the extra-large
     set (56 contacts / 224 rows) re-steps it from its untouched pre-step record in a second, tiny launch.  Random-action
-    rollout of the peg task on the SMALL set (16 contacts / 64 rows: ~1 % of the env steps overflow) against the same
-    rollout on the LARGE set: identical trajectories, overflow_states == 0 on both, and the redo pass did real work."""
-    n, steps = 4096, 160
+    press-down rollout of the peg task (16 contacts / 64 rows in the step kernel: ~1 % of the env steps overflow):
+    overflow_states == 0 and the redo pass did real work.  In each of the last `checked` steps, every env that the fp64
+    checker (64 contacts / 256 rows), stepped from the same state, finds beyond 16 contacts or 64 rows matches it at the
+    tolerances of test_one_step_parity_from_identical_states.  (Of the ~50 envs redone in a step, about a third end it
+    beyond those capacities: the rest overflowed in an earlier substep or were heavy from the step before.)"""
+    n, steps, checked = 4096, 160, 3
     acts = np.random.RandomState(5).uniform(-1, 1, (steps, n, 4)).astype(np.float32)
     acts[:, :, 2] -= 0.35                                  # bias the hands down onto the peg / table: more contacts
 
-    def run(capset, redo="1"):
-        monkeypatch.setenv("EARL_MJ_CAPSET", capset)
+    def run(redo):
+        """the rollout up to its last `checked` steps"""
         monkeypatch.setenv("EARL_MJ_REDO", redo)
         env = sawyer_peg.SawyerPegV2(reward_type="sparse", num_envs=n, device="cuda:0", seed=1)
         env.reset()
-        for t in range(steps):
-            o, r, d, _ = env.step(torch.from_numpy(acts[t]).cuda())
-        return o.cpu().numpy().copy(), env.get_state(), env.work_counters()
+        for t in range(steps - checked):
+            env.step(torch.from_numpy(acts[t]).cuda())
+        return env
 
-    o_s, st_s, wc_s = run("small")
-    o_l, st_l, wc_l = run("large")
-    _, _, wc_drop = run("small", redo="0")
+    env_drop = run("0")
+    for t in range(steps - checked, steps):
+        env_drop.step(torch.from_numpy(acts[t]).cuda())
+    wc_drop = env_drop.work_counters()
     assert wc_drop["overflow_states"] > 50 and wc_drop["redone_states"] == 0          # round 1's behaviour: dropped work
-    assert wc_s["overflow_states"] == 0 and wc_l["overflow_states"] == 0 and wc_s["bad_states"] == 0
-    assert wc_s["redone_states"] > 50 and wc_s["redone_states"] >= wc_l["redone_states"]
-    # same physics whichever set did the work: the capacities only size the workspace
-    dq = np.abs(st_s["qpos"] - st_l["qpos"]).max(axis=1)
-    assert np.median(dq) == 0.0 and (dq < 1e-4).mean() > 0.99, (np.median(dq), (dq < 1e-4).mean(), dq.max())
+    del env_drop
+
+    env = run("1")
+    e, nv = oracle.e, oracle.e.nv
+    worst = dict(q=0.0, v=0.0, obs=0.0)
+    beyond = 0
+    for t in range(steps - checked, steps):
+        before, redone_before = env.get_state(), env.work_counters()["redone_states"]
+        obs, rew, _, _ = env.step(torch.from_numpy(acts[t]).cuda())
+        got, wc, obs, rew = env.get_state(), env.work_counters(), obs.cpu().numpy(), rew.cpu().numpy()
+        assert wc["redone_states"] > redone_before, t
+        for i in range(n):
+            e.reset()
+            e.qpos[:], e.qvel[:], e.mocap_pos[:] = before["qpos"][i], before["qvel"][i], before["mocap_pos"][i]
+            e.arr("qacc_warmstart", (32,))[:nv] = before["qacc_warmstart"][i]
+            ob_ref, r_ref = oracle.step(acts[t, i])
+            if e.ncon <= 16 and e.nefc <= 64:              # within the step kernel's capacities
+                continue
+            beyond += 1
+            worst["q"] = max(worst["q"], np.abs(got["qpos"][i] - e.qpos).max())
+            worst["v"] = max(worst["v"], np.abs(got["qvel"][i] - e.qvel).max())
+            worst["obs"] = max(worst["obs"], np.abs(obs[i] - ob_ref).max())
+            assert float(rew[i]) == r_ref, (t, i)
+    print("peg redo parity:", worst, "env steps beyond 16 contacts / 64 rows", beyond)
+    assert wc["overflow_states"] == 0 and wc["bad_states"] == 0 and wc["redone_states"] > 50
+    assert beyond >= 20
+    assert worst["q"] < TOL and worst["v"] < 5e-4 and worst["obs"] < 1e-5, worst
 
 
 def test_peg_demonstrations_replayed_on_the_device_by_episode():
