@@ -145,7 +145,8 @@ class EARLEnvs(object):
         elif self._env_name == 'kitchen':
             from .envs import kitchen
             kitchen_task = self._kwargs.get('kitchen_task', deployment_eval_config[self._env_name]['task'])
-            eval_env = kitchen.Kitchen(task=kitchen_task, reward_type=self._reward_type, **self._shard_kwargs(1))
+            eval_env = kitchen.Kitchen(task=kitchen_task, reward_type=self._reward_type,
+                                       eval_stats=self._kwargs.get('eval_stats', True), **self._shard_kwargs(1))
         else:
             self._not_built()
         return persistent_state_wrapper.PersistentStateWrapper(eval_env, episode_horizon=self._eval_horizon)

@@ -144,6 +144,7 @@ SIGNATURES = [
     ("earl_mjk_get_state", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mjk_set_state", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mjk_counters", C.c_int, [_VP, C.POINTER(_I64), _VP, _VP, _VP, _VP]),
+    ("earl_mjk_eval_stats", C.c_int, [_VP, _VP, _VP]),
     ("earl_mjk_work_counters", C.c_int, [_VP, _VP]),
     ("earl_mjk_redo_count", _I64, [_VP]),
 ]

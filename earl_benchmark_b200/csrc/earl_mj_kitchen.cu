@@ -34,6 +34,7 @@
 
 #include <cuda_runtime.h>
 
+#include "eval_stats.cuh"
 #include "mj_model_host.hpp"
 #include "mj_step.cuh"
 
@@ -160,6 +161,10 @@ struct TaskArgs {
   const double* ring_table;
   unsigned* ring_cursor;
   int ring_rows;
+  // episode statistics (EARL_FLAG_EVAL_STATS, null otherwise; after the fields above so that their parameter offsets stay):
+  // the return and bit 0 success at any step / bit 1 success at the last step since the env's last reset
+  double* ep_return;                // [N]
+  unsigned char* ep_success;        // [N]
 };
 enum { kRedoCount = 0, kRedoNext = 1, kMainDone = 2, kNextChunk = 3, kSchedWords = 4 };
 
@@ -360,6 +365,10 @@ __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const
       if (failed) { rew = 0.0; ok = false; }
       io.reward_out[env] = rew;
       if (io.success_out) io.success_out[env] = ok;
+      if (a.ep_return) {  // exactly what this step returns (a failed step: 0 and no success)
+        a.ep_return[env] += rew;
+        a.ep_success[env] = (a.ep_success[env] & 1) | (ok ? 3 : 0);
+      }
       const unsigned st = a.steps_since_reset[env] + 1;  // PersistentStateWrapper.step (persistent_state_wrapper.py:22-31)
       a.steps_since_reset[env] = st;
       io.done_out[env] = (long long)st >= a.horizon;
@@ -380,6 +389,7 @@ __device__ __forceinline__ bool task_env(const Model& m, const real* hull, const
       }
     } else {
       a.steps_since_reset[env] = 0;                     // PersistentStateWrapper.reset (:17-20)
+      if (a.ep_return) { a.ep_return[env] = 0.0; a.ep_success[env] = 0; }
       a.steps_since_goal_change[env] = 0;               // LifelongWrapper.reset (:25-28)
       a.num_interventions[env] += 1;
       a.heavy[env] = 0;
@@ -601,6 +611,24 @@ __global__ void mjk_iota_kernel(int* order, int n) {
   if (i < n) order[i] = i;
 }
 
+// (sum of episode returns, #success at the last step, #success at any step, N) -> out4 (pre-zeroed).  ONE block of
+// kEvalThreads: the strided partial sums, the block reduction and the single atomic add onto zero run in a fixed order, so
+// the same per-env values give the same bits on every call (the returns are not integers; multi-block atomics would not).
+constexpr int kEvalThreads = 1024;
+__global__ void __launch_bounds__(kEvalThreads) mjk_eval_stats_kernel(const double* __restrict__ ep_return,
+                                                                     const unsigned char* __restrict__ ep_success, int n,
+                                                                     double* __restrict__ out4) {
+  double ret = 0.0, last = 0.0, any = 0.0, cnt = 0.0;
+  for (int i = threadIdx.x; i < n; i += kEvalThreads) {
+    const unsigned s = ep_success[i];
+    ret += ep_return[i];
+    last += (s & 2u) ? 1.0 : 0.0;
+    any += (s & 1u) ? 1.0 : 0.0;
+    cnt += 1.0;
+  }
+  earl::block_add_eval_stats(ret, last, any, cnt, out4);
+}
+
 }  // namespace
 
 struct earl_mjk_engine {
@@ -753,7 +781,7 @@ int earl_mjk_create(const earl_mjk_config* cfg, const void* model_blob, size_t m
   if (!cfg || !model_blob || !out) return failf(EARL_ERR_INVALID, "null argument");
   *out = nullptr;
   if (cfg->num_envs <= 0 || cfg->frame_skip <= 0 || cfg->episode_horizon <= 0) return failf(EARL_ERR_INVALID, "bad kitchen config");
-  if (cfg->flags & ~(uint32_t)(EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET)) return failf(EARL_ERR_UNSUPPORTED, "unsupported flags %#x", cfg->flags);
+  if (cfg->flags & ~(uint32_t)(EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS)) return failf(EARL_ERR_UNSUPPORTED, "unsupported flags %#x", cfg->flags);
   earl_mjk_engine* eng = nullptr;
   if (int rc = earl_mjk_engine_create(model_blob, model_nbytes, cfg->device, &eng)) return rc;
   earl_mjk_handle* h = new (std::nothrow) earl_mjk_handle();
@@ -792,6 +820,8 @@ int earl_mjk_create(const earl_mjk_config* cfg, const void* model_blob, size_t m
     if ((rc = h->alloc(&a.redo_list, n))) { earl_mjk_destroy(h); return rc; }
   if (const char* e = getenv("EARL_MJ_REDO_SMS")) { const int r = atoi(e); if (r >= 1 && r < eng->sm_count / 8) { h->redo_sms = r; h->redo_sms_fixed = true; } }
   if ((rc = h->alloc(&a.heavy, n))) { earl_mjk_destroy(h); return rc; }
+  if (cfg->flags & EARL_FLAG_EVAL_STATS)
+    if ((rc = h->alloc(&a.ep_return, n)) || (rc = h->alloc(&a.ep_success, n))) { earl_mjk_destroy(h); return rc; }
   if (cudaHostAlloc(reinterpret_cast<void**>(&h->h_redo_seen), sizeof(unsigned), cudaHostAllocDefault) == cudaSuccess) *h->h_redo_seen = 0;
   else { h->h_redo_seen = nullptr; cudaGetLastError(); }
   *out = h;
@@ -924,6 +954,18 @@ int earl_mjk_counters(earl_mjk_handle* h, int64_t* total_steps_host, int64_t* nu
   if (num_interventions_dev) CU(cudaMemcpyAsync(num_interventions_dev, h->a.num_interventions, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
   if (steps_since_reset_dev) CU(cudaMemcpyAsync(steps_since_reset_dev, h->a.steps_since_reset, n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
   if (lifelong_return_dev) CU(cudaMemcpyAsync(lifelong_return_dev, h->a.lifelong_return, n * sizeof(double), cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+
+int earl_mjk_eval_stats(earl_mjk_handle* h, double* out4_dev, void* stream) {
+  if (!h) return failf(EARL_ERR_INVALID, "null handle");
+  if (!out4_dev) return failf(EARL_ERR_INVALID, "null out4");
+  if (!h->a.ep_return) return failf(EARL_ERR_INVALID, "eval stats need EARL_FLAG_EVAL_STATS");
+  CU(cudaSetDevice(h->eng->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  CU(cudaMemsetAsync(out4_dev, 0, 4 * sizeof(double), s));
+  mjk_eval_stats_kernel<<<1, kEvalThreads, 0, s>>>(h->a.ep_return, h->a.ep_success, h->a.n, out4_dev);
+  CU(cudaGetLastError());
   return 0;
 }
 

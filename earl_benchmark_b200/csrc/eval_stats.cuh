@@ -1,5 +1,6 @@
-// eval_stats.cuh -- the device reduction behind earl_eval_stats and earl_tt3_eval_stats: four fp64 per-thread partial sums
-// (episode return, #success at the last step, #success at any step, #envs) reduced over the block and added to out4.
+// eval_stats.cuh -- the device reduction behind earl_eval_stats, earl_tt3_eval_stats and earl_mjk_eval_stats: four fp64
+// per-thread partial sums (episode return, #success at the last step, #success at any step, #envs) reduced over the block
+// and added to out4.
 #pragma once
 
 #include <cuda_runtime.h>

@@ -28,7 +28,7 @@ def init_from_env(backend=None):
 
 def all_reduce_eval_stats(stats, group=None):
     """Sum the [4] float64 statistics tensor of an env's `eval_stats()` over all ranks, in place: the tabletop, the
-    three-object tabletop, sawyer_door and sawyer_peg envs built with `eval_stats=True`.
+    three-object tabletop, sawyer_door, sawyer_peg and kitchen envs built with `eval_stats=True`.
 
     stats = (sum of episode returns, #envs successful at their last step, #envs successful at any step, N).
     Returns a dict with the job-wide means."""

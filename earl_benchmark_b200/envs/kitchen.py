@@ -129,7 +129,7 @@ class Kitchen:
     max_path_length = int(1e8)
 
     def __init__(self, task="all_pairs", reward_type="dense", num_envs=1, device=None, seed=0, env_offset=0, total_envs=None,
-                 model_path=None, auto_reset=False, reset_stream_rows=64, **_unused):
+                 model_path=None, auto_reset=False, reset_stream_rows=64, eval_stats=False, **_unused):
         if reward_type != 'dense':
             raise ValueError("Kitchen environment only supports dense rewards.")     # kitchen.py:91-92
         self._initial_states = copy.deepcopy(initial_states)
@@ -160,6 +160,8 @@ class Kitchen:
         self._auto_reset, self._reset_stream_rows = bool(auto_reset), int(reset_stream_rows)
         if self._reset_stream_rows < 1:
             raise ValueError("reset_stream_rows must be >= 1")
+        # eval_stats=True: every env keeps its episode return and success on the device, reduced by eval_stats()
+        self._eval_stats = bool(eval_stats)
 
     # ------------------------------------------------------------------ reference surface
     def get_task(self):
@@ -201,7 +203,8 @@ class Kitchen:
             return
         cfg = MjkConfig()
         cfg.num_envs, cfg.device, cfg.frame_skip = self.num_envs, self.device.index or 0, FRAME_SKIP
-        cfg.flags = (_lib.FLAG_LIFELONG if self._lifelong else 0) | (_lib.FLAG_AUTO_RESET if self._auto_reset else 0)
+        cfg.flags = (_lib.FLAG_LIFELONG if self._lifelong else 0) | (_lib.FLAG_AUTO_RESET if self._auto_reset else 0) | \
+            (_lib.FLAG_EVAL_STATS if self._eval_stats else 0)
         cfg.episode_horizon = self._episode_horizon
         cfg.goal_change_frequency = self._goal_change_frequency if self._lifelong else 0
         cfg.goal[:] = self.goal.tolist()
@@ -345,6 +348,15 @@ class Kitchen:
         _lib.check(_lib.lib().earl_mjk_counters(self._handle, C.byref(total), interv.data_ptr(), since.data_ptr(),
                                                 None if ll is None else ll.data_ptr(), _stream()))
         return total.value, interv, since, ll
+
+    def eval_stats(self):
+        """float64 CUDA tensor [4] = (sum of episode returns, #envs successful at their last step, #envs successful at any
+        step of the episode, N), reduced on the device in the current stream; needs eval_stats=True.  A reset clears an
+        env's statistics.  Sum it over shards with distributed.all_reduce_eval_stats."""
+        self._ensure()
+        out = torch.empty((4,), dtype=torch.float64, device=self.device)
+        _lib.check(_lib.lib().earl_mjk_eval_stats(self._handle, out.data_ptr(), _stream()))
+        return out
 
     def work_counters(self):
         self._ensure()

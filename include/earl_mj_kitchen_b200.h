@@ -44,7 +44,8 @@ typedef struct earl_mjk_handle earl_mjk_handle;
 
 typedef struct {
   int32_t num_envs, device;
-  uint32_t flags;                 /* EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET (any other flag is rejected) */
+  uint32_t flags;                 /* EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS (any other flag is
+                                     rejected) */
   int32_t frame_skip;             /* 40 (KitchenV0.__init__, kitchen_multitask_v0.py:38) */
   int64_t episode_horizon;        /* PersistentStateWrapper(episode_horizon) */
   int64_t goal_change_frequency;  /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
@@ -100,6 +101,13 @@ EARL_API int earl_mjk_set_state(earl_mjk_handle* h, const double* qpos_host, con
 /* total_steps (host), num_interventions i64 [N], steps_since_reset u32 [N], lifelong_return f64 [N] (device, may be NULL) */
 EARL_API int earl_mjk_counters(earl_mjk_handle* h, int64_t* total_steps_host, int64_t* num_interventions_dev,
                                uint32_t* steps_since_reset_dev, double* lifelong_return_dev, void* stream);
+/* EARL_FLAG_EVAL_STATS: out4_dev f64 [4] = { sum over envs of the episode return, #envs successful at their last step,
+ * #envs successful at any step, N }.  Every step adds the reward it returns to its env's return and records the success
+ * it returns (a failed step adds 0 and is not successful); any reset of an env -- earl_mjk_reset, masked or not, and the
+ * auto-reset after a step -- clears its statistics.  Without auto-reset, steps past the horizon keep accumulating.
+ * Zeroes out4 and reduces in `stream`, on the device, in one block: the same per-env values give the same bits on every
+ * call.  EARL_ERR_INVALID on a handle created without the flag. */
+EARL_API int earl_mjk_eval_stats(earl_mjk_handle* h, double* out4_dev, void* stream);
 /* { env_steps, substeps, newton_iterations, constraint_rows, contacts, bad_states, overflow_states } since creation */
 EARL_API int earl_mjk_work_counters(earl_mjk_handle* h, uint64_t* out7_host);
 /* env steps re-stepped by the extra-large capacity set since creation (a substep of theirs outgrew the 112 rows / 24 contacts of the primary set;
