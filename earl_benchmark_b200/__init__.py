@@ -5,7 +5,9 @@
         .get_envs() / .get_initial_states() / .get_goal_states() / .get_demonstrations() / .has_demos()
 and adds the batched arguments `num_envs`, `device`, `seed`, `state_dtype`, `auto_reset` (with `reset_stream_rows` for
 sawyer_door, sawyer_peg and kitchen), `eval_stats`,
-`rank` / `world_size` (shard a global batch of `num_envs` across processes, one GPU each).
+`rank` / `world_size` (shard a global batch of `num_envs` across processes, one GPU each), and `per_env_goals`
+(tabletop_manipulation, sawyer_door and sawyer_peg: the train and eval envs take a goal vector per env, effective at once,
+through `set_goals(goals, mask=None)` and report them through `get_goals()`; kitchen raises).
 """
 from . import demos
 from .wrappers import lifelong_wrapper, persistent_state_wrapper
@@ -29,6 +31,7 @@ continuing_eval_config = {
 }
 
 _BUILT = ("tabletop_manipulation", "sawyer_door", "sawyer_peg", "kitchen")
+_PER_ENV_GOALS = ("tabletop_manipulation", "sawyer_door", "sawyer_peg")
 
 
 def shard_range(num_envs, rank, world_size):
@@ -59,6 +62,10 @@ class EARLEnvs(object):
         self._batched = dict(device=kwargs.get('device'), seed=int(kwargs.get('seed', 0)),
                              state_dtype=kwargs.get('state_dtype', 'float32'),
                              goal_stream_rows=int(kwargs.get('goal_stream_rows', 64)))
+        if kwargs.get('per_env_goals', False):
+            if env_name not in _PER_ENV_GOALS:
+                raise NotImplementedError(f"{env_name}: per_env_goals is built for {', '.join(_PER_ENV_GOALS)} only")
+            self._batched['per_env_goals'] = True
 
         # resolve to default parameters if not provided by the user (KeyError on unknown env, as the reference)
         if not self._setup_as_lifelong_learning:

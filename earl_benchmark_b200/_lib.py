@@ -19,6 +19,8 @@ FLAG_LIFELONG = 0x08
 FLAG_AUTO_RESET = 0x10
 FLAG_RESET_AT_GOAL = 0x20
 FLAG_EVAL_STATS = 0x40
+FLAG_PER_ENV_GOALS = 0x80
+GOAL_F32, GOAL_F64 = 0, 1
 TABLETOP_MAGIC = 0x54544142
 
 
@@ -73,6 +75,8 @@ SIGNATURES = [
     ("earl_reset", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_set_goal", C.c_int, [_VP, _VP, _VP, _VP]),
     ("earl_set_goal_table", C.c_int, [_VP, _VP, _I32, _I32]),
+    ("earl_set_goals", C.c_int, [_VP, _VP, _I32, _VP, _VP, _VP]),
+    ("earl_get_goals", C.c_int, [_VP, _VP, _VP]),
     ("earl_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_rollout", C.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _VP, _VP, _I32, _VP]),
     ("earl_step_host", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
@@ -117,6 +121,8 @@ SIGNATURES = [
     ("earl_mj_nq", C.c_int, [_VP]),
     ("earl_mj_nv", C.c_int, [_VP]),
     ("earl_mj_set_goal_table", C.c_int, [_VP, _VP, _I32]),
+    ("earl_mj_set_goals", C.c_int, [_VP, _VP, _I32, _VP, _VP, _VP]),
+    ("earl_mj_get_goals", C.c_int, [_VP, _VP, _VP]),
     ("earl_mj_build_reset_template", C.c_int, [_VP, _VP, _VP, _I32]),
     ("earl_mj_set_reset_stream", C.c_int, [_VP, _VP, _VP, _I32, _VP]),
     ("earl_mj_reset", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),

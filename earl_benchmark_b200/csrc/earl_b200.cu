@@ -106,8 +106,11 @@ namespace {
 
 bool f64(const earl_handle* h) { return h->cfg.flags & EARL_FLAG_STATE_F64; }
 
+bool per_env_goals(const earl_handle* h) { return h->cfg.flags & EARL_FLAG_PER_ENV_GOALS; }
+
 bool fast_path(const earl_handle* h) {
-  return !(h->cfg.flags & (EARL_FLAG_DENSE_REWARD | EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS));
+  return !(h->cfg.flags & (EARL_FLAG_DENSE_REWARD | EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS |
+                           EARL_FLAG_PER_ENV_GOALS));
 }
 
 int check_handle(const earl_handle* h) {
@@ -176,9 +179,11 @@ int launch_step_range(earl_handle* h, int first, int count, const float* actions
   const int grid = tiles < h->step_grid ? tiles : h->step_grid;
   if (f64(h)) {
     if (fast) earl::tabletop_step_kernel<true, true><<<grid, earl::kTTBlock, 0, s>>>(p);
+    else if (per_env_goals(h)) earl::tabletop_step_kernel<true, false, 1, true><<<grid, earl::kTTBlock, 0, s>>>(p);
     else earl::tabletop_step_kernel<true, false><<<grid, earl::kTTBlock, 0, s>>>(p);
   } else {
     if (fast) CU(launch_pdl(earl::tabletop_step_kernel<false, true>, grid, s, p));
+    else if (per_env_goals(h)) earl::tabletop_step_kernel<false, false, 1, true><<<grid, earl::kTTBlock, 0, s>>>(p);
     else earl::tabletop_step_kernel<false, false><<<grid, earl::kTTBlock, 0, s>>>(p);
   }
   CU(cudaGetLastError());
@@ -275,6 +280,7 @@ int earl_create(const earl_config* cfg, const void* model_blob, size_t model_nby
   if (!rc) rc = h->alloc(&g64, 256 * 6);
   if (!rc && (cfg->flags & EARL_FLAG_LIFELONG)) { rc = h->alloc(&p.ll_steps, n); if (!rc) rc = h->alloc(&p.ll_return, n); }
   if (!rc && (cfg->flags & EARL_FLAG_EVAL_STATS)) rc = h->alloc(&p.ep_return, n);
+  if (!rc && per_env_goals(h)) rc = h->alloc(&p.env_goal, n * 2);
   if (!rc) rc = h->alloc(&h->d_stats, 4);
   if (rc) { earl_destroy(h); return rc; }
   p.goal_stream = stream_rows;
@@ -294,12 +300,23 @@ int earl_create(const earl_config* cfg, const void* model_blob, size_t model_nby
   earl_tabletop_thresholds(m->threshold, m->success_radius, &p.attach_sq, &p.success_sq);
   for (int k = 0; k < 4; ++k) p.init_qpos[k] = m->initial_state[k];
   rc = upload_goal_tables(h);
+  if (!rc && per_env_goals(h)) {
+    // every env starts on the goal of its (zeroed) meta row, row 0, as a handle without per-env goals does
+    earl::TabletopGoalArgs a{p.goal32, 0, 0, nullptr, nullptr};
+    earl::tabletop_set_goals_kernel<false><<<(p.n + 255) / 256, 256>>>(p, a);
+    cudaError_t le = cudaGetLastError();
+    if (le == cudaSuccess) le = cudaDeviceSynchronize();
+    if (le != cudaSuccess) rc = fail(EARL_ERR_CUDA, "per-env goal initialisation: %s", cudaGetErrorString(le));
+    h->launches += 1;
+  }
   if (rc) { earl_destroy(h); return rc; }
 
   const bool fast = fast_path(h);
   if (f64(h)) rc = fast ? occupancy_grid(earl::tabletop_step_kernel<true, true>, h->sm_count, &h->step_grid)
+                 : per_env_goals(h) ? occupancy_grid(earl::tabletop_step_kernel<true, false, 1, true>, h->sm_count, &h->step_grid)
                         : occupancy_grid(earl::tabletop_step_kernel<true, false>, h->sm_count, &h->step_grid);
   else rc = fast ? occupancy_grid(earl::tabletop_step_kernel<false, true>, h->sm_count, &h->step_grid)
+                 : per_env_goals(h) ? occupancy_grid(earl::tabletop_step_kernel<false, false, 1, true>, h->sm_count, &h->step_grid)
                  : occupancy_grid(earl::tabletop_step_kernel<false, false>, h->sm_count, &h->step_grid);
   if (rc) { earl_destroy(h); return rc; }
   // measured on B200 (DESIGN.md section 4): while the 24 B/env state fits in L2 next to the streams the persistent LSU
@@ -370,6 +387,33 @@ int earl_reset(earl_handle* h, const uint8_t* mask_dev, const int32_t* goal_idx_
 
 int earl_set_goal(earl_handle* h, const uint8_t* mask_dev, const int32_t* goal_idx_dev, void* stream) {
   return reset_impl(h, mask_dev, goal_idx_dev, nullptr, nullptr, 1, stream);
+}
+
+int earl_set_goals(earl_handle* h, const void* goals_dev, int32_t goal_dtype, const uint8_t* mask_dev, float* obs_out_dev,
+                   void* stream) {
+  if (int rc = check_handle(h)) return rc;
+  if (!per_env_goals(h)) return fail(EARL_ERR_INVALID, "earl_set_goals needs a handle created with EARL_FLAG_PER_ENV_GOALS");
+  if (!goals_dev) return fail(EARL_ERR_INVALID, "null goals");
+  if (goal_dtype != EARL_GOAL_F32 && goal_dtype != EARL_GOAL_F64) return fail(EARL_ERR_INVALID, "goal_dtype must be EARL_GOAL_F32 or EARL_GOAL_F64");
+  if ((uintptr_t)obs_out_dev & 15u) return fail(EARL_ERR_INVALID, "obs_out must be 16-byte aligned");
+  earl::TabletopGoalArgs a{goals_dev, goal_dtype == EARL_GOAL_F64, 6, mask_dev, obs_out_dev};
+  const int grid = (h->p.n + 255) / 256;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (f64(h)) earl::tabletop_set_goals_kernel<true><<<grid, 256, 0, s>>>(h->p, a);
+  else earl::tabletop_set_goals_kernel<false><<<grid, 256, 0, s>>>(h->p, a);
+  CU(cudaGetLastError());
+  h->launches += 1;
+  return note_stream(h, s);
+}
+
+int earl_get_goals(earl_handle* h, float* goals_out_dev, void* stream) {
+  if (int rc = check_handle(h)) return rc;
+  if (!per_env_goals(h)) return fail(EARL_ERR_INVALID, "earl_get_goals needs a handle created with EARL_FLAG_PER_ENV_GOALS");
+  if (!goals_out_dev) return fail(EARL_ERR_INVALID, "null goals_out");
+  // the first 6 of the 8 floats of every env's slot
+  CU(cudaMemcpy2DAsync(goals_out_dev, 6 * sizeof(float), h->p.env_goal, 2 * sizeof(float4), 6 * sizeof(float), (size_t)h->p.n,
+                       cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
+  return 0;
 }
 
 int earl_step(earl_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev,

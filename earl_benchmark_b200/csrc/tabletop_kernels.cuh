@@ -41,7 +41,7 @@ constexpr uint32_t kGoalMask = 0xffu << kGoalShift;
 
 // feature bits (mirror EARL_FLAG_*)
 constexpr uint32_t kDense = 0x01u, kWide = 0x02u, kF64 = 0x04u, kLifelong = 0x08u, kAutoReset = 0x10u,
-                   kResetAtGoal = 0x20u, kEvalStats = 0x40u;
+                   kResetAtGoal = 0x20u, kEvalStats = 0x40u, kPerEnvGoals = 0x80u;
 
 struct TabletopParams {
   // hot state
@@ -81,6 +81,9 @@ struct TabletopParams {
   double attach_sq;
   float success_sq;
   double init_qpos[4];
+  // EARL_FLAG_PER_ENV_GOALS: the goal each env pursues, [N][2] float4 (goal[0:4], goal[4:6] + 2 pad), null otherwise.
+  // Every assignment of a goal row (reset, reset_goal, lifelong swap, auto-reset) also copies that row here.
+  float4* env_goal;
 };
 
 // Programmatic dependent launch: step t+1 may be scheduled while step t drains; nothing of the state is
@@ -206,9 +209,12 @@ __device__ __forceinline__ void tt_store_obs_tile(float* __restrict__ obs, const
 }
 
 // The hot kernel.  FAST = sparse reward, no lifelong / auto-reset / eval-stats (the headline config);
-// the general instantiation handles every feature with warp-uniform runtime branches.
-template <bool F64, bool FAST, int MINB = 1>
+// the general instantiation handles every feature with warp-uniform runtime branches.  GOALS (general kernel only) =
+// EARL_FLAG_PER_ENV_GOALS: each env's goal is streamed from p.env_goal (+32 B read per env step) instead of being
+// looked up in the goal table through the row in meta.
+template <bool F64, bool FAST, int MINB = 1, bool GOALS = false>
 __global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const TabletopParams p) {
+  static_assert(!(FAST && GOALS), "per-env goals run on the general kernel");
   __shared__ __align__(16) float tiles[kTTBlock / 32][32 * kTTObs];
   pdl_wait_prior_grid();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -231,8 +237,13 @@ __global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const Tab
       const float a1 = __ldcs(p.actions + (size_t)i * kTTAct + 1);
       const float a2 = __ldcs(p.actions + (size_t)i * kTTAct + 2);
       uint32_t gi = (s.flags & kGoalMask) >> kGoalShift;
-      g0 = __ldg(p.goal32 + 2 * gi);
-      g1 = __ldg(p.goal32 + 2 * gi + 1);
+      if (GOALS) {
+        g0 = p.env_goal[2 * (size_t)i];
+        g1 = p.env_goal[2 * (size_t)i + 1];
+      } else {
+        g0 = __ldg(p.goal32 + 2 * gi);
+        g1 = __ldg(p.goal32 + 2 * gi + 1);
+      }
 
       tt_move(s, a0, a1, a2, p);
       pos32 = make_float4(__double2float_rn(s.fx), __double2float_rn(s.fy), __double2float_rn(s.mx),
@@ -261,6 +272,7 @@ __global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const Tab
             s.flags = (s.flags & ~kGoalMask) | (gi << kGoalShift);
             g0 = __ldg(p.goal32 + 2 * gi);  // the returned obs carries the NEW goal, the reward the old one
             g1 = __ldg(p.goal32 + 2 * gi + 1);
+            if (GOALS) { p.env_goal[2 * (size_t)i] = g0; p.env_goal[2 * (size_t)i + 1] = g1; }
           }
           p.ll_steps[i] = ls;
         }
@@ -273,6 +285,7 @@ __global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const Tab
           s.flags = gi << kGoalShift;
           g0 = __ldg(p.goal32 + 2 * gi);
           g1 = __ldg(p.goal32 + 2 * gi + 1);
+          if (GOALS) { p.env_goal[2 * (size_t)i] = g0; p.env_goal[2 * (size_t)i + 1] = g1; }
           if (p.features & kResetAtGoal) {
             const double* g = p.goal64 + 6 * gi;
             s.fx = g[0]; s.fy = g[1]; s.mx = g[2]; s.my = g[3];
@@ -420,6 +433,10 @@ __global__ void tabletop_reset_kernel(const TabletopParams p, const TabletopRese
     gi = p.goal_stream[(size_t)(c % (uint32_t)p.goal_stream_rows) * p.n_total + i];
     p.goal_cursor[i] = c + 1u;
   }
+  if (p.env_goal) {  // the assigned row replaces any goal set with earl_set_goals
+    p.env_goal[2 * (size_t)i] = p.goal32[2 * gi];
+    p.env_goal[2 * (size_t)i + 1] = p.goal32[2 * gi + 1];
+  }
   if (a.set_goal_only) {
     s.flags = (s.flags & ~kGoalMask) | (gi << kGoalShift);
   } else {
@@ -459,11 +476,55 @@ __global__ void tabletop_get_obs_kernel(const TabletopParams p, float* __restric
   uint32_t steps;
   tt_load_state<F64>(p, i, s, steps);
   const uint32_t gi = (s.flags & kGoalMask) >> kGoalShift;
-  const float4 g0 = p.goal32[2 * gi], g1 = p.goal32[2 * gi + 1];
+  const float4* g = p.env_goal ? p.env_goal + 2 * (size_t)i : p.goal32 + 2 * gi;
+  const float4 g0 = g[0], g1 = g[1];
   const float att = (s.flags & kAttached) ? 0.f : -1.f;
   float4* row = reinterpret_cast<float4*>(obs + (size_t)i * kTTObs);
   row[0] = make_float4(__double2float_rn(s.fx), __double2float_rn(s.fy), __double2float_rn(s.mx),
                        __double2float_rn(s.my));
+  row[1] = make_float4(att, att, g0.x, g0.y);
+  row[2] = make_float4(g0.z, g0.w, g1.x, g1.y);
+}
+
+// earl_set_goals: env i (mask[i] != 0, or every env when mask is null) pursues goals[i * goal_stride .. + 6] from now on,
+// fp64 input rounded to fp32 as the goal-table upload rounds it; then the observation row of EVERY env (the current one
+// for envs outside the mask) goes to obs_out when it is non-null.  The goal row in meta is left alone: it is what the
+// snapshot records, and the next row assignment overrides the custom goal.
+struct TabletopGoalArgs {
+  const void* goals;   // f32 or f64 [N][goal_stride]
+  int goal_f64;
+  int goal_stride;     // 6, or 0 = the same goal for every env
+  const uint8_t* mask;
+  float* obs_out;
+};
+
+template <bool F64>
+__global__ void tabletop_set_goals_kernel(const TabletopParams p, const TabletopGoalArgs a) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.n) return;
+  float4 g0, g1;
+  if (!a.mask || a.mask[i]) {
+    float v[6];
+    const size_t at = (size_t)a.goal_stride * i;
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+      v[k] = a.goal_f64 ? __double2float_rn(static_cast<const double*>(a.goals)[at + k]) : static_cast<const float*>(a.goals)[at + k];
+    g0 = make_float4(v[0], v[1], v[2], v[3]);
+    g1 = make_float4(v[4], v[5], 0.f, 0.f);
+    p.env_goal[2 * (size_t)i] = g0;
+    p.env_goal[2 * (size_t)i + 1] = g1;
+  } else {
+    if (!a.obs_out) return;
+    g0 = p.env_goal[2 * (size_t)i];
+    g1 = p.env_goal[2 * (size_t)i + 1];
+  }
+  if (!a.obs_out) return;
+  TTState s;
+  uint32_t steps;
+  tt_load_state<F64>(p, i, s, steps);
+  const float att = (s.flags & kAttached) ? 0.f : -1.f;
+  float4* row = reinterpret_cast<float4*>(a.obs_out + (size_t)i * kTTObs);
+  row[0] = make_float4(__double2float_rn(s.fx), __double2float_rn(s.fy), __double2float_rn(s.mx), __double2float_rn(s.my));
   row[1] = make_float4(att, att, g0.x, g0.y);
   row[2] = make_float4(g0.z, g0.w, g1.x, g1.y);
 }

@@ -9,6 +9,7 @@ import numpy as np
 import torch
 
 from .. import _lib, rng
+from ._goals import goal_args
 from ._hostio import HostBuffers
 from ..mjcf.compile import Model
 from ..spaces import Box
@@ -35,7 +36,7 @@ class SawyerBatchedEnv:
 
     def __init__(self, reward_type="sparse", reset_at_goal=False, num_envs=1, device=None, seed=0, eval_stats=False,
                  env_offset=0, total_envs=None, model_path=None, max_newton=0, host_io=False, auto_reset=False,
-                 reset_stream_rows=64, **_tabletop_only):
+                 reset_stream_rows=64, per_env_goals=False, **_tabletop_only):
         name = type(self).__name__
         if reward_type == "dense" and not self.HAS_DENSE_REWARD:
             raise NotImplementedError(f"{name}: the dense reward (metaworld reward_utils, gripper caging) is not built yet")
@@ -73,6 +74,8 @@ class SawyerBatchedEnv:
         self._reset_stream_rows = int(reset_stream_rows)
         if self._reset_stream_rows < 1:
             raise ValueError("reset_stream_rows must be >= 1")
+        # per_env_goals=True: every env can be given its own goal vector, effective at once (set_goals / get_goals)
+        self._per_env_goals = bool(per_env_goals)
 
     # ------------------------------------------------------------------ task hooks
     def _task_spec(self):
@@ -106,6 +109,7 @@ class SawyerBatchedEnv:
         L = _lib.lib()
         flags = (_lib.FLAG_EVAL_STATS if self._eval_stats else 0) | (_lib.FLAG_LIFELONG if self._lifelong else 0)
         flags |= _lib.FLAG_AUTO_RESET if self._auto_reset else 0
+        flags |= _lib.FLAG_PER_ENV_GOALS if self._per_env_goals else 0
         if self._reward_type == "dense":
             flags |= _lib.FLAG_DENSE_REWARD
         cfg = _lib.MjConfig(self.ENV_KIND, self.num_envs, self.device.index or 0, flags, self._episode_horizon,
@@ -169,6 +173,33 @@ class SawyerBatchedEnv:
     @property
     def goal(self):
         return np.stack([self._goal_table[r] for r in self._goal_rows.cpu().numpy()])
+
+    def set_goals(self, goals, mask=None):
+        """reset_goal(goal) with any goal per env, effective at once (per_env_goals=True envs only).
+
+        goals: CUDA float32 / float64 tensor [N,7], or [7] for every env; mask: CUDA bool / uint8 [N] or None (all envs).
+        The masked envs pursue their new goal from now on: the returned observation [N,14] carries it (the other rows are
+        the current observation) and the next step's reward (sparse and dense), success, statistics and lifelong return are
+        measured against it.  float64 goals are rounded to float32 as the goal table rounds them.  The goal the next reset
+        assigns (reset_goal) is unchanged, so a reset, auto-reset or lifelong goal swap gives the env the task's goal back.
+        One launch on the current stream, no synchronisation.  host_io=True envs also take numpy / CPU input and return
+        numpy."""
+        if not self._per_env_goals:
+            raise RuntimeError("set_goals needs an env built with per_env_goals=True")
+        self._ensure()
+        g, dtype, m = goal_args(goals, mask, self.num_envs, 7, self.device, self._host_mode)
+        obs = torch.empty((self.num_envs, OBS_DIM), dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().earl_mj_set_goals(self._handle, g.data_ptr(), dtype, _ptr(m), obs.data_ptr(), _stream()))
+        return obs.cpu().numpy() if self._host_mode else obs
+
+    def get_goals(self):
+        """CUDA float32 [N,7]: the goal every env pursues now (per_env_goals=True envs only)."""
+        if not self._per_env_goals:
+            raise RuntimeError("get_goals needs an env built with per_env_goals=True")
+        self._ensure()
+        out = torch.empty((self.num_envs, 7), dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().earl_mj_get_goals(self._handle, out.data_ptr(), _stream()))
+        return out
 
     # ------------------------------------------------------------------ reset / step
     def _mask(self, mask):

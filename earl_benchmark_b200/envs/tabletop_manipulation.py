@@ -19,6 +19,7 @@ import torch
 
 from .. import _lib, rng
 from . import _hostio
+from ._goals import goal_args
 from ._hostio import HostBuffers
 from ..spaces import Box
 
@@ -48,12 +49,14 @@ class TabletopManipulation:
     Reference-compatible arguments: task_list, reward_type, reset_at_goal, wide_init_distr
     (tabletop_manipulation.py:24-28).  Batched extras: num_envs, device, seed, state_dtype ('float32' |
     'float64'), goal_stream_rows, auto_reset, eval_stats, env_offset/total_envs (this shard's slice of a
-    larger job: the goal stream is drawn for `total_envs` envs and columns [env_offset, env_offset+N) kept).
+    larger job: the goal stream is drawn for `total_envs` envs and columns [env_offset, env_offset+N) kept),
+    per_env_goals (every env keeps its own goal vector: set_goals() / get_goals()).
     """
 
     def __init__(self, task_list="rc_r-rc_k-rc_g-rc_b", reward_type="dense", reset_at_goal=False,
                  wide_init_distr=False, num_envs=1, device=None, seed=0, state_dtype="float32",
-                 goal_stream_rows=64, auto_reset=False, eval_stats=False, env_offset=0, total_envs=None, host_io=False):
+                 goal_stream_rows=64, auto_reset=False, eval_stats=False, env_offset=0, total_envs=None, host_io=False,
+                 per_env_goals=False):
         if reward_type not in ("sparse", "dense"):
             raise ValueError(f"reward_type must be 'sparse' or 'dense', got {reward_type!r}")
         if state_dtype not in ("float32", "float64"):
@@ -68,6 +71,7 @@ class TabletopManipulation:
         self._goal_stream_rows = int(goal_stream_rows)
         self._auto_reset = bool(auto_reset)
         self._eval_stats = bool(eval_stats)
+        self._per_env_goals = bool(per_env_goals)
         self._env_offset = int(env_offset)
         self._total_envs = int(total_envs) if total_envs is not None else self.num_envs + self._env_offset
         if device is None:
@@ -140,6 +144,8 @@ class TabletopManipulation:
             f |= _lib.FLAG_RESET_AT_GOAL
         if self._eval_stats:
             f |= _lib.FLAG_EVAL_STATS
+        if self._per_env_goals:
+            f |= _lib.FLAG_PER_ENV_GOALS
         return f
 
     def _model_blob(self):
@@ -250,8 +256,36 @@ class TabletopManipulation:
     @property
     def goal(self):
         """Current goals [N,6] float64 (reference attribute `self.goal`)."""
+        if self._per_env_goals:
+            return self.get_goals().cpu().numpy().astype(np.float64)
         snap = self.get_state()
         return np.stack([self._goal_table[r] for r in snap["goal_row"]])
+
+    def set_goals(self, goals, mask=None):
+        """reset_goal(goal) with any goal per env, effective at once (per_env_goals=True envs only).
+
+        goals: CUDA float32 / float64 tensor [N,6], or [6] for every env; mask: CUDA bool / uint8 [N] or None (all envs).
+        The masked envs pursue their new goal from now on: the returned observation [N,12] carries it (the other rows are
+        the current observation) and the next step's reward, success, statistics and lifelong return are measured against
+        it.  float64 goals are rounded to float32 as the goal table rounds them.  A later reset, reset_goal, lifelong goal
+        swap or auto-reset gives the env the task's goal back.  One launch on the current stream, no synchronisation.
+        host_io=True envs also take numpy / CPU input and return numpy."""
+        if not self._per_env_goals:
+            raise RuntimeError("set_goals needs an env built with per_env_goals=True")
+        self._ensure()
+        g, dtype, m = goal_args(goals, mask, self.num_envs, 6, self.device, self._host_mode)
+        obs = torch.empty((self.num_envs, OBS_DIM), dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().earl_set_goals(self._handle, g.data_ptr(), dtype, _ptr(m), obs.data_ptr(), _stream()))
+        return obs.cpu().numpy() if self._host_mode else obs
+
+    def get_goals(self):
+        """CUDA float32 [N,6]: the goal every env pursues now (per_env_goals=True envs only)."""
+        if not self._per_env_goals:
+            raise RuntimeError("get_goals needs an env built with per_env_goals=True")
+        self._ensure()
+        out = torch.empty((self.num_envs, 6), dtype=torch.float32, device=self.device)
+        _lib.check(_lib.lib().earl_get_goals(self._handle, out.data_ptr(), _stream()))
+        return out
 
     # ------------------------------------------------------------------ reset / step
     def _mask(self, mask):

@@ -63,6 +63,11 @@ typedef enum {
 #define EARL_FLAG_AUTO_RESET 0x10u    /* reset inside the step kernel when the horizon fires (throughput runs) */
 #define EARL_FLAG_RESET_AT_GOAL 0x20u /* reset_at_goal=True: resets place the env at its new goal (:109-111) */
 #define EARL_FLAG_EVAL_STATS 0x40u    /* accumulate per-env episode return / success for earl_eval_stats */
+#define EARL_FLAG_PER_ENV_GOALS 0x80u /* every env keeps its own goal vector, set on the device (earl_set_goals) */
+
+/* goal_dtype of earl_set_goals / earl_mj_set_goals */
+#define EARL_GOAL_F32 0
+#define EARL_GOAL_F64 1
 
 typedef struct {
   int32_t env_kind;              /* earl_env_kind */
@@ -132,6 +137,21 @@ EARL_API int earl_set_goal(earl_handle* h, const uint8_t* mask_dev, const int32_
 
 /* Replace rows of the goal table (custom goals passed to reset_goal(goal)). */
 EARL_API int earl_set_goal_table(earl_handle* h, const double* rows_host /*[count,6]*/, int32_t first_row, int32_t count);
+
+/* env.reset_goal(goal) with an arbitrary goal per env, on an EARL_FLAG_PER_ENV_GOALS handle
+ * (tabletop_manipulation.py:78-81, without the goal table): every env with mask[i] != 0 (mask NULL = all) pursues
+ * goals[i,:] from now on -- the next step's reward, success, statistics and lifelong return are measured against it.
+ * goals is [N,6] f32 (EARL_GOAL_F32) or f64 (EARL_GOAL_F64, rounded to f32 as the goal-table upload rounds it).
+ * Writes the observation row of EVERY env to obs_out [N,12] when non-NULL (16-byte aligned): the new goal for the
+ * masked envs, the current observation for the others.  One launch on `stream`; no host synchronisation.
+ * Any later assignment of a goal row (reset, earl_set_goal, lifelong goal swap, auto-reset) replaces the env's goal
+ * with that row's; snapshots (earl_get_state / earl_set_state) neither record nor change the per-env goals. */
+EARL_API int earl_set_goals(earl_handle* h, const void* goals_dev, int32_t goal_dtype, const uint8_t* mask_dev,
+                            float* obs_out_dev, void* stream);
+
+/* env.goal: the goal every env pursues now, f32 [N,6], on an EARL_FLAG_PER_ENV_GOALS handle.  A device-to-device
+ * copy on `stream`, no launch. */
+EARL_API int earl_get_goals(earl_handle* h, float* goals_out_dev, void* stream);
 
 /* ---------------------------------------------------------------- the hot path
  * One PersistentStateWrapper.step (persistent_state_wrapper.py:22-31) of every env, i.e. env.step

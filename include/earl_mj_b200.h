@@ -23,7 +23,8 @@ typedef struct {
   int32_t env_kind;         /* EARL_ENV_SAWYER_DOOR or EARL_ENV_SAWYER_PEG */
   int32_t num_envs;
   int32_t device;
-  uint32_t flags;           /* EARL_FLAG_EVAL_STATS | EARL_FLAG_LIFELONG | EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET */
+  uint32_t flags;           /* EARL_FLAG_EVAL_STATS | EARL_FLAG_LIFELONG | EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET |
+                               EARL_FLAG_PER_ENV_GOALS */
   int64_t episode_horizon;  /* PersistentStateWrapper(episode_horizon), persistent_state_wrapper.py:10-12 */
   int64_t goal_change_frequency; /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
 } earl_mj_config;
@@ -64,6 +65,20 @@ EARL_API int earl_mj_nv(const earl_mj_handle* h);
 
 /* Goal table, f64 [count,7] on the host (goal_states, sawyer_door.py:15-16; reset_goal(goal) for custom goals). */
 EARL_API int earl_mj_set_goal_table(earl_mj_handle* h, const double* rows_host, int32_t count);
+
+/* env.reset_goal(goal) with an arbitrary goal per env, taking effect at once, on an EARL_FLAG_PER_ENV_GOALS handle
+ * (sawyer_door.py:100-102; door and peg reset_goal() sets the goal that _get_obs() and compute_reward() read).
+ * Such a handle has a private goal row per env next to the goal table: every env with mask[i] != 0 (mask NULL = all)
+ * gets goals[i,:] in its private row and points its state record at it, so the next step's observation, sparse and
+ * dense reward, success, statistics and lifelong return are measured against it.  goals is [N,7] f32 (EARL_GOAL_F32)
+ * or f64 (EARL_GOAL_F64, rounded to f32 as earl_mj_set_goal_table rounds it).  Writes the observation row of EVERY env
+ * to obs_out [N,14] when non-NULL (the current observation for envs outside the mask).  One launch on `stream`; no host
+ * synchronisation.  The goal row the next reset assigns (goal_idx / the reset stream / row 0) is not changed, so a reset
+ * -- host, auto-reset or the lifelong goal swap -- gives the env the task's goal back. */
+EARL_API int earl_mj_set_goals(earl_mj_handle* h, const void* goals_dev, int32_t goal_dtype, const uint8_t* mask_dev,
+                               float* obs_out_dev, void* stream);
+/* The goal every env pursues now, f32 [N,7], on an EARL_FLAG_PER_ENV_GOALS handle (one launch on `stream`). */
+EARL_API int earl_mj_get_goals(earl_mj_handle* h, float* goals_out_dev, void* stream);
 
 /* sim.reset() + SawyerXYZEnv._reset_hand(steps): from qpos0, `steps` times { mocap_pos <- hand_init_pos; mocap_quat <-
  * [1,0,1,0]; do_simulation(ctrl, frame_skip) }.  Deterministic, so it is run ONCE on the device and the resulting
