@@ -7,7 +7,9 @@ and adds the batched arguments `num_envs`, `device`, `seed`, `state_dtype`, `aut
 sawyer_door, sawyer_peg and kitchen), `eval_stats`,
 `rank` / `world_size` (shard a global batch of `num_envs` across processes, one GPU each), and `per_env_goals`
 (tabletop_manipulation, sawyer_door and sawyer_peg: the train and eval envs take a goal vector per env, effective at once,
-through `set_goals(goals, mask=None)` and report them through `get_goals()`; kitchen raises).
+through `set_goals(goals, mask=None)` and report them through `get_goals()`; kitchen raises), and `final_obs` (with
+`auto_reset`: the train env's step() adds info["final_observation"], the last observation of every episode the step ended;
+eval envs never auto-reset and do not take it).
 """
 from . import demos
 from .wrappers import lifelong_wrapper, persistent_state_wrapper
@@ -53,6 +55,8 @@ class EARLEnvs(object):
         self._reset_train_env_at_goal = reset_train_env_at_goal
         self._setup_as_lifelong_learning = setup_as_lifelong_learning
         self._kwargs = kwargs
+        if kwargs.get('final_obs', False) and not kwargs.get('auto_reset', False):
+            raise ValueError("final_obs=True needs auto_reset=True: without it, the observation step() returns on done is the final one")
 
         # batched / device arguments (not in the reference)
         self._num_envs = int(kwargs.get('num_envs', 1))
@@ -90,7 +94,8 @@ class EARLEnvs(object):
     def _auto_reset_kwargs(self):
         """train envs of the articulated-body tasks: reset in the step when the horizon fires (eval envs never do)"""
         return dict(auto_reset=bool(self._kwargs.get('auto_reset', False)),
-                    reset_stream_rows=int(self._kwargs.get('reset_stream_rows', 64)))
+                    reset_stream_rows=int(self._kwargs.get('reset_stream_rows', 64)),
+                    final_obs=bool(self._kwargs.get('final_obs', False)))
 
     def _not_built(self):
         raise NotImplementedError(
@@ -106,6 +111,7 @@ class EARLEnvs(object):
                 reset_at_goal=self._reset_train_env_at_goal,
                 wide_init_distr=self._kwargs.get('wide_init_distr', False),
                 auto_reset=self._kwargs.get('auto_reset', False),
+                final_obs=self._kwargs.get('final_obs', False),
                 eval_stats=False,
                 **self._shard_kwargs(0))
         elif self._env_name == 'sawyer_door':

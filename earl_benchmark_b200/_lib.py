@@ -20,6 +20,7 @@ FLAG_AUTO_RESET = 0x10
 FLAG_RESET_AT_GOAL = 0x20
 FLAG_EVAL_STATS = 0x40
 FLAG_PER_ENV_GOALS = 0x80
+FLAG_FINAL_OBS = 0x100
 GOAL_F32, GOAL_F64 = 0, 1
 TABLETOP_MAGIC = 0x54544142
 
@@ -77,6 +78,7 @@ SIGNATURES = [
     ("earl_set_goal_table", C.c_int, [_VP, _VP, _I32, _I32]),
     ("earl_set_goals", C.c_int, [_VP, _VP, _I32, _VP, _VP, _VP]),
     ("earl_get_goals", C.c_int, [_VP, _VP, _VP]),
+    ("earl_set_final_obs", C.c_int, [_VP, _VP]),
     ("earl_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_rollout", C.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _VP, _VP, _I32, _VP]),
     ("earl_step_host", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
@@ -111,6 +113,7 @@ SIGNATURES = [
     ("earl_tt3_get_state", C.c_int, [_VP, _VP, _VP, _VP]),
     ("earl_tt3_set_state", C.c_int, [_VP, _VP, _VP, _VP]),
     ("earl_tt3_set_reset_stream", C.c_int, [_VP, _VP, _I32]),
+    ("earl_tt3_set_final_obs", C.c_int, [_VP, _VP]),
     ("earl_tt3_eval_stats", C.c_int, [_VP, _VP, _VP]),
     ("earl_tt3_launch_count", _I64, [_VP]),
     # include/earl_mj_b200.h
@@ -127,6 +130,7 @@ SIGNATURES = [
     ("earl_mj_set_reset_stream", C.c_int, [_VP, _VP, _VP, _I32, _VP]),
     ("earl_mj_reset", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mj_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    ("earl_mj_set_final_obs", C.c_int, [_VP, _VP]),
     ("earl_mj_step_host", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mj_get_obs", C.c_int, [_VP, _VP, _VP]),
     ("earl_mj_get_state", C.c_int, [_VP, _VP, _VP, _VP, _VP]),
@@ -147,6 +151,7 @@ SIGNATURES = [
     ("earl_mjk_set_reset_stream", C.c_int, [_VP, _VP, _I32, _VP, _I32]),
     ("earl_mjk_reset", C.c_int, [_VP, _VP, C.c_int32, _VP, _VP, _VP]),
     ("earl_mjk_step", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    ("earl_mjk_set_final_obs", C.c_int, [_VP, _VP]),
     ("earl_mjk_get_state", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mjk_set_state", C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP]),
     ("earl_mjk_counters", C.c_int, [_VP, C.POINTER(_I64), _VP, _VP, _VP, _VP]),

@@ -86,6 +86,7 @@ struct earl_handle {
   cudaEvent_t order_ev = nullptr;
   bool order_pending = false;
   double* d_stats = nullptr;
+  float* final_obs = nullptr;  // EARL_FLAG_FINAL_OBS: the caller's [N,12] buffer (earl_set_final_obs)
 
   template <typename T>
   int alloc(T** ptr, size_t count, bool zero = true) {
@@ -107,6 +108,8 @@ namespace {
 bool f64(const earl_handle* h) { return h->cfg.flags & EARL_FLAG_STATE_F64; }
 
 bool per_env_goals(const earl_handle* h) { return h->cfg.flags & EARL_FLAG_PER_ENV_GOALS; }
+
+bool has_final_obs(const earl_handle* h) { return h->cfg.flags & EARL_FLAG_FINAL_OBS; }
 
 bool fast_path(const earl_handle* h) {
   return !(h->cfg.flags & (EARL_FLAG_DENSE_REWARD | EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS |
@@ -177,7 +180,12 @@ int launch_step_range(earl_handle* h, int first, int count, const float* actions
     return 0;
   }
   const int grid = tiles < h->step_grid ? tiles : h->step_grid;
-  if (f64(h)) {
+  if (has_final_obs(h)) {
+    if (f64(h) && per_env_goals(h)) earl::tabletop_step_kernel<true, false, 1, true, true><<<grid, earl::kTTBlock, 0, s>>>(p, h->final_obs);
+    else if (f64(h)) earl::tabletop_step_kernel<true, false, 1, false, true><<<grid, earl::kTTBlock, 0, s>>>(p, h->final_obs);
+    else if (per_env_goals(h)) earl::tabletop_step_kernel<false, false, 1, true, true><<<grid, earl::kTTBlock, 0, s>>>(p, h->final_obs);
+    else earl::tabletop_step_kernel<false, false, 1, false, true><<<grid, earl::kTTBlock, 0, s>>>(p, h->final_obs);
+  } else if (f64(h)) {
     if (fast) earl::tabletop_step_kernel<true, true><<<grid, earl::kTTBlock, 0, s>>>(p);
     else if (per_env_goals(h)) earl::tabletop_step_kernel<true, false, 1, true><<<grid, earl::kTTBlock, 0, s>>>(p);
     else earl::tabletop_step_kernel<true, false><<<grid, earl::kTTBlock, 0, s>>>(p);
@@ -203,6 +211,12 @@ int note_stream(earl_handle* h, cudaStream_t s) {
   if (!h->order_ev) CU(cudaEventCreateWithFlags(&h->order_ev, cudaEventDisableTiming));
   CU(cudaEventRecord(h->order_ev, s));
   h->order_pending = true;
+  return 0;
+}
+
+// a final-observation handle steps only once its buffer is registered, like an auto-reset handle with a stream
+int check_final_obs(const earl_handle* h) {
+  if (has_final_obs(h) && !h->final_obs) return fail(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS handles need earl_set_final_obs before the first step");
   return 0;
 }
 
@@ -242,6 +256,8 @@ int earl_create(const earl_config* cfg, const void* model_blob, size_t model_nby
   if (cfg->episode_horizon < 1) return fail(EARL_ERR_INVALID, "episode_horizon must be >= 1");
   if ((cfg->flags & EARL_FLAG_LIFELONG) && cfg->goal_change_frequency < 1)
     return fail(EARL_ERR_INVALID, "lifelong handles need goal_change_frequency >= 1");
+  if ((cfg->flags & EARL_FLAG_FINAL_OBS) && !(cfg->flags & EARL_FLAG_AUTO_RESET))
+    return fail(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS needs EARL_FLAG_AUTO_RESET");
   if (!model_blob || model_nbytes != sizeof(earl_tabletop_model))
     return fail(EARL_ERR_INVALID, "model blob must be an earl_tabletop_model (%zu B), got %zu B", sizeof(earl_tabletop_model), model_nbytes);
   const earl_tabletop_model* m = static_cast<const earl_tabletop_model*>(model_blob);
@@ -312,7 +328,12 @@ int earl_create(const earl_config* cfg, const void* model_blob, size_t model_nby
   if (rc) { earl_destroy(h); return rc; }
 
   const bool fast = fast_path(h);
-  if (f64(h)) rc = fast ? occupancy_grid(earl::tabletop_step_kernel<true, true>, h->sm_count, &h->step_grid)
+  if (has_final_obs(h))
+    rc = f64(h) ? (per_env_goals(h) ? occupancy_grid(earl::tabletop_step_kernel<true, false, 1, true, true>, h->sm_count, &h->step_grid)
+                                    : occupancy_grid(earl::tabletop_step_kernel<true, false, 1, false, true>, h->sm_count, &h->step_grid))
+                : (per_env_goals(h) ? occupancy_grid(earl::tabletop_step_kernel<false, false, 1, true, true>, h->sm_count, &h->step_grid)
+                                    : occupancy_grid(earl::tabletop_step_kernel<false, false, 1, false, true>, h->sm_count, &h->step_grid));
+  else if (f64(h)) rc = fast ? occupancy_grid(earl::tabletop_step_kernel<true, true>, h->sm_count, &h->step_grid)
                  : per_env_goals(h) ? occupancy_grid(earl::tabletop_step_kernel<true, false, 1, true>, h->sm_count, &h->step_grid)
                         : occupancy_grid(earl::tabletop_step_kernel<true, false>, h->sm_count, &h->step_grid);
   else rc = fast ? occupancy_grid(earl::tabletop_step_kernel<false, true>, h->sm_count, &h->step_grid)
@@ -416,10 +437,19 @@ int earl_get_goals(earl_handle* h, float* goals_out_dev, void* stream) {
   return 0;
 }
 
+int earl_set_final_obs(earl_handle* h, float* final_obs_dev) {
+  if (int rc = check_handle(h)) return rc;
+  if (!has_final_obs(h)) return fail(EARL_ERR_INVALID, "earl_set_final_obs needs a handle created with EARL_FLAG_FINAL_OBS");
+  if (!final_obs_dev || ((uintptr_t)final_obs_dev & 15u)) return fail(EARL_ERR_INVALID, "final_obs must be non-null and 16-byte aligned");
+  h->final_obs = final_obs_dev;
+  return 0;
+}
+
 int earl_step(earl_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev,
               uint8_t* success_dev, void* stream) {
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_io(actions_dev, obs_dev, reward_dev, done_dev)) return rc;
+  if (int rc = check_final_obs(h)) return rc;
   if (int rc = launch_step(h, actions_dev, obs_dev, reward_dev, done_dev, success_dev, static_cast<cudaStream_t>(stream))) return rc;
   return note_stream(h, static_cast<cudaStream_t>(stream));
 }
@@ -429,6 +459,7 @@ int earl_rollout(earl_handle* h, const float* actions_dev, int32_t action_ring, 
   if (int rc = check_handle(h)) return rc;
   if (int rc = check_io(actions_dev, obs_dev, reward_dev, done_dev)) return rc;
   if (action_ring < 1 || out_ring < 1 || num_steps < 0) return fail(EARL_ERR_INVALID, "rings must be >= 1 and num_steps >= 0");
+  if (has_final_obs(h)) return fail(EARL_ERR_INVALID, "earl_rollout does not take EARL_FLAG_FINAL_OBS handles (one final-observation buffer per step)");
   const size_t n = (size_t)h->p.n;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   for (int32_t t = 0; t < num_steps; ++t) {
@@ -485,6 +516,7 @@ int earl_step_host(earl_handle* h, const float* actions_host, float* obs_host, f
                    uint8_t* success_host) {
   if (int rc = check_handle(h)) return rc;
   if (!actions_host || !obs_host || !reward_host || !done_host) return fail(EARL_ERR_INVALID, "null host buffer");
+  if (int rc = check_final_obs(h)) return rc;
   {
     int rc = 0;
     if (step_host_zerocopy(h, actions_host, obs_host, reward_host, done_host, success_host, &rc)) return rc;

@@ -35,6 +35,7 @@
 #include <cuda_runtime.h>
 
 #include "eval_stats.cuh"
+#include "final_obs.cuh"
 #include "mj_model_host.hpp"
 #include "mj_step.cuh"
 
@@ -722,6 +723,7 @@ struct earl_mjk_handle {
   bool redo_sms_fixed = false;      // EARL_MJ_REDO_SMS given: no adaptation
   unsigned* h_redo_seen = nullptr;  // pinned: redo-list length of a recent step (async copy, read without waiting)
   int ring_configs = 0;             // rows of the reset stream's configuration table
+  double* final_obs = nullptr;      // EARL_FLAG_FINAL_OBS: the caller's [N,46] buffer (earl_mjk_set_final_obs)
   int redo_sms = 4;          // SMs the step kernel leaves to the concurrent redo kernel (EARL_MJ_REDO_SMS; measured 2: 1.49e5, 4: 1.54e5, 6: 1.53e5)
   std::vector<void*> owned;
   template <typename T>
@@ -781,7 +783,10 @@ int earl_mjk_create(const earl_mjk_config* cfg, const void* model_blob, size_t m
   if (!cfg || !model_blob || !out) return failf(EARL_ERR_INVALID, "null argument");
   *out = nullptr;
   if (cfg->num_envs <= 0 || cfg->frame_skip <= 0 || cfg->episode_horizon <= 0) return failf(EARL_ERR_INVALID, "bad kitchen config");
-  if (cfg->flags & ~(uint32_t)(EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS)) return failf(EARL_ERR_UNSUPPORTED, "unsupported flags %#x", cfg->flags);
+  if (cfg->flags & ~(uint32_t)(EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS | EARL_FLAG_FINAL_OBS))
+    return failf(EARL_ERR_UNSUPPORTED, "unsupported flags %#x", cfg->flags);
+  if ((cfg->flags & EARL_FLAG_FINAL_OBS) && !(cfg->flags & EARL_FLAG_AUTO_RESET))
+    return failf(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS needs EARL_FLAG_AUTO_RESET");
   earl_mjk_engine* eng = nullptr;
   if (int rc = earl_mjk_engine_create(model_blob, model_nbytes, cfg->device, &eng)) return rc;
   earl_mjk_handle* h = new (std::nothrow) earl_mjk_handle();
@@ -889,6 +894,8 @@ int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev,
                   void* stream) {
   if (!h || !actions_dev || !obs_dev || !reward_dev || !done_dev) return failf(EARL_ERR_INVALID, "null argument");
   if ((h->a.flags & EARL_FLAG_AUTO_RESET) && !h->a.ring_rows) return failf(EARL_ERR_INVALID, "auto-reset handles need earl_mjk_set_reset_stream before the first step");
+  if ((h->a.flags & EARL_FLAG_FINAL_OBS) && !h->final_obs)
+    return failf(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS handles need earl_mjk_set_final_obs before the first step");
   CU(cudaSetDevice(h->eng->device));
   h->a.mocap_quat = make_float4(h->eng->mocap_quat[0], h->eng->mocap_quat[1], h->eng->mocap_quat[2], h->eng->mocap_quat[3]);
   h->total_steps += 1;
@@ -899,9 +906,19 @@ int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev,
   mjk_order_kernel<<<64, 256, 0, s>>>(h->d_bucket, h->d_rank, h->a.n, h->d_counts, h->d_order);
   CU(cudaGetLastError());
   if (h->h_redo_seen && h->a.redo_list) CU(cudaMemcpyAsync(h->h_redo_seen, h->a.sched + kRedoCount, sizeof(unsigned), cudaMemcpyDeviceToHost, s));
+  // final observations: the rows the reset pass below replaces, after the step, redo, bucket and order kernels
+  if (h->final_obs) CU(earl::launch_final_obs_capture(obs_dev, done_dev, h->final_obs, h->a.n, kObs, h->eng->sm_count, s));
   // auto reset: the envs whose horizon fired in this step, after the step, redo, bucket and order kernels (plain launch)
   if (h->a.flags & EARL_FLAG_AUTO_RESET)
     if (int rc = launch_task(h, 3, nullptr, h->a.n, nullptr, nullptr, obs_dev, nullptr, done_dev, nullptr, stream)) return rc;
+  return 0;
+}
+
+int earl_mjk_set_final_obs(earl_mjk_handle* h, double* final_obs_dev) {
+  if (!h) return failf(EARL_ERR_INVALID, "null handle");
+  if (!(h->a.flags & EARL_FLAG_FINAL_OBS)) return failf(EARL_ERR_INVALID, "earl_mjk_set_final_obs needs a handle created with EARL_FLAG_FINAL_OBS");
+  if (!final_obs_dev) return failf(EARL_ERR_INVALID, "null final_obs");
+  h->final_obs = final_obs_dev;
   return 0;
 }
 

@@ -114,97 +114,19 @@ __device__ __forceinline__ void next_reset_qpos(const T3Params& p, int i, double
 // and the auto-reset, each behind a warp-uniform test of p.features.
 template <bool GENERAL>
 __global__ void __launch_bounds__(kBlock) tt3_step_kernel(const __grid_constant__ T3Params p) {
-  __shared__ float4 s_obs[kBlock * 5];
-  __shared__ float4 s_act4[kBlock * kAct / 4];
-  float* s_act = reinterpret_cast<float*>(s_act4);
-  const int end = p.first + p.count;
-  const int base = p.first + blockIdx.x * kBlock;
-  const int t = threadIdx.x;
-  const int i = base + t;
-  const int rows = min(kBlock, end - base);
-  pdl_wait_prior_grid();  // nothing is read before the previous grid in the stream (the previous step, or the
-                          // caller's action producer) has completed and flushed
-  {  // actions of the tile: contiguous 16-byte loads when the tile starts on a 16-byte boundary (always, unless the
-     // caller's buffer or a ring slot of a batch that is not a multiple of 4 envs is only 4-byte aligned)
-    const float* asrc = p.actions + (size_t)base * kAct;
-    if ((reinterpret_cast<uintptr_t>(asrc) & 15u) == 0) {
-      const float4* src = reinterpret_cast<const float4*>(asrc);
-      const int full = rows * kAct / 4;
-      if (t < full) s_act4[t] = __ldcs(src + t);
-      const int rem = rows * kAct - full * 4;
-      if (t < rem) s_act[full * 4 + t] = asrc[full * 4 + t];
-    } else {
-      for (int k = t; k < rows * kAct; k += kBlock) s_act[k] = asrc[k];
-    }
-  }
-  __syncthreads();
-  if (i < end) {
-    const double2 f = p.q[0][i], oa = p.q[1][i], ob = p.q[2][i], oc = p.q[3][i];
-    const uint2 m = p.meta[i];
-    const uint32_t row = (m.x >> 8) & 0xffu;
-    EnvState st{f.x, f.y, {oa.x, ob.x, oc.x}, {oa.y, ob.y, oc.y}, m.x & 3u};
-    const EnvConst ec{p.act_lo, p.act_span, p.threshold, p.clip, p.success_radius};
-    earl::tt3::move(ec, st, s_act[kAct * t], s_act[kAct * t + 1], s_act[kAct * t + 2]);  // 3OBJ:86-144
-    const uint32_t att = st.att;
-    p.q[0][i] = make_double2(st.fx, st.fy);
-#pragma unroll
-    for (int k = 0; k < 3; ++k)  // only the dragged object's plane is written back
-      if (att == (uint32_t)(k + 1)) p.q[1 + k][i] = make_double2(st.ox[k], st.oy[k]);
-    float o[8];
-    earl::tt3::observe8(st, o);  // 3OBJ:49-54
-    float g[10];
-    {
-      const float2* gr = reinterpret_cast<const float2*>(p.goal_f32 + row * 10);
-#pragma unroll
-      for (int k = 0; k < 5; ++k) {
-        const float2 v = __ldg(gr + k);
-        g[2 * k] = v.x;
-        g[2 * k + 1] = v.y;
-      }
-    }
-    if (!GENERAL) stage_obs(s_obs, t, o, marker(att), g);
-    const bool succ = earl::tt3::success(o, g, p.success_radius);
-    const float rew = p.dense ? (float)earl::tt3::dense(o, g) : (succ ? 1.0f : 0.0f);  // 3OBJ:146-159
-    // PSW:22-31
-    const uint32_t steps = m.y == 0xffffffffu ? m.y : m.y + 1u;
-    if (!GENERAL) p.meta[i] = make_uint2((m.x & ~3u) | att, steps);
-    __stcs(p.reward + i, rew);
-    const bool done = (unsigned long long)steps >= p.horizon;
-    p.done[i] = done ? 1 : 0;
-    if (p.success) p.success[i] = succ ? 1 : 0;
-    if (GENERAL) {
-      uint32_t mx = (m.x & ~3u) | att, ms = steps;
-      const bool reset = done && (p.features & kAutoReset);
-      if (p.features & kEvalStats) {
-        p.ep_return[i] = reset ? 0.0 : p.ep_return[i] + (double)rew;
-        mx = (mx & ~kSuccLast) | (succ ? (kSuccLast | kSuccAny) : 0u);
-      }
-      if (reset) {  // what earl_tt3_reset(init_qpos NULL) does to this env, fused: PSW:17-20 + 3OBJ:67-84
-        double2 q[4];
-        next_reset_qpos(p, i, q);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          p.q[k][i] = q[k];
-          o[2 * k] = (float)q[k].x;
-          o[2 * k + 1] = (float)q[k].y;
-        }
-        p.interventions[i] += 1;
-        mx &= ~(0xff00u | 0xfu);  // goal row 0 (get_next_goal() over one goal), nothing attached, success bits cleared
-        ms = 0u;
-        const float2* gr = reinterpret_cast<const float2*>(p.goal_f32);
-#pragma unroll
-        for (int k = 0; k < 5; ++k) {
-          const float2 v = __ldg(gr + k);
-          g[2 * k] = v.x;
-          g[2 * k + 1] = v.y;
-        }
-      }
-      p.meta[i] = make_uint2(mx, ms);
-      stage_obs(s_obs, t, o, marker(mx & 3u), g);
-    }
-  }
-  __syncthreads();
-  flush_obs(s_obs, p.obs, base, end);
+  constexpr bool FINAL = false;
+  float* const final_obs = nullptr;
+#include "tt3_step_body.inc"
+}
+
+// EARL_FLAG_FINAL_OBS handles run tt3_step_kernel<true, true>: the fused auto-reset first stores the env's pre-reset
+// observation row to final_obs [N,20].  An overload with one more template parameter and the buffer as a second argument,
+// sharing the body above textually, so that the kernels of every other handle keep their symbol names, parameter layout
+// and code.
+template <bool GENERAL, bool FINAL>
+__global__ void __launch_bounds__(kBlock) tt3_step_kernel(const __grid_constant__ T3Params p, float* final_obs) {
+  static_assert(GENERAL || !FINAL, "final observations need the auto-reset of the GENERAL step");
+#include "tt3_step_body.inc"
 }
 
 // PSW:17-20 + 3OBJ:67-84 for the masked envs; also serves reset_goal (state untouched) and _get_obs
@@ -336,6 +258,7 @@ struct earl_tt3_handle {
   int64_t launches = 0;
   int sm_count = 0;
   void (*step_kernel)(T3Params) = nullptr;  // chosen once from the flags in earl_tt3_create
+  float* final_obs = nullptr;               // EARL_FLAG_FINAL_OBS: the caller's [N,20] buffer (earl_tt3_set_final_obs)
   std::vector<void*> owned;
   float* d_act = nullptr;
   float* d_obs = nullptr;
@@ -376,6 +299,13 @@ int check_stream(const earl_tt3_handle* h) {
   return 0;
 }
 
+// a final-observation handle steps only once its buffer is registered
+int check_final_obs(const earl_tt3_handle* h) {
+  if ((h->cfg.flags & EARL_FLAG_FINAL_OBS) && !h->final_obs)
+    return fail(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS handles need earl_tt3_set_final_obs before the first step");
+  return 0;
+}
+
 int grid_for(long long n) { return (int)((n + kBlock - 1) / kBlock); }
 
 int launch_step(earl_tt3_handle* h, int first, int count, const float* actions, float* obs, float* reward, uint8_t* done,
@@ -397,7 +327,8 @@ int launch_step(earl_tt3_handle* h, int first, int count, const float* actions, 
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  CU(cudaLaunchKernelEx(&cfg, h->step_kernel, p));
+  if (h->cfg.flags & EARL_FLAG_FINAL_OBS) CU(cudaLaunchKernelEx(&cfg, tt3_step_kernel<true, true>, p, h->final_obs));
+  else CU(cudaLaunchKernelEx(&cfg, h->step_kernel, p));
   h->launches += 1;
   return 0;
 }
@@ -413,8 +344,11 @@ int earl_tt3_create(const earl_tt3_config* cfg, size_t cfg_nbytes, earl_tt3_hand
   if (cfg_nbytes != sizeof(earl_tt3_config)) return fail(EARL_ERR_INVALID, "earl_tt3_config size mismatch (%zu)", cfg_nbytes);
   if (cfg->num_envs < 1) return fail(EARL_ERR_INVALID, "num_envs must be >= 1");
   if (cfg->num_goals < 1 || cfg->num_goals > EARL_TT3_MAX_GOALS) return fail(EARL_ERR_INVALID, "num_goals out of range");
-  const uint32_t supported = EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL | EARL_FLAG_EVAL_STATS;
+  const uint32_t supported = EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL | EARL_FLAG_EVAL_STATS |
+                             EARL_FLAG_FINAL_OBS;
   if (cfg->flags & ~supported) return fail(EARL_ERR_UNSUPPORTED, "unsupported flag for the three-object tabletop");
+  if ((cfg->flags & EARL_FLAG_FINAL_OBS) && !(cfg->flags & EARL_FLAG_AUTO_RESET))
+    return fail(EARL_ERR_INVALID, "EARL_FLAG_FINAL_OBS needs EARL_FLAG_AUTO_RESET");
   if (cfg->episode_horizon < 1) return fail(EARL_ERR_INVALID, "episode_horizon must be >= 1");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || cfg->device < 0 || cfg->device >= ndev) {
@@ -512,6 +446,7 @@ int earl_tt3_step(earl_tt3_handle* h, const float* actions_dev, float* obs_dev, 
   if (!actions_dev || !obs_dev || !reward_dev || !done_dev) return fail(EARL_ERR_INVALID, "null device buffer");
   if (!aligned16(obs_dev)) return fail(EARL_ERR_INVALID, "obs must be 16-byte aligned");
   if (int rc = check_stream(h)) return rc;
+  if (int rc = check_final_obs(h)) return rc;
   if (int rc = launch_step(h, 0, h->p.n, actions_dev, obs_dev, reward_dev, done_dev, success_dev, (cudaStream_t)stream)) return rc;
   h->total_steps += 1;
   return 0;
@@ -522,6 +457,8 @@ int earl_tt3_rollout(earl_tt3_handle* h, const float* actions_dev, int32_t actio
   if (int rc = check(h)) return rc;
   if (!actions_dev || !obs_dev || !reward_dev || !done_dev || action_ring < 1 || out_ring < 1 || num_steps < 0)
     return fail(EARL_ERR_INVALID, "bad rollout argument");
+  if (h->cfg.flags & EARL_FLAG_FINAL_OBS)
+    return fail(EARL_ERR_INVALID, "earl_tt3_rollout does not take EARL_FLAG_FINAL_OBS handles (one final-observation buffer per step)");
   const size_t n = (size_t)h->p.n;
   if (!aligned16(obs_dev)) return fail(EARL_ERR_INVALID, "obs must be 16-byte aligned");
   if (int rc = check_stream(h)) return rc;
@@ -540,6 +477,7 @@ int earl_tt3_step_host(earl_tt3_handle* h, const float* actions_host, float* obs
   if (int rc = check(h)) return rc;
   if (!actions_host || !obs_host || !reward_host || !done_host) return fail(EARL_ERR_INVALID, "null host buffer");
   if (int rc = check_stream(h)) return rc;
+  if (int rc = check_final_obs(h)) return rc;
   const size_t n = (size_t)h->p.n;
   if (!h->d_act) {
     int rc = h->alloc(&h->d_act, n * kAct, false);
@@ -599,6 +537,14 @@ int earl_tt3_set_reset_stream(earl_tt3_handle* h, const double* qpos_rows_host, 
   }
   CU(cudaMemcpy(const_cast<double*>(h->p.reset_qpos), qpos_rows_host, (size_t)rows * n * 8 * sizeof(double), cudaMemcpyHostToDevice));
   CU(cudaMemset(h->p.reset_cursor, 0, n * sizeof(uint32_t)));
+  return 0;
+}
+
+int earl_tt3_set_final_obs(earl_tt3_handle* h, float* final_obs_dev) {
+  if (int rc = check(h)) return rc;
+  if (!(h->cfg.flags & EARL_FLAG_FINAL_OBS)) return fail(EARL_ERR_INVALID, "earl_tt3_set_final_obs needs a handle created with EARL_FLAG_FINAL_OBS");
+  if (!final_obs_dev || !aligned16(final_obs_dev)) return fail(EARL_ERR_INVALID, "final_obs must be non-null and 16-byte aligned");
+  h->final_obs = final_obs_dev;
   return 0;
 }
 

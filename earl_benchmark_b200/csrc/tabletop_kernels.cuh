@@ -214,106 +214,18 @@ __device__ __forceinline__ void tt_store_obs_tile(float* __restrict__ obs, const
 // looked up in the goal table through the row in meta.
 template <bool F64, bool FAST, int MINB = 1, bool GOALS = false>
 __global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const TabletopParams p) {
-  static_assert(!(FAST && GOALS), "per-env goals run on the general kernel");
-  __shared__ __align__(16) float tiles[kTTBlock / 32][32 * kTTObs];
-  pdl_wait_prior_grid();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float* tile = tiles[warp];
-  const bool dense = !FAST && (p.features & kDense);
-  const bool wide = p.features & kWide;
+  constexpr bool FINAL = false;
+  float* const final_obs = nullptr;
+#include "tabletop_step_body.inc"
+}
 
-  for (int base = p.first + blockIdx.x * kTTBlock; base < p.n; base += gridDim.x * kTTBlock) {
-    const int i = base + threadIdx.x;
-    const int warp_base = base + warp * 32;
-    if (warp_base >= p.n) break;  // warp-uniform
-    const bool valid = i < p.n;
-    float4 pos32 = make_float4(0.f, 0.f, 0.f, 0.f), g0 = pos32, g1 = pos32;
-    float att = -1.f;
-    if (valid) {
-      TTState s;
-      uint32_t steps;
-      tt_load_state<F64>(p, i, s, steps);
-      const float a0 = __ldcs(p.actions + (size_t)i * kTTAct + 0);
-      const float a1 = __ldcs(p.actions + (size_t)i * kTTAct + 1);
-      const float a2 = __ldcs(p.actions + (size_t)i * kTTAct + 2);
-      uint32_t gi = (s.flags & kGoalMask) >> kGoalShift;
-      if (GOALS) {
-        g0 = p.env_goal[2 * (size_t)i];
-        g1 = p.env_goal[2 * (size_t)i + 1];
-      } else {
-        g0 = __ldg(p.goal32 + 2 * gi);
-        g1 = __ldg(p.goal32 + 2 * gi + 1);
-      }
-
-      tt_move(s, a0, a1, a2, p);
-      pos32 = make_float4(__double2float_rn(s.fx), __double2float_rn(s.fy), __double2float_rn(s.mx),
-                          __double2float_rn(s.my));
-      const bool succ = tt_success(pos32, g0, wide, p.success_sq);
-      float rew = succ ? 1.f : 0.f;
-      if (!FAST && dense) rew = (float)tt_dense_reward(pos32, g0);
-
-      // PersistentStateWrapper.step: counters, then the horizon (persistent_state_wrapper.py:25-29)
-      steps = steps == 0xffffffffu ? steps : steps + 1u;
-      const bool done = (unsigned long long)steps >= p.horizon;
-
-      if (!FAST) {
-        if (p.features & kEvalStats) {
-          p.ep_return[i] += (double)rew;
-          s.flags = (s.flags & ~kSuccessLast) | (succ ? (kSuccessLast | kSuccessAny) : 0u);
-        }
-        if (p.features & kLifelong) {  // LifelongWrapper.step (lifelong_wrapper.py:31-42)
-          uint32_t ls = p.ll_steps[i] + 1u;
-          p.ll_return[i] += (double)rew;
-          if ((unsigned long long)ls >= p.goal_change_frequency) {
-            ls = 0u;
-            const uint32_t c = p.goal_cursor[i];
-            gi = p.goal_stream[(size_t)(c % (uint32_t)p.goal_stream_rows) * p.n_total + i];
-            p.goal_cursor[i] = c + 1u;
-            s.flags = (s.flags & ~kGoalMask) | (gi << kGoalShift);
-            g0 = __ldg(p.goal32 + 2 * gi);  // the returned obs carries the NEW goal, the reward the old one
-            g1 = __ldg(p.goal32 + 2 * gi + 1);
-            if (GOALS) { p.env_goal[2 * (size_t)i] = g0; p.env_goal[2 * (size_t)i + 1] = g1; }
-          }
-          p.ll_steps[i] = ls;
-        }
-        if (done && (p.features & kAutoReset)) {  // what the user's reset() would do, fused
-          const uint32_t c = p.goal_cursor[i];
-          gi = p.goal_stream[(size_t)(c % (uint32_t)p.goal_stream_rows) * p.n_total + i];
-          p.goal_cursor[i] = c + 1u;
-          p.interventions[i] += 1;
-          steps = 0u;
-          s.flags = gi << kGoalShift;
-          g0 = __ldg(p.goal32 + 2 * gi);
-          g1 = __ldg(p.goal32 + 2 * gi + 1);
-          if (GOALS) { p.env_goal[2 * (size_t)i] = g0; p.env_goal[2 * (size_t)i + 1] = g1; }
-          if (p.features & kResetAtGoal) {
-            const double* g = p.goal64 + 6 * gi;
-            s.fx = g[0]; s.fy = g[1]; s.mx = g[2]; s.my = g[3];
-          } else {
-            s.fx = p.init_qpos[0]; s.fy = p.init_qpos[1]; s.mx = p.init_qpos[2]; s.my = p.init_qpos[3];
-          }
-          pos32 = make_float4(__double2float_rn(s.fx), __double2float_rn(s.fy), __double2float_rn(s.mx),
-                              __double2float_rn(s.my));
-          if (p.features & kLifelong) p.ll_steps[i] = 0u;
-          if (p.features & kEvalStats) p.ep_return[i] = 0.0;
-        }
-      }
-
-      tt_store_state<F64>(p, i, s, pos32, steps);
-      __stcs(p.reward + i, rew);
-      p.done[i] = done ? 1 : 0;
-      if (p.success) p.success[i] = succ ? 1 : 0;
-      att = (s.flags & kAttached) ? 0.f : -1.f;
-    }
-    // obs row = [fist xy, mug xy | att, att, goal[0:2] | goal[2:6]]  (tabletop_manipulation.py:55-60)
-    float4* row = reinterpret_cast<float4*>(tile + lane * kTTObs);
-    row[0] = pos32;
-    row[1] = make_float4(att, att, g0.x, g0.y);
-    row[2] = make_float4(g0.z, g0.w, g1.x, g1.y);
-    __syncwarp();
-    tt_store_obs_tile(p.obs, tile, warp_base, p.n, lane);
-    __syncwarp();
-  }
+// EARL_FLAG_FINAL_OBS handles (general kernel, FINAL = true): the fused auto-reset first stores the env's pre-reset
+// observation row to final_obs [N,12].  An overload with one more template parameter and the buffer as a second argument,
+// sharing the body above textually: the kernels of every other handle keep their symbol names, parameter layout and code
+// (moving the body into an inlined device function reorders their registers).
+template <bool F64, bool FAST, int MINB, bool GOALS, bool FINAL>
+__global__ void __launch_bounds__(kTTBlock, MINB) tabletop_step_kernel(const TabletopParams p, float* final_obs) {
+#include "tabletop_step_body.inc"
 }
 
 // ------------------------------------------------------------------------------------------ tile kernel

@@ -38,8 +38,13 @@ class HostBuffers:
         return self.sets[self.turn]
 
     @staticmethod
-    def as_numpy(ho, hr, hd, hs):
-        return ho.numpy(), hr.numpy(), hd.numpy().view(np.bool_), {"success": hs.numpy().view(np.bool_)}
+    def as_numpy(ho, hr, hd, hs, final_obs=None):
+        """numpy views of one output set; `final_obs` (the env's device buffer of final observations, final_obs=True envs)
+        is added to info as a host copy, taken after the synchronous host step has written it"""
+        info = {"success": hs.numpy().view(np.bool_)}
+        if final_obs is not None:
+            info["final_observation"] = final_obs.cpu().numpy()
+        return ho.numpy(), hr.numpy(), hd.numpy().view(np.bool_), info
 
 
 def ranks_on_this_host():

@@ -36,8 +36,10 @@ class SawyerBatchedEnv:
 
     def __init__(self, reward_type="sparse", reset_at_goal=False, num_envs=1, device=None, seed=0, eval_stats=False,
                  env_offset=0, total_envs=None, model_path=None, max_newton=0, host_io=False, auto_reset=False,
-                 reset_stream_rows=64, per_env_goals=False, **_tabletop_only):
+                 reset_stream_rows=64, per_env_goals=False, final_obs=False, **_tabletop_only):
         name = type(self).__name__
+        if final_obs and not auto_reset:
+            raise ValueError("final_obs=True needs auto_reset=True: without it, the observation step() returns on done is the final one")
         if reward_type == "dense" and not self.HAS_DENSE_REWARD:
             raise NotImplementedError(f"{name}: the dense reward (metaworld reward_utils, gripper caging) is not built yet")
         if reward_type not in ("sparse", "dense"):
@@ -65,7 +67,7 @@ class SawyerBatchedEnv:
         self._goal_change_frequency = 0
         self._handle = None
         self._np_random = rng.NumpyLegacyRandom(self._seed & 0xFFFFFFFF)
-        self._obs = self._reward = self._done = self._success = None
+        self._obs = self._reward = self._done = self._success = self._final_obs = None
         self._host_bufs = None
         self._host_mode = bool(host_io)   # host_io=True: reset() returns numpy like the numpy-driven step()
         # auto_reset=True: an env whose horizon fires is reset inside step() on the device, and every reset without an
@@ -76,6 +78,9 @@ class SawyerBatchedEnv:
             raise ValueError("reset_stream_rows must be >= 1")
         # per_env_goals=True: every env can be given its own goal vector, effective at once (set_goals / get_goals)
         self._per_env_goals = bool(per_env_goals)
+        # final_obs=True (with auto_reset): every step's info["final_observation"] holds the last observation of each
+        # episode the step ended (see step())
+        self._keep_final_obs = bool(final_obs)
 
     # ------------------------------------------------------------------ task hooks
     def _task_spec(self):
@@ -110,6 +115,7 @@ class SawyerBatchedEnv:
         flags = (_lib.FLAG_EVAL_STATS if self._eval_stats else 0) | (_lib.FLAG_LIFELONG if self._lifelong else 0)
         flags |= _lib.FLAG_AUTO_RESET if self._auto_reset else 0
         flags |= _lib.FLAG_PER_ENV_GOALS if self._per_env_goals else 0
+        flags |= _lib.FLAG_FINAL_OBS if self._keep_final_obs else 0
         if self._reward_type == "dense":
             flags |= _lib.FLAG_DENSE_REWARD
         cfg = _lib.MjConfig(self.ENV_KIND, self.num_envs, self.device.index or 0, flags, self._episode_horizon,
@@ -130,6 +136,9 @@ class SawyerBatchedEnv:
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._goal_rows = torch.zeros((n,), dtype=torch.int32, device=dev)   # the handle reads it (auto reset): never rebound
+        if self._keep_final_obs:   # rows of envs that have not ended an episode yet hold NaN
+            self._final_obs = torch.full((n, OBS_DIM), float("nan"), dtype=torch.float32, device=dev)
+            _lib.check(L.earl_mj_set_final_obs(h, self._final_obs.data_ptr()))
         if self._auto_reset:
             qpos, rows = self._reset_stream(self._reset_stream_rows)
             qpos = np.ascontiguousarray(qpos, np.float64)
@@ -218,7 +227,10 @@ class SawyerBatchedEnv:
 
     def step(self, action, out=None):
         """One step of every env.  CUDA float32 tensor [N,4] -> CUDA tensors (obs [N,14], reward [N], done [N] bool,
-        info), owned by the env and valid until the next step; numpy / CPU tensor -> host path, numpy arrays."""
+        info), owned by the env and valid until the next step; numpy / CPU tensor -> host path, numpy arrays.
+        final_obs=True envs add info["final_observation"] [N,14]: on rows where done is set, the observation the step
+        reached before the auto-reset replaced it; other rows keep what an earlier step stored there (NaN before an env's
+        first episode ends).  The env-owned tensor, valid until the next step; a numpy copy on the host path."""
         self._ensure()
         if isinstance(action, torch.Tensor) and action.is_cuda:
             a = action
@@ -229,7 +241,10 @@ class SawyerBatchedEnv:
             obs, rew, done, succ = out if out is not None else (self._obs, self._reward, self._done, self._success)
             _lib.check(_lib.lib().earl_mj_step(self._handle, a.data_ptr(), obs.data_ptr(), rew.data_ptr(), done.data_ptr(),
                                                _ptr(succ), _stream()))
-            return obs, rew, done.view(torch.bool), {"success": None if succ is None else succ.view(torch.bool)}
+            info = {"success": None if succ is None else succ.view(torch.bool)}
+            if self._final_obs is not None:
+                info["final_observation"] = self._final_obs
+            return obs, rew, done.view(torch.bool), info
         return self._step_host(action)
 
     def _step_host(self, action):
@@ -242,7 +257,7 @@ class SawyerBatchedEnv:
         ho, hr, hd, hs = hb.next_outputs()
         _lib.check(_lib.lib().earl_mj_step_host(self._handle, src.data_ptr(), ho.data_ptr(), hr.data_ptr(), hd.data_ptr(),
                    hs.data_ptr()))
-        return HostBuffers.as_numpy(ho, hr, hd, hs)
+        return HostBuffers.as_numpy(ho, hr, hd, hs, self._final_obs)
 
     def _get_obs(self):
         self._ensure()

@@ -129,7 +129,9 @@ class Kitchen:
     max_path_length = int(1e8)
 
     def __init__(self, task="all_pairs", reward_type="dense", num_envs=1, device=None, seed=0, env_offset=0, total_envs=None,
-                 model_path=None, auto_reset=False, reset_stream_rows=64, eval_stats=False, **_unused):
+                 model_path=None, auto_reset=False, reset_stream_rows=64, eval_stats=False, final_obs=False, **_unused):
+        if final_obs and not auto_reset:
+            raise ValueError("final_obs=True needs auto_reset=True: without it, the observation step() returns on done is the final one")
         if reward_type != 'dense':
             raise ValueError("Kitchen environment only supports dense rewards.")     # kitchen.py:91-92
         self._initial_states = copy.deepcopy(initial_states)
@@ -162,6 +164,10 @@ class Kitchen:
             raise ValueError("reset_stream_rows must be >= 1")
         # eval_stats=True: every env keeps its episode return and success on the device, reduced by eval_stats()
         self._eval_stats = bool(eval_stats)
+        # final_obs=True (with auto_reset): every step's info["final_observation"] holds the last observation of each
+        # episode the step ended (see step())
+        self._keep_final_obs = bool(final_obs)
+        self._final_obs = None
 
     # ------------------------------------------------------------------ reference surface
     def get_task(self):
@@ -204,7 +210,7 @@ class Kitchen:
         cfg = MjkConfig()
         cfg.num_envs, cfg.device, cfg.frame_skip = self.num_envs, self.device.index or 0, FRAME_SKIP
         cfg.flags = (_lib.FLAG_LIFELONG if self._lifelong else 0) | (_lib.FLAG_AUTO_RESET if self._auto_reset else 0) | \
-            (_lib.FLAG_EVAL_STATS if self._eval_stats else 0)
+            (_lib.FLAG_EVAL_STATS if self._eval_stats else 0) | (_lib.FLAG_FINAL_OBS if self._keep_final_obs else 0)
         cfg.episode_horizon = self._episode_horizon
         cfg.goal_change_frequency = self._goal_change_frequency if self._lifelong else 0
         cfg.goal[:] = self.goal.tolist()
@@ -224,6 +230,9 @@ class Kitchen:
         self._reward = torch.empty((n,), dtype=torch.float64, device=dev)
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
+        if self._keep_final_obs:   # rows of envs that have not ended an episode yet hold NaN
+            self._final_obs = torch.full((n, OBS_DIM), float("nan"), dtype=torch.float64, device=dev)
+            _lib.check(_lib.lib().earl_mjk_set_final_obs(h, self._final_obs.data_ptr()))
         self.seed(self._env_seed)
         if self._auto_reset:
             config, table = reset_stream(self._seed, self._total_envs, self._env_offset, n, self._reset_stream_rows, self._task)
@@ -288,7 +297,10 @@ class Kitchen:
 
     def step(self, action, b=None):
         """CUDA float32 tensor [N,9] -> CUDA tensors (obs float64 [N,46], reward float64 [N], done bool [N], info); numpy
-        in -> numpy out (copies through the device)."""
+        in -> numpy out (copies through the device).  final_obs=True envs add info["final_observation"] float64 [N,46]:
+        on rows where done is set, the observation the step reached before the auto-reset replaced it; other rows keep
+        what an earlier step stored there (NaN before an env's first episode ends).  The env-owned tensor, valid until
+        the next step; a numpy copy for numpy input."""
         self._ensure()
         host = not (isinstance(action, torch.Tensor) and action.is_cuda)
         a = torch.as_tensor(np.asarray(action, np.float32)).to(self.device) if host else action
@@ -299,9 +311,11 @@ class Kitchen:
         _lib.check(_lib.lib().earl_mjk_step(self._handle, a.data_ptr(), self._obs.data_ptr(), self._reward.data_ptr(),
                                             self._done.data_ptr(), self._success.data_ptr(), _stream()))
         info = {"success": self._success.view(torch.bool)}
+        if self._final_obs is not None:
+            info["final_observation"] = self._final_obs
         if host:
             return self._obs.cpu().numpy(), self._reward.cpu().numpy(), self._done.cpu().numpy().view(np.bool_), \
-                {"success": self._success.cpu().numpy().view(np.bool_)}
+                {k: v.cpu().numpy().view(np.bool_) if k == "success" else v.cpu().numpy() for k, v in info.items()}
         return self._obs, self._reward, self._done.view(torch.bool), info
 
     def _get_obs(self):

@@ -50,13 +50,16 @@ class TabletopManipulation:
     (tabletop_manipulation.py:24-28).  Batched extras: num_envs, device, seed, state_dtype ('float32' |
     'float64'), goal_stream_rows, auto_reset, eval_stats, env_offset/total_envs (this shard's slice of a
     larger job: the goal stream is drawn for `total_envs` envs and columns [env_offset, env_offset+N) kept),
-    per_env_goals (every env keeps its own goal vector: set_goals() / get_goals()).
+    per_env_goals (every env keeps its own goal vector: set_goals() / get_goals()), final_obs (with auto_reset: every
+    step's info["final_observation"] holds the last observation of each episode the step ended, see step()).
     """
 
     def __init__(self, task_list="rc_r-rc_k-rc_g-rc_b", reward_type="dense", reset_at_goal=False,
                  wide_init_distr=False, num_envs=1, device=None, seed=0, state_dtype="float32",
                  goal_stream_rows=64, auto_reset=False, eval_stats=False, env_offset=0, total_envs=None, host_io=False,
-                 per_env_goals=False):
+                 per_env_goals=False, final_obs=False):
+        if final_obs and not auto_reset:
+            raise ValueError("final_obs=True needs auto_reset=True: without it, the observation step() returns on done is the final one")
         if reward_type not in ("sparse", "dense"):
             raise ValueError(f"reward_type must be 'sparse' or 'dense', got {reward_type!r}")
         if state_dtype not in ("float32", "float64"):
@@ -72,6 +75,7 @@ class TabletopManipulation:
         self._auto_reset = bool(auto_reset)
         self._eval_stats = bool(eval_stats)
         self._per_env_goals = bool(per_env_goals)
+        self._keep_final_obs = bool(final_obs)
         self._env_offset = int(env_offset)
         self._total_envs = int(total_envs) if total_envs is not None else self.num_envs + self._env_offset
         if device is None:
@@ -99,7 +103,7 @@ class TabletopManipulation:
         self._goal_change_frequency = 0
         self._handle = None
         self._np_random = rng.NumpyLegacyRandom(self._seed & 0xFFFFFFFF)  # np.random stream (wide-init resets)
-        self._obs = self._reward = self._done = self._success = None
+        self._obs = self._reward = self._done = self._success = self._final_obs = None
         self._host_bufs = None
         self._host_mode = bool(host_io)   # host_io=True: reset() returns numpy like the numpy-driven step()
 
@@ -146,6 +150,8 @@ class TabletopManipulation:
             f |= _lib.FLAG_EVAL_STATS
         if self._per_env_goals:
             f |= _lib.FLAG_PER_ENV_GOALS
+        if self._keep_final_obs:
+            f |= _lib.FLAG_FINAL_OBS
         return f
 
     def _model_blob(self):
@@ -200,6 +206,9 @@ class TabletopManipulation:
         self._reward = torch.empty((n,), dtype=torch.float32, device=dev)
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
+        if self._keep_final_obs:   # rows of envs that have not ended an episode yet hold NaN
+            self._final_obs = torch.full((n, OBS_DIM), float("nan"), dtype=torch.float32, device=dev)
+            _lib.check(L.earl_set_final_obs(h, self._final_obs.data_ptr()))
 
     def close(self):
         if self._handle is not None:
@@ -346,6 +355,10 @@ class TabletopManipulation:
                 success) to write elsewhere).
                 numpy array / CPU tensor [N,3] -> host path (H2D copy, kernel, D2H copies inside the call),
                 returns numpy arrays.
+        final_obs=True envs add info["final_observation"] [N,12]: on rows where done is set, the observation the step
+        reached before the auto-reset replaced it (obs holds the post-reset one); other rows keep what an earlier step
+        stored there (NaN before an env's first episode ends).  The env-owned tensor, valid until the next step like obs;
+        a numpy copy on the host path.
         """
         self._ensure()
         if isinstance(action, torch.Tensor) and action.is_cuda:
@@ -357,7 +370,10 @@ class TabletopManipulation:
             obs, rew, done, succ = out if out is not None else (self._obs, self._reward, self._done, self._success)
             _lib.check(_lib.lib().earl_step(self._handle, a.data_ptr(), obs.data_ptr(), rew.data_ptr(), done.data_ptr(),
                                             _ptr(succ), _stream()))
-            return obs, rew, done.view(torch.bool), {"success": None if succ is None else succ.view(torch.bool)}
+            info = {"success": None if succ is None else succ.view(torch.bool)}
+            if self._final_obs is not None:
+                info["final_observation"] = self._final_obs
+            return obs, rew, done.view(torch.bool), info
         return self._step_host(action)
 
     def _step_host(self, action):
@@ -370,11 +386,13 @@ class TabletopManipulation:
         ho, hr, hd, hs = hb.next_outputs()
         _lib.check(_lib.lib().earl_step_host(self._handle, src.data_ptr(), ho.data_ptr(), hr.data_ptr(), hd.data_ptr(),
                    hs.data_ptr()))
-        return HostBuffers.as_numpy(ho, hr, hd, hs)
+        return HostBuffers.as_numpy(ho, hr, hd, hs, self._final_obs)
 
     def rollout_into(self, actions, num_steps, obs, reward, done, success=None):
         """`num_steps` back-to-back steps: step t reads actions[t % K], writes slot t % R of obs/reward/done
-        (shapes [K,N,3]; [R,N,12], [R,N], [R,N])."""
+        (shapes [K,N,3]; [R,N,12], [R,N], [R,N]).  Not available on final_obs=True envs."""
+        if self._keep_final_obs:
+            raise RuntimeError("rollout_into does not keep final observations: step() a final_obs=True env")
         self._ensure()
         K, R = actions.shape[0], obs.shape[0]
         assert actions.is_cuda and actions.dtype == torch.float32 and actions.is_contiguous()

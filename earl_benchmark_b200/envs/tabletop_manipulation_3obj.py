@@ -68,11 +68,14 @@ class TabletopManipulation:
     Batched extras: num_envs, device, seed, auto_reset (reset on the device when the horizon fires), reset_stream_rows
     (rows of the pre-drawn reset_at_goal stream of an auto_reset env), eval_stats (per-env episode return and success,
     reduced by eval_stats()), env_offset / total_envs (this shard's slice of a larger job: reset_at_goal draws are made
-    for `total_envs` envs and columns [env_offset, env_offset + N) kept).
+    for `total_envs` envs and columns [env_offset, env_offset + N) kept), final_obs (with auto_reset: every step's
+    info["final_observation"] holds the last observation of each episode the step ended, see step()).
     """
 
     def __init__(self, reward_type="dense", reset_at_goal=False, num_envs=1, device=None, seed=0, host_io=False,
-                 auto_reset=False, reset_stream_rows=64, eval_stats=False, env_offset=0, total_envs=None):
+                 auto_reset=False, reset_stream_rows=64, eval_stats=False, env_offset=0, total_envs=None, final_obs=False):
+        if final_obs and not auto_reset:
+            raise ValueError("final_obs=True needs auto_reset=True: without it, the observation step() returns on done is the final one")
         if reward_type not in ("sparse", "dense"):
             raise ValueError(f"reward_type must be 'sparse' or 'dense', got {reward_type!r}")
         self._reward_type = reward_type
@@ -84,6 +87,7 @@ class TabletopManipulation:
         if self._reset_stream_rows < 1:
             raise ValueError("reset_stream_rows must be >= 1")
         self._eval_stats = bool(eval_stats)
+        self._keep_final_obs = bool(final_obs)
         self._env_offset = int(env_offset)
         self._total_envs = int(total_envs) if total_envs is not None else self.num_envs + self._env_offset
         if self._env_offset < 0 or self._env_offset + self.num_envs > self._total_envs:
@@ -105,7 +109,7 @@ class TabletopManipulation:
         self._episode_horizon = _NEVER
         self._handle = None
         self._np_random = rng.NumpyLegacyRandom(self._seed & 0xFFFFFFFF)
-        self._obs = self._reward = self._done = self._success = None
+        self._obs = self._reward = self._done = self._success = self._final_obs = None
         self._host_bufs = None
         self._host_mode = bool(host_io)   # host_io=True: reset() returns numpy like the numpy-driven step()
 
@@ -126,6 +130,7 @@ class TabletopManipulation:
         cfg.flags |= _lib.FLAG_AUTO_RESET if self._auto_reset else 0
         cfg.flags |= _lib.FLAG_RESET_AT_GOAL if self._reset_at_goal else 0
         cfg.flags |= _lib.FLAG_EVAL_STATS if self._eval_stats else 0
+        cfg.flags |= _lib.FLAG_FINAL_OBS if self._keep_final_obs else 0
         cfg.num_goals = MAX_GOALS          # every row is addressable; unused rows repeat row 0 until set
         cfg.episode_horizon = self._episode_horizon
         cfg.threshold, cfg.move_distance, cfg.clip, cfg.success_radius = self.threshold, self.move_distance, 2.8, 0.4
@@ -149,6 +154,9 @@ class TabletopManipulation:
         self._done = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._success = torch.empty((n,), dtype=torch.uint8, device=dev)
         self._goal_rows = np.zeros(n, np.int32)
+        if self._keep_final_obs:   # rows of envs that have not ended an episode yet hold NaN
+            self._final_obs = torch.full((n, OBS_DIM), float("nan"), dtype=torch.float32, device=dev)
+            _lib.check(_lib.lib().earl_tt3_set_final_obs(h, self._final_obs.data_ptr()))
 
     def _stream_resets(self):
         """resets without init_qpos take their qpos from the device's reset stream"""
@@ -253,7 +261,10 @@ class TabletopManipulation:
 
     def step(self, action, out=None):
         """One step of every env.  CUDA float32 [N,3] in -> CUDA tensors out (obs [N,20], reward [N], done [N] bool,
-        info; owned by the env, valid until the next step).  numpy / CPU tensor in -> host path, numpy out."""
+        info; owned by the env, valid until the next step).  numpy / CPU tensor in -> host path, numpy out.
+        final_obs=True envs add info["final_observation"] [N,20]: on rows where done is set, the observation the step
+        reached before the auto-reset replaced it; other rows keep what an earlier step stored there (NaN before an env's
+        first episode ends).  The env-owned tensor, valid until the next step; a numpy copy on the host path."""
         self._ensure()
         if isinstance(action, torch.Tensor) and action.is_cuda:
             a = action
@@ -264,7 +275,10 @@ class TabletopManipulation:
             obs, rew, done, succ = out if out is not None else (self._obs, self._reward, self._done, self._success)
             _lib.check(_lib.lib().earl_tt3_step(self._handle, a.data_ptr(), obs.data_ptr(), rew.data_ptr(), done.data_ptr(),
                                                 _ptr(succ), _stream()))
-            return obs, rew, done.view(torch.bool), {"success": None if succ is None else succ.view(torch.bool)}
+            info = {"success": None if succ is None else succ.view(torch.bool)}
+            if self._final_obs is not None:
+                info["final_observation"] = self._final_obs
+            return obs, rew, done.view(torch.bool), info
         return self._step_host(action)
 
     def _step_host(self, action):
@@ -277,10 +291,13 @@ class TabletopManipulation:
         ho, hr, hd, hs = hb.next_outputs()
         _lib.check(_lib.lib().earl_tt3_step_host(self._handle, src.data_ptr(), ho.data_ptr(), hr.data_ptr(), hd.data_ptr(),
                    hs.data_ptr()))
-        return HostBuffers.as_numpy(ho, hr, hd, hs)
+        return HostBuffers.as_numpy(ho, hr, hd, hs, self._final_obs)
 
     def rollout_into(self, actions, num_steps, obs, reward, done, success=None):
-        """`num_steps` back-to-back steps: step t reads actions[t % K], writes slot t % R ([K,N,3]; [R,N,20], [R,N])."""
+        """`num_steps` back-to-back steps: step t reads actions[t % K], writes slot t % R ([K,N,3]; [R,N,20], [R,N]).
+        Not available on final_obs=True envs."""
+        if self._keep_final_obs:
+            raise RuntimeError("rollout_into does not keep final observations: step() a final_obs=True env")
         self._ensure()
         K, R = actions.shape[0], obs.shape[0]
         assert actions.is_cuda and actions.dtype == torch.float32 and actions.is_contiguous()

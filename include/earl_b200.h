@@ -64,6 +64,8 @@ typedef enum {
 #define EARL_FLAG_RESET_AT_GOAL 0x20u /* reset_at_goal=True: resets place the env at its new goal (:109-111) */
 #define EARL_FLAG_EVAL_STATS 0x40u    /* accumulate per-env episode return / success for earl_eval_stats */
 #define EARL_FLAG_PER_ENV_GOALS 0x80u /* every env keeps its own goal vector, set on the device (earl_set_goals) */
+#define EARL_FLAG_FINAL_OBS 0x100u    /* with EARL_FLAG_AUTO_RESET only: keep the last observation of every episode a step
+                                         ends in a caller buffer (earl_set_final_obs and its per-task siblings) */
 
 /* goal_dtype of earl_set_goals / earl_mj_set_goals */
 #define EARL_GOAL_F32 0
@@ -162,9 +164,21 @@ EARL_API int earl_get_goals(earl_handle* h, float* goals_out_dev, void* stream);
 EARL_API int earl_step(earl_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev,
               uint8_t* success_dev, void* stream);
 
+/* Final observations of an EARL_FLAG_AUTO_RESET | EARL_FLAG_FINAL_OBS handle (EARL_ERR_INVALID on any other handle,
+ * and EARL_ERR_INVALID from every step of such a handle before this is called): final_obs [N,12] f32, device, 16-byte
+ * aligned like obs, owned by the caller and kept until the handle is destroyed or another buffer is registered.
+ * After a step (earl_step / earl_step_host) in which done[i] is set, row i of final_obs is bit for bit the observation row
+ * the same handle would have returned from that step without auto-reset: the state, the attached flag and the goal
+ * before the reset (after a lifelong goal swap of the same step).  The step's obs row i stays the post-reset
+ * observation.  Rows of envs that did not finish are not written: they keep what was last stored there.  Written by
+ * the step kernel inside its fused reset (no extra launch, 48 B per reset env); every other output and all state are
+ * what the handle without the flag computes.  earl_rollout refuses such a handle (one buffer cannot hold K steps). */
+EARL_API int earl_set_final_obs(earl_handle* h, float* final_obs_dev);
+
 /* `num_steps` consecutive steps launched back to back without returning to the caller: step t reads
  * actions[t % action_ring] and writes obs/reward/done slot t % out_ring of the rollout buffers
- * ([ring,N,...]).  For open-loop action sequences (random-action throughput runs, demo replay). */
+ * ([ring,N,...]).  For open-loop action sequences (random-action throughput runs, demo replay).
+ * EARL_ERR_INVALID on an EARL_FLAG_FINAL_OBS handle. */
 EARL_API int earl_rollout(earl_handle* h, const float* actions_dev, int32_t action_ring, int32_t num_steps, float* obs_dev,
                  float* reward_dev, uint8_t* done_dev, uint8_t* success_dev, int32_t out_ring, void* stream);
 

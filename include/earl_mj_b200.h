@@ -24,7 +24,8 @@ typedef struct {
   int32_t num_envs;
   int32_t device;
   uint32_t flags;           /* EARL_FLAG_EVAL_STATS | EARL_FLAG_LIFELONG | EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET |
-                               EARL_FLAG_PER_ENV_GOALS */
+                               EARL_FLAG_PER_ENV_GOALS | EARL_FLAG_FINAL_OBS (with EARL_FLAG_AUTO_RESET only, else
+                               EARL_ERR_INVALID) */
   int64_t episode_horizon;  /* PersistentStateWrapper(episode_horizon), persistent_state_wrapper.py:10-12 */
   int64_t goal_change_frequency; /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
 } earl_mj_config;
@@ -117,6 +118,16 @@ EARL_API int earl_mj_reset(earl_mj_handle* h, const uint8_t* mask_dev, const dou
  * obs [N,14] f32; reward [N] f32; done [N] u8; success [N] u8 or NULL. */
 EARL_API int earl_mj_step(earl_mj_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev, uint8_t* done_dev,
                           uint8_t* success_dev, void* stream);
+/* Final observations of an EARL_FLAG_AUTO_RESET | EARL_FLAG_FINAL_OBS handle (EARL_ERR_INVALID on any other handle, and
+ * from every step of such a handle before this is called): final_obs [N,14] f32, device, owned by the caller and kept
+ * until the handle is destroyed or another buffer is registered.  After a step (earl_mj_step / earl_mj_step_host) in which
+ * done[i] is set, row i of final_obs is bit for bit the observation row the same handle would have returned from that step
+ * without auto-reset -- what the step kernel, or the redo kernel for an env it re-stepped, wrote, including the contained
+ * last stable observation after a failed simulation and the goal after a lifelong goal swap; the step's obs row i stays
+ * the post-reset observation.  Rows of envs that did not finish are not written.  One more launch per step (launch_count
+ * shows it), in `stream` between the ordering kernel and the reset pass, copying the rows of the reset envs only; every
+ * other output and all state, statistics and reset-stream cursors are what the handle without the flag computes. */
+EARL_API int earl_mj_set_final_obs(earl_mj_handle* h, float* final_obs_dev);
 /* Same with HOST buffers (copies inside the call, synchronous). */
 EARL_API int earl_mj_step_host(earl_mj_handle* h, const float* actions_host, float* obs_host, float* reward_host,
                                uint8_t* done_host, uint8_t* success_host);

@@ -44,8 +44,8 @@ typedef struct earl_mjk_handle earl_mjk_handle;
 
 typedef struct {
   int32_t num_envs, device;
-  uint32_t flags;                 /* EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS (any other flag is
-                                     rejected) */
+  uint32_t flags;                 /* EARL_FLAG_LIFELONG | EARL_FLAG_AUTO_RESET | EARL_FLAG_EVAL_STATS | EARL_FLAG_FINAL_OBS
+                                     (the last with EARL_FLAG_AUTO_RESET only; any other flag is rejected) */
   int32_t frame_skip;             /* 40 (KitchenV0.__init__, kitchen_multitask_v0.py:38) */
   int64_t episode_horizon;        /* PersistentStateWrapper(episode_horizon) */
   int64_t goal_change_frequency;  /* LifelongWrapper(goal_change_frequency), lifelong_wrapper.py:19-24; 0 = unused */
@@ -92,6 +92,16 @@ EARL_API int earl_mjk_reset(earl_mjk_handle* h, const int32_t* env_ids_dev, int3
  * u8 [N] or NULL. */
 EARL_API int earl_mjk_step(earl_mjk_handle* h, const float* actions_dev, double* obs_dev, double* reward_dev, uint8_t* done_dev,
                            uint8_t* success_dev, void* stream);
+/* Final observations of an EARL_FLAG_AUTO_RESET | EARL_FLAG_FINAL_OBS handle (EARL_ERR_INVALID on any other handle, and
+ * from every step of such a handle before this is called): final_obs f64 [N,46], device, owned by the caller and kept
+ * until the handle is destroyed or another buffer is registered.  After an earl_mjk_step in which done[i] is set, row i of
+ * final_obs is bit for bit the observation row the same handle would have returned from that step without auto-reset:
+ * the noisy observation (the lifelong second draw when the goal swap fell on that step), as the step or redo kernel wrote
+ * it; the step's obs row i stays the post-reset observation.  Rows of envs that did not finish are not written.  One more
+ * launch per step, in `stream` between the ordering kernels and the reset pass, copying the rows of the reset envs only;
+ * every other output and all state, statistics, noise streams and reset-stream cursors are what the handle without the
+ * flag computes. */
+EARL_API int earl_mjk_set_final_obs(earl_mjk_handle* h, double* final_obs_dev);
 /* sim state as host arrays (synchronous): qpos, qvel, qacc_warmstart f64 [N,23], mocap_pos f64 [N,3], last noisy robot
  * qpos f64 [N,9] (the Robot_VelAct observation cache), site positions f64 [N,8,3] of the last forward pass. NULL = skip. */
 EARL_API int earl_mjk_get_state(earl_mjk_handle* h, double* qpos_host, double* qvel_host, double* warm_host, double* mocap_host,

@@ -33,7 +33,8 @@ typedef struct {
   int32_t num_envs;          /* N >= 1 */
   int32_t device;            /* CUDA device ordinal */
   uint32_t flags;            /* EARL_FLAG_DENSE_REWARD | EARL_FLAG_AUTO_RESET | EARL_FLAG_RESET_AT_GOAL |
-                                EARL_FLAG_EVAL_STATS (earl_b200.h); any other flag is EARL_ERR_UNSUPPORTED */
+                                EARL_FLAG_EVAL_STATS | EARL_FLAG_FINAL_OBS (earl_b200.h; the last only with
+                                EARL_FLAG_AUTO_RESET, else EARL_ERR_INVALID); any other flag is EARL_ERR_UNSUPPORTED */
   int32_t num_goals;         /* rows used in goal_table, 1..EARL_TT3_MAX_GOALS (reference: 1, :12-18) */
   int64_t episode_horizon;   /* PersistentStateWrapper(episode_horizon) */
   double threshold;          /* 0.4  attach radius, strict <            (:38, :107) */
@@ -71,7 +72,18 @@ EARL_API int earl_tt3_set_goal(earl_tt3_handle* h, const uint8_t* mask_dev, cons
 EARL_API int earl_tt3_step(earl_tt3_handle* h, const float* actions_dev, float* obs_dev, float* reward_dev,
                            uint8_t* done_dev, uint8_t* success_dev, void* stream);
 
-/* `num_steps` steps back to back: step t reads actions[t % action_ring], writes output slot t % out_ring */
+/* Final observations of an EARL_FLAG_AUTO_RESET | EARL_FLAG_FINAL_OBS handle (EARL_ERR_INVALID on any other handle, and
+ * from every step of such a handle before this is called): final_obs [N,20] f32, device, 16-byte aligned, owned by the
+ * caller and kept until the handle is destroyed or another buffer is registered.  After a step (earl_tt3_step /
+ * earl_tt3_step_host) in which done[i] is set, row i of final_obs is bit for bit the observation row the same handle
+ * would have returned from that step without auto-reset (qpos[0:8], attached marker, goal before the reset); the step's
+ * obs row i stays the post-reset observation.  Rows of envs that did not finish are not written.  Written by the step
+ * kernel inside its fused reset (no extra launch, 80 B per reset env); every other output and all state, statistics and
+ * reset-stream cursors are what the handle without the flag computes.  earl_tt3_rollout refuses such a handle. */
+EARL_API int earl_tt3_set_final_obs(earl_tt3_handle* h, float* final_obs_dev);
+
+/* `num_steps` steps back to back: step t reads actions[t % action_ring], writes output slot t % out_ring
+ * (EARL_ERR_INVALID on an EARL_FLAG_FINAL_OBS handle) */
 EARL_API int earl_tt3_rollout(earl_tt3_handle* h, const float* actions_dev, int32_t action_ring, int32_t num_steps,
                               float* obs_dev, float* reward_dev, uint8_t* done_dev, uint8_t* success_dev,
                               int32_t out_ring, void* stream);
