@@ -8,6 +8,7 @@
 #include "../../earl_benchmark_b200/csrc/mj_engine.cuh"
 #include "../../earl_benchmark_b200/csrc/mj_model_host.hpp"
 #include "../../earl_benchmark_b200/csrc/mj_step.cuh"
+#include "phases.hpp"
 
 using namespace earl::mj;
 
@@ -34,13 +35,7 @@ void emu_destroy(void* h) { delete static_cast<Emu*>(h); }
 void emu_set_state(void* h, const double* qpos, const double* qvel, const double* warm, const double* mocap_pos,
                    const double* mocap_quat, const double* ctrl) {
   Emu* e = static_cast<Emu*>(h);
-  const Model& m = e->hm.m;
-  for (int k = 0; k < m.nq; ++k) e->w.qpos[k] = (real)qpos[k];
-  for (int k = 0; k < m.nv; ++k) { e->w.qvel[k] = (real)qvel[k]; e->w.warm[k] = (real)warm[k]; }
-  for (int k = 0; k < 3; ++k) e->w.mocap_pos[k] = mocap_pos[k];
-  for (int k = 0; k < 4; ++k) e->w.mocap_quat[k] = (real)mocap_quat[k];
-  for (int k = 0; k < m.nu; ++k) e->w.ctrl[k] = (real)ctrl[k];
-  e->w.broad_valid = 0;  // a new state: the cached broad-phase candidates are stale
+  load_state(e->hm.m, e->w, qpos, qvel, warm, mocap_pos, mocap_quat, ctrl);  // also: the cached broad-phase candidates are stale
 }
 void emu_get_state(void* h, double* qpos, double* qvel, double* warm, double* mocap_pos) {
   Emu* e = static_cast<Emu*>(h);
@@ -84,16 +79,6 @@ int emu_info(void* h, int what) {
   }
   return -1;
 }
-void emu_contacts(void* h, double* dist, double* pos, double* frame, int* geoms) {
-  Emu* e = static_cast<Emu*>(h);
-  for (int c = 0; c < e->w.ncon; ++c) {
-    dist[c] = e->w.con_dist[c];
-    for (int k = 0; k < 3; ++k) pos[3 * c + k] = e->w.con_pos[c][k];
-    for (int k = 0; k < 9; ++k) frame[9 * c + k] = e->w.con_frame[c][k];
-    geoms[2 * c] = e->w.con_g1[c];
-    geoms[2 * c + 1] = e->w.con_g2[c];
-  }
-}
 }
 extern "C" int emu_hits(void* h, int* pairs) {
   Emu* e = static_cast<Emu*>(h);
@@ -123,4 +108,46 @@ extern "C" int emu_mpr(int t1, const float* size1, const float* p1, const float*
   S.o1 = CObj{t1, 0, 0.5f * margin, p1, R1, size1, nullptr};
   S.o2 = CObj{t2, 0, 0.5f * margin, p2, R2, size2, nullptr};
   return mpr_penetration<1>(S.o1, S.o2, out, out + 1, out + 4, &S, 0);
+}
+
+// the phases of one substep (tests/host_emulation/phases.hpp) and readers of what they leave behind; the signatures are
+// those of the device harness (devemul.cu), where `i` picks one of a batch of states -- here there is one state, i = 0
+extern "C" {
+void ph_caps(int* out) { read_caps(out); }
+void emu_run(void* h, int stage, int nsub) {
+  Emu* e = static_cast<Emu*>(h);
+  run_stage<1>(e->hm.m, e->hm.hull_vert.data(), e->w, stage, nsub, 0);
+}
+int ph_state(void* h, int i, double* qpos, double* qvel, double* warm) {
+  if (i != 0) return -1;
+  read_state(static_cast<Emu*>(h)->hm.m, static_cast<Emu*>(h)->w, qpos, qvel, warm);
+  return 0;
+}
+int ph_info(void* h, int i, int* out) {
+  if (i != 0) return -1;
+  read_info(static_cast<Emu*>(h)->w, out);
+  return 0;
+}
+int ph_forward(void* h, int i, double* xpos, double* xmat, double* M, double* bias) {
+  if (i != 0) return -1;
+  read_forward(static_cast<Emu*>(h)->hm.m, static_cast<Emu*>(h)->w, xpos, xmat, M, bias);
+  return 0;
+}
+int ph_hits(void* h, int i, int* pairs) { return i != 0 ? -1 : read_hits(static_cast<Emu*>(h)->hm.m, static_cast<Emu*>(h)->w, pairs); }
+int ph_contacts(void* h, int i, double* dist, double* pos, double* frame, int* geoms) {
+  return i != 0 ? -1 : read_contacts(static_cast<Emu*>(h)->w, dist, pos, frame, geoms);
+}
+int ph_rows(void* h, int i, int* type, double* J, double* pos, double* R, double* D, double* aref, int* con, double* mu, double* fri) {
+  return i != 0 ? -1 : read_rows(static_cast<Emu*>(h)->hm.m, static_cast<Emu*>(h)->w, type, J, pos, R, D, aref, con, mu, fri);
+}
+int ph_solve(void* h, int i, double* acc, double* fcon, double* smooth, double* force) {
+  if (i != 0) return -1;
+  read_solve(static_cast<Emu*>(h)->hm.m, static_cast<Emu*>(h)->w, acc, fcon, smooth, force);
+  return 0;
+}
+// spd_solve<1> (chol_factor + chol_solve) on one caller matrix in the LDM-padded layout A [MAXV][LDM], x [MAXV]
+int emu_spd_solve(int n, float* A, float* x) {
+  if (n < 1 || n > MAXV) return -1;
+  return spd_solve<1>(reinterpret_cast<real(*)[LDM]>(A), n, x, 0);
+}
 }

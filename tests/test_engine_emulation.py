@@ -1,6 +1,8 @@
 """The engine kernel source (csrc/mj_*.cuh) compiled for the host with one lane, checked against the fp64 checker
 (oracle/mjengine.c) -- the CPU-side guard for the code the GPU runs.  North-star bar: from identical states and
 actions, one-step qpos / qvel within 1e-4 absolute (fp32 engine vs fp64)."""
+import os
+
 import numpy as np
 import pytest
 
@@ -161,3 +163,12 @@ def test_peg_scene_one_step_parity(peg):
         max_con = max(max_con, e.ncon)
     assert max_con >= 10
     assert worst_q < TOL and worst_v < TOL, (worst_q, worst_v)
+
+
+def test_device_harness_compiles_for_every_capacity_set(tmp_path):
+    """The 32-lane twin of this file's one-lane build (tests/host_emulation/devemul.cu, run on the GPU by
+    test_engine_device_phases_gpu.py) cross-compiles for sm_100a with the product's engine flags in all four capacity
+    sets: door / peg primary and extra-large, kitchen primary and extra-large.  No GPU needed."""
+    from host_emulation.emu import CAPSETS, build_device
+    for so in build_device(tuple(CAPSETS), out_dir=str(tmp_path)):
+        assert os.path.getsize(so) > 0
